@@ -62,7 +62,13 @@ def parse():
     ap.add_argument("--two-kernels", action="store_true",
                     help="random-policy kernel + step kernel per step instead of the policy fused into the step kernel")
     ap.add_argument("--u-noise", type=float, default=0.0, help="motor noise of the headline workload (core.py:232-236)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned (obs, reward, done, individual reward, "
+                         "recorded actions) as DIR/<name>.npy, for a fixed sample of envs when all would exceed 16 MB")
+    a = ap.parse_args()
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs applies to the CUDA path (--impl b200)")
+    return a
 
 
 def hbm_peak():
@@ -222,6 +228,38 @@ def workload_config(a, envs_per_unit, where):
             "l2": "inputs larger than L2 (step traffic > 126 MB), no flush" if where == "gpu" else None}
 
 
+DUMP_BYTES = 16 * 10 ** 6
+
+
+def env_snapshot(torch, env):
+    """Host Philox tick and a copy of every device buffer of a BatchedFormationEnv (state, outputs, device tick)."""
+    return env._tick, {k: v.clone() for k, v in vars(env).items() if torch.is_tensor(v) and v.is_cuda}
+
+
+def env_restore(env, snapshot):
+    """Put a snapshot back in place: the env's buffers keep their addresses, so captured CUDA graphs stay valid."""
+    env._tick = snapshot[0]
+    for k, v in snapshot[1].items():
+        getattr(env, k).copy_(v)
+
+
+def dump_outputs(out_dir, torch, env):
+    """What the step last returned -- obs, reward, done, individual reward -- and the actions it recorded, as
+    DIR/<name>.npy in the env's float type.  Envs are sampled with a fixed seed (ascending index order) when all of
+    them would exceed DUMP_BYTES."""
+    import numpy as np
+    outs = {"obs": env.obs, "reward": env.reward, "done": env.done, "individual_reward": env.indiv,
+            "actions": env.actions}
+    outs = {k: v for k, v in outs.items() if v is not None}
+    per_env = sum(v[0].numel() for v in outs.values()) * torch.finfo(env.dtype).bits // 8
+    n = max(1, min(env.E, DUMP_BYTES // per_env))
+    idx = np.sort(np.random.RandomState(0).choice(env.E, n, replace=False)) if n < env.E else np.arange(env.E)
+    sel = torch.as_tensor(idx, device=env.device)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in outs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), v.index_select(0, sel).to(env.dtype).cpu().numpy())
+
+
 def run_b200(a):
     import torch
     import torch.distributed as dist
@@ -276,6 +314,9 @@ def run_b200(a):
     if graph is not None:
         graph.replay()
     torch.cuda.synchronize()
+    # the settle phase below runs for a fixed time, not a fixed number of steps: the state it leaves is put back, so
+    # that the timed steps start from the same state and draw the same actions in every run
+    snapshot = env_snapshot(torch, env)
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     sampler = ClockSampler(local_rank) if rank == 0 else None
     if sampler:
@@ -291,6 +332,8 @@ def run_b200(a):
             one_step(); settle_steps += 1
         if settle_steps % (8 * chunk) == 0:
             torch.cuda.synchronize()
+    env_restore(env, snapshot)
+    del snapshot
     launches0 = env.launches
     barrier(); torch.cuda.synchronize()
     ev0.record()
@@ -302,6 +345,8 @@ def run_b200(a):
             one_step()
     ev1.record()
     torch.cuda.synchronize(); barrier()
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, torch, env)
     launches = (2 if a.two_kernels else 1) * K                    # (fg::k_random_actions +) step kernel per step
     ms = ev0.elapsed_time(ev1)
 

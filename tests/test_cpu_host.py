@@ -331,20 +331,49 @@ def test_render_bridge_rgb_array_on_host():
     assert env.render(close=True) == []
 
 
+_STAND_IN_REFERENCE = {
+    # a minimal package with the reference's layout and make_env / step API, so that staging and the harness are
+    # exercised without a checkout of the reference
+    "formation_gym/__init__.py": "def make_env(scenario_name, benchmark=False, num_agents=3):\n"
+                                 "    from formation_gym.environment import MultiAgentEnv\n"
+                                 "    return MultiAgentEnv(num_agents)\n",
+    "formation_gym/core.py": "class World(object):\n    world_length = 25\n",
+    "formation_gym/environment.py": "from formation_gym.core import World\n\n\n"
+                                    "class MultiAgentEnv(object):\n"
+                                    "    def __init__(self, n):\n"
+                                    "        self.n, self.world, self.t = n, World(), 0\n\n"
+                                    "    def reset(self):\n"
+                                    "        self.t = 0\n"
+                                    "        return [[0.0]] * self.n\n\n"
+                                    "    def step(self, act_n):\n"
+                                    "        self.t += 1\n"
+                                    "        done = self.t >= self.world.world_length\n"
+                                    "        return [[0.0]] * self.n, [[0.0]] * self.n, [done] * self.n, [{}] * self.n\n",
+    "formation_gym/scenario.py": "class BaseScenario(object):\n    pass\n",
+    "formation_gym/envs/__init__.py": "",
+    "formation_gym/envs/formation_hd_env.py": "from formation_gym.scenario import BaseScenario\n\n\n"
+                                              "class Scenario(BaseScenario):\n    pass\n",
+}
+
+
 def test_staged_reference_is_byte_identical_and_runs():
-    """oracle/make_ref.py stages the files of the reference's step path byte for byte (sha256 manifest) into the
-    git-ignored oracle/_ref, and the harness runs an env from that copy -- what the GPU box does."""
-    if not os.path.isfile("/root/reference/formation_gym/core.py"):
-        pytest.skip("no reference checkout in this environment")
+    """oracle/make_ref.py stages the files of the reference's step path byte for byte (sha256 manifest) into a
+    git-ignored directory like oracle/_ref, and the harness runs an env from that copy.  The source is a stand-in
+    tree with the reference's layout."""
     import hashlib
     from oracle import make_ref
     with tempfile.TemporaryDirectory() as d:
-        dst = make_ref.make(dst=os.path.join(d, "_ref"), quiet=True)
+        src = os.path.join(d, "reference")
+        for rel, text in _STAND_IN_REFERENCE.items():
+            os.makedirs(os.path.dirname(os.path.join(src, rel)), exist_ok=True)
+            open(os.path.join(src, rel), "w").write(text)
+        dst = make_ref.make(src=src, dst=os.path.join(d, "_ref"), quiet=True)
         assert make_ref.staged_ok(dst)
         man = json.load(open(os.path.join(dst, "MANIFEST.json")))["files"]
         assert "formation_gym/core.py" in man and "formation_gym/envs/formation_hd_env.py" in man
+        assert sorted(man) == sorted(_STAND_IN_REFERENCE)
         for rel, h in man.items():
-            assert hashlib.sha256(open(os.path.join("/root/reference", rel), "rb").read()).hexdigest() == h
+            assert hashlib.sha256(open(os.path.join(src, rel), "rb").read()).hexdigest() == h
         env = dict(os.environ, FG_REFERENCE_ROOT=dst)
         out = subprocess.run([sys.executable, os.path.join(ROOT, "oracle", "ref_harness.py"), "--agents", "3", "--procs", "1",
                               "--max-steps", "5", "--warmup", "1"], capture_output=True, text=True, timeout=300, env=env)
