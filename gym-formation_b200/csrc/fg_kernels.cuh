@@ -122,6 +122,28 @@ __device__ __forceinline__ void tick_arrive(uint32_t* tick_dev, unsigned partici
 }
 
 // ------------------------------------------------------------------------------------------------
+// Contact cut-off of an env (DESIGN.md "contact cut-off").  Every pair loop skips a pair when its squared distance
+// passes !(d2 >= cut2) -- NaN distances stay, but d2 = +inf would be dropped, where the reference (no cut-off,
+// core.py:304-312) turns it into dist = inf, pen = 0 and force = 0 * inf / inf = NaN.  So an env with a non-finite
+// old position of a colliding entity sends every pair to contact_force: through a NaN cut-off (env_cut2: k_lm_warp,
+// k_step_obst) or, off the hot pair loops, through its near mask (k_hd_warp) or an all-pairs loop (k_step).  Finite
+// envs keep the plain cut-off and their exact results.
+template <typename T>
+__device__ __forceinline__ bool nonfinite2(T x, T y) { return !(fabs(x) < (T)INFINITY) || !(fabs(y) < (T)INFINITY); }
+
+template <typename R2>
+__device__ __forceinline__ bool any_nonfinite(const R2* p, int n) {
+    bool bad = false;
+    for (int j = 0; j < n; ++j) bad |= nonfinite2(p[j].x, p[j].y);
+    return bad;
+}
+
+template <typename T>
+__device__ __forceinline__ T env_cut2(T cut2, bool env_nonfinite) {
+    return env_nonfinite ? Ops<T>::from_bits(~(typename Ops<T>::Bits)0 >> 1) : cut2;
+}
+
+// ------------------------------------------------------------------------------------------------
 // get_entity_collision_force (core.py:289-322), both entities movable colliders (agents).
 // (dx,dy) = p_a - p_b with a < b in entity order.  Returns `force` (core.py:312).
 template <typename T>
@@ -410,18 +432,30 @@ __global__ void __launch_bounds__(kBlock, (OM == 3 && SCN == kScnBasic) ? 5 : (O
         // an env's rows over two CTAs that both run the physics would not shrink it: with every CTA writing only HALF
         // of its rows (timing experiment) the fit is 24.4 us + 0.111 us per CTA, so 1024 envs as 2048 half-CTAs cost
         // 245.6 us against 241.1 us now.)
-        bool early = false;
+        // The barrier also tells whether some env of the tile holds a non-finite old position (only then do the
+        // threads scan their env for one, see env_cut2).  s_old[t] is this thread's own write.
+        bool obad = false;
+        if (PHYS && active && a.collide) { const R2 q = a.cpos ? s_old[t] : p; obad = nonfinite2(q.x, q.y); }
+        bool early = false, tile_nf;
         if constexpr (OM == 2 && sizeof(R2) == 8) {
             if (a.obs && a.row_early) {
                 const bool will_reset = active && a.auto_reset && a.step && (stp + 1 >= a.world_length);
                 asm volatile("fence.proxy.async.shared::cta;" ::: "memory");     // images (generic proxy) -> async proxy
-                early = !__syncthreads_or(will_reset ? 1 : 0);
+                tile_nf = __syncthreads_or((will_reset || obad) ? 1 : 0) != 0;   // rare: then ask both questions
+                if (tile_nf) {
+                    early = !__syncthreads_or(will_reset ? 1 : 0);
+                    tile_nf = __syncthreads_or(obad ? 1 : 0) != 0;
+                } else {
+                    early = true;
+                }
             } else {
-                __syncthreads();
+                tile_nf = __syncthreads_or(obad ? 1 : 0) != 0;
             }
         } else {
-            __syncthreads();
+            tile_nf = __syncthreads_or(obad ? 1 : 0) != 0;
         }
+        // my env holds a non-finite old position: every pair goes to the contact force, in the loop below
+        const bool env_nf = tile_nf && active && any_nonfinite(s_old + le * N, N);
 
         CellPos cpos = {0, 0, 1, 1};                                        // FP + cells: my cell (old positions)
         if constexpr (FP && PHYS) {
@@ -457,6 +491,30 @@ __global__ void __launch_bounds__(kBlock, (OM == 3 && SCN == kScnBasic) ? 5 : (O
                 // i in ascending order of the other index, exactly the reference's order.
                 if (a.collide) {
                     const R2* envp = s_old + le * N;
+                    if (env_nf) {
+                        // rare: an env with a non-finite old position -- no cut-off (see env_cut2), every pair in
+                        // ascending j, masses and sizes as in the loops below
+                        const bool cached = a.cpos != nullptr;
+                        const R2 pc = envp[i];
+                        for (int j = 0; j < N; ++j) {
+                            if (j == i) continue;
+                            R2 q = envp[j];
+                            T dx = (j < i) ? O::sub(q.x, pc.x) : O::sub(pc.x, q.x);   // delta = p_a - p_b, a<b
+                            T dy = (j < i) ? O::sub(q.y, pc.y) : O::sub(pc.y, q.y);
+                            const T dmin = HET ? O::add((j < i) ? s_het[N + j] : size_i, (j < i) ? size_i : s_het[N + j])
+                                               : O::add(a.size, a.size);
+                            T fx, fy;
+                            contact_force<T>(dx, dy, dmin, a.margin, a.cforce, &fx, &fy, cached);
+                            if (HET) {
+                                T m_j = s_het[j];
+                                if (j < i) { T c = -O::div((T)1, O::div(m_i, m_j)); Fx = O::add(O::mul(c, fx), Fx); Fy = O::add(O::mul(c, fy), Fy); }
+                                else       { T r = O::div(m_j, m_i); Fx = O::add(O::mul(r, fx), Fx); Fy = O::add(O::mul(r, fy), Fy); }
+                            } else {
+                                if (j < i) { Fx = O::add(-fx, Fx); Fy = O::add(-fy, Fy); }
+                                else       { Fx = O::add(fx, Fx);  Fy = O::add(fy, Fy); }
+                            }
+                        }
+                    } else
                     if constexpr (FP) {
                         // candidate groups of four partners from the packed filter, then the reference's exact
                         // test and force for the members of flagged groups, in ascending j
@@ -519,7 +577,7 @@ __global__ void __launch_bounds__(kBlock, (OM == 3 && SCN == kScnBasic) ? 5 : (O
                                 T dx = O::sub(p.x, q.x), dy = O::sub(p.y, q.y);
                                 T d2 = dx * dx + dy * dy;
                                 // Far pairs: softplus(-(d-dmin)/k) < exp(-kcut) -- below the rounding of
-                                // F (DESIGN.md "contact cut-off").  !(>=) keeps NaN positions propagating.
+                                // F (DESIGN.md "contact cut-off").  !(>=) keeps NaN pairs; inf ones: env_nf above.
                                 near |= (!(d2 >= a.cut2)) ? (1u << jj) : 0u;
                             }
                             if ((unsigned)(i - j0) < 32u) near &= ~(1u << (i - j0));
@@ -553,7 +611,7 @@ __global__ void __launch_bounds__(kBlock, (OM == 3 && SCN == kScnBasic) ? 5 : (O
                                 cut2 = a.cut2;
                             }
                             // Far pairs: softplus(-(d-dmin)/k) < exp(-kcut) -- below the rounding of F
-                            // (DESIGN.md "contact cut-off").  !(>=) keeps NaN positions propagating.
+                            // (DESIGN.md "contact cut-off").  !(>=) keeps NaN pairs; inf ones: env_nf above.
                             if (!(d2 >= cut2)) {
                                 T fx, fy;
                                 contact_force<T>(dx, dy, dmin, a.margin, a.cforce, &fx, &fy, cached);

@@ -93,9 +93,25 @@ __global__ void __launch_bounds__(kBlock, 2) k_step_obst(const __grid_constant__
         if (!PHYS) s_on[q] = a.lm[gi];
     }
 
+    if (PHYS) __syncthreads();                               // the obstacle positions above, for the checks below
+
     for (int ts = 0; ts < a.n_steps; ++ts) {
         if (t < EPC) { s_rowmax[t] = 0; s_col[t] = 0; s_bad[t] = 0; }
-        __syncthreads();
+        // some env of the tile holds a non-finite old agent or obstacle position: then every thread scans its env and
+        // such an env runs with NaN contact cut-offs (env_cut2, fg_kernels.cuh).  Each check reads this thread's own
+        // writes: s_old[t] (= p) and, for ts > 0, the obstacle entries of the stride loop at the end of the step.
+        bool obad = false;
+        if (PHYS) {                                           // (obstacle pairs collide whatever a.collide says)
+            obad = active && nonfinite2(p.x, p.y);
+            for (int q = t; q < nvalid * NO; q += kBlock) {
+                const R2 po = s_lm[(q / NO) * L + LG + q % NO];
+                obad |= nonfinite2(po.x, po.y);
+            }
+        }
+        const bool tile_nf = __syncthreads_or(obad ? 1 : 0) != 0;
+        auto env_nf = [&](int qe) -> bool {
+            return tile_nf && (any_nonfinite(s_old + qe * N, N) || any_nonfinite(s_lm + qe * L + LG, NO));
+        };
 
         // =============================== World.step (core.py:206-225) ===========================
         if (PHYS) {
@@ -114,6 +130,8 @@ __global__ void __launch_bounds__(kBlock, 2) k_step_obst(const __grid_constant__
                     Fy = O_::add(Fy, O_::mul(n1, a.u_noise));
                 }
                 if (a.collide) {
+                    const bool nf = env_nf(le);
+                    const T c2_aa = env_cut2(a.cut2, nf), c2_ao = env_cut2(cut2_ao, nf);
                     // agent-agent pairs, other index ascending (equal masses: ratio 1)
                     const R2* envp = s_old + le * N;
                     for (int j = 0; j < N; ++j) {
@@ -121,7 +139,7 @@ __global__ void __launch_bounds__(kBlock, 2) k_step_obst(const __grid_constant__
                         R2 q = envp[j];
                         T dx = (j < i) ? O_::sub(q.x, p.x) : O_::sub(p.x, q.x);     // delta = p_a - p_b, a < b
                         T dy = (j < i) ? O_::sub(q.y, p.y) : O_::sub(p.y, q.y);
-                        if (!(dx * dx + dy * dy >= a.cut2)) {                       // far pairs: see DESIGN.md cut-off
+                        if (!(dx * dx + dy * dy >= c2_aa)) {                        // far pairs: see DESIGN.md cut-off
                             T fx, fy;
                             contact_force<T>(dx, dy, dmin_aa, a.margin, a.cforce, &fx, &fy);
                             if (j < i) { Fx = O_::add(-fx, Fx); Fy = O_::add(-fy, Fy); }
@@ -134,7 +152,7 @@ __global__ void __launch_bounds__(kBlock, 2) k_step_obst(const __grid_constant__
                     for (int k = 0; k < NO; ++k) {
                         R2 q = envo[k];
                         T dx = O_::sub(p.x, q.x), dy = O_::sub(p.y, q.y);
-                        if (!(dx * dx + dy * dy >= cut2_ao)) {
+                        if (!(dx * dx + dy * dy >= c2_ao)) {
                             T fx, fy;
                             contact_force<T>(dx, dy, dmin_ao, a.margin, a.cforce, &fx, &fy);
                             Fx = O_::add(O_::mul(ratio, fx), Fx); Fy = O_::add(O_::mul(ratio, fy), Fy);
@@ -165,13 +183,15 @@ __global__ void __launch_bounds__(kBlock, 2) k_step_obst(const __grid_constant__
                 const R2* envo = s_lm + qe * L + LG;
                 const R2 po = envo[k];
                 T Fx = (T)0, Fy = (T)0;                                          // p_force[b] = 0.0 (core.py:252-253)
+                const bool nf = env_nf(qe);
+                const T c2_ao = env_cut2(cut2_ao, nf), c2_oo = env_cut2(cut2_oo, nf);
                 if (a.collide) {
                     const R2* envp = s_old + qe * N;
                     const T c = -O_::div((T)1, O_::div(a.omass, a.mass));
                     for (int j = 0; j < N; ++j) {
                         R2 pj = envp[j];
                         T dx = O_::sub(pj.x, po.x), dy = O_::sub(pj.y, po.y);
-                        if (!(dx * dx + dy * dy >= cut2_ao)) {
+                        if (!(dx * dx + dy * dy >= c2_ao)) {
                             T fx, fy;
                             contact_force<T>(dx, dy, dmin_ao, a.margin, a.cforce, &fx, &fy);
                             Fx = O_::add(O_::mul(c, fx), Fx); Fy = O_::add(O_::mul(c, fy), Fy);
@@ -183,7 +203,7 @@ __global__ void __launch_bounds__(kBlock, 2) k_step_obst(const __grid_constant__
                     R2 q2 = envo[m];
                     T dx = (m < k) ? O_::sub(q2.x, po.x) : O_::sub(po.x, q2.x);
                     T dy = (m < k) ? O_::sub(q2.y, po.y) : O_::sub(po.y, q2.y);
-                    if (!(dx * dx + dy * dy >= cut2_oo)) {
+                    if (!(dx * dx + dy * dy >= c2_oo)) {
                         T fx, fy;
                         contact_force<T>(dx, dy, dmin_oo, a.margin, a.cforce, &fx, &fy);
                         if (m < k) { Fx = O_::add(-fx, Fx); Fy = O_::add(-fy, Fy); }     // equal obstacle masses

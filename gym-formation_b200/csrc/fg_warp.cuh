@@ -236,6 +236,12 @@ __global__ void __launch_bounds__(32 * WarpLayout<T, N, WOBS>::MAXW, (SCN == kSc
     for (int ts = 0; ts < n_steps; ++ts) {
         if (lane < EPW) { s_max[lane] = 0; s_col[lane] = 0; }
         if (lane < NA) s_pold[lane] = p;
+        // Does my env hold a non-finite old position?  Then every pair goes to the contact force (env_cut2,
+        // fg_kernels.cuh).  The warp-uniform vote on |x| + |y| (inactive lanes hold zeros) keeps the common path at a few
+        // instructions; the exact per-env ballot runs only in a warp that has such a position (or one near FLT_MAX).
+        const bool warp_nf = f_collide && __any_sync(FULL, !(fabs(p.x) + fabs(p.y) < (T)INFINITY));
+        bool env_nf = false;
+        if (warp_nf) env_nf = (__ballot_sync(FULL, active && nonfinite2(p.x, p.y)) & envmask) != 0u;
         __syncwarp();
 
         // =============================== World.step (core.py:206-225) ===========================
@@ -271,6 +277,7 @@ __global__ void __launch_bounds__(32 * WarpLayout<T, N, WOBS>::MAXW, (SCN == kSc
                     T d2 = dx * dx + dy * dy;
                     near |= (!(d2 >= a.cut2)) ? (1u << j) : 0u;             // !(>=) keeps NaN pairs
                 }
+                if (warp_nf && env_nf) near = (N == 32) ? 0xffffffffu : ((1u << (N & 31)) - 1u);   // and inf ones
                 near &= ~(1u << i);
                 // (Round 2: the point differences of this loop and of the reward loop as ONE packed FMA each --
                 // fma.rn.f32x2 p * (-1, -1) + q, bit-identical to two FSUBs, 35 FFMA2 and 40 fewer SASS instructions at

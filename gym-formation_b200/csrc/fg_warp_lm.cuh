@@ -201,6 +201,16 @@ __global__ void __launch_bounds__(32 * LmLayout<T, N, L, SCN, NOBS>::MAXW, 3) k_
     for (int ts = 0; ts < n_steps; ++ts) {
         if (lane < EPW) { s_max[lane] = 0; s_col[lane] = 0; }
         if (lane < NA) s_pold[lane] = p;
+        // contact cut-offs of my env: NaN when one of its old agent or obstacle positions is not finite (env_cut2,
+        // fg_kernels.cuh)
+        T cut2 = a.cut2, c2_ao = cut2_ao, c2_oo = cut2_oo;
+        if (f_collide || OBST) {                                            // (obstacle pairs collide whatever collide says)
+            bool bad = active && nonfinite2(p.x, p.y);
+            if (obst_lane) { const R2 po = s_lm[le * L + LG + i]; bad |= nonfinite2(po.x, po.y); }
+            const bool env_nf = (__ballot_sync(FULL, bad) & envmask) != 0u;
+            cut2 = env_cut2(a.cut2, env_nf);
+            if constexpr (OBST) { c2_ao = env_cut2(cut2_ao, env_nf); c2_oo = env_cut2(cut2_oo, env_nf); }
+        }
         __syncwarp();
 
         // =============================== World.step (core.py:206-225) ===========================
@@ -231,7 +241,7 @@ __global__ void __launch_bounds__(32 * LmLayout<T, N, L, SCN, NOBS>::MAXW, 3) k_
                     R2 q = ep[j];
                     T dx = O::sub(p.x, q.x), dy = O::sub(p.y, q.y);
                     T d2 = dx * dx + dy * dy;
-                    near |= (!(d2 >= a.cut2)) ? (1u << j) : 0u;             // !(>=) keeps NaN pairs
+                    near |= (!(d2 >= cut2)) ? (1u << j) : 0u;               // !(>=) keeps NaN pairs; see env_cut2
                 }
                 near &= ~(1u << i);
                 const T dmin = O::add(a.size, a.size);                      // core.py:307
@@ -255,7 +265,7 @@ __global__ void __launch_bounds__(32 * LmLayout<T, N, L, SCN, NOBS>::MAXW, 3) k_
                     for (int k = 0; k < NO; ++k) {
                         R2 q = envo[k];
                         T dx = O::sub(p.x, q.x), dy = O::sub(p.y, q.y);
-                        if (!(dx * dx + dy * dy >= cut2_ao)) {
+                        if (!(dx * dx + dy * dy >= c2_ao)) {
                             T fx, fy;
                             contact_force<T>(dx, dy, dmin_ao, a.margin, a.cforce, &fx, &fy);
                             Fx = O::add(O::mul(ratio, fx), Fx); Fy = O::add(O::mul(ratio, fy), Fy);
@@ -301,7 +311,7 @@ __global__ void __launch_bounds__(32 * LmLayout<T, N, L, SCN, NOBS>::MAXW, 3) k_
                     for (int j = 0; j < N; ++j) {
                         R2 pj = envp[j];
                         T dx = O::sub(pj.x, po.x), dy = O::sub(pj.y, po.y);
-                        if (!(dx * dx + dy * dy >= cut2_ao)) {
+                        if (!(dx * dx + dy * dy >= c2_ao)) {
                             T fx, fy;
                             contact_force<T>(dx, dy, dmin_ao, a.margin, a.cforce, &fx, &fy);
                             Fx = O::add(O::mul(c, fx), Fx); Fy = O::add(O::mul(c, fy), Fy);
@@ -314,7 +324,7 @@ __global__ void __launch_bounds__(32 * LmLayout<T, N, L, SCN, NOBS>::MAXW, 3) k_
                     R2 q2 = envo[m];
                     T dx = (m < i) ? O::sub(q2.x, po.x) : O::sub(po.x, q2.x);
                     T dy = (m < i) ? O::sub(q2.y, po.y) : O::sub(po.y, q2.y);
-                    if (!(dx * dx + dy * dy >= cut2_oo)) {
+                    if (!(dx * dx + dy * dy >= c2_oo)) {
                         T fx, fy;
                         contact_force<T>(dx, dy, dmin_oo, a.margin, a.cforce, &fx, &fy);
                         if (m < i) { Fx = O::add(-fx, Fx); Fy = O::add(-fy, Fy); }     // equal obstacle masses
