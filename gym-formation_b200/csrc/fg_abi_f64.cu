@@ -26,12 +26,24 @@ int fg_step_fused_f64(const fg_params* p, const fg_buffers* b, int scenario, int
                       int random_actions, int auto_reset, uint64_t seed, uint32_t tick, uint32_t env_offset,
                       void* stream) {
     return step_fused_impl<double>(p, b, scenario, E, N, L, n_steps, random_actions, auto_reset, seed, tick,
-                                   env_offset, stream);
+                                   env_offset, stream, nullptr);
+}
+
+int fg_step_fused_targets_f64(const fg_params* p, const fg_buffers* b, int scenario, int E, int N, int L, int n_steps,
+                              int random_actions, int auto_reset, uint64_t seed, uint32_t tick, uint32_t env_offset,
+                              void* stream, const fg_targets* t) {
+    return step_fused_impl<double>(p, b, scenario, E, N, L, n_steps, random_actions, auto_reset, seed, tick,
+                                   env_offset, stream, t);
 }
 
 int fg_reset_f64(const fg_params* p, const fg_buffers* b, int scenario, int E, int N, int L, const uint8_t* mask,
                  uint64_t seed, uint32_t tick, uint32_t env_offset, void* stream) {
-    return reset_impl<double>(p, b, scenario, E, N, L, mask, seed, tick, env_offset, stream);
+    return reset_impl<double>(p, b, scenario, E, N, L, mask, seed, tick, env_offset, stream, nullptr);
+}
+
+int fg_reset_targets_f64(const fg_params* p, const fg_buffers* b, int scenario, int E, int N, int L, const uint8_t* mask,
+                         uint64_t seed, uint32_t tick, uint32_t env_offset, void* stream, const fg_targets* t) {
+    return reset_impl<double>(p, b, scenario, E, N, L, mask, seed, tick, env_offset, stream, t);
 }
 
 int fg_random_actions_f64(void* act, int E, int N, uint64_t seed, uint32_t tick, uint32_t env_offset,

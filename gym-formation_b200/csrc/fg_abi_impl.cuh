@@ -241,6 +241,30 @@ int fill_args(fg::KArgs<T>& a, const fg_params* p, const fg_buffers* b, int scen
     return FG_OK;
 }
 
+// Target bank (fg_targets): validated before anything else (no device call on a bad argument); tg == NULL = no bank.
+template <typename T>
+int check_targets(const fg_targets* tg, int scenario, const char* who) {
+    typedef typename fg::Ops<T>::R2 R2;
+    if (!tg) return FG_OK;
+    if (scenario != FG_SCENARIO_HD)
+        return fail(FG_ERR_ARG, "%s: target banks are defined for formation_hd_env only", who);
+    if (tg->count < 1) return fail(FG_ERR_ARG, "%s: fg_targets.count must be >= 1", who);
+    if (!tg->shapes) return fail(FG_ERR_ARG, "%s: fg_targets.shapes must be non-null", who);
+    if (((uintptr_t)tg->shapes % sizeof(R2)) != 0 || ((uintptr_t)tg->vels % sizeof(R2)) != 0)
+        return fail(FG_ERR_ARG, "%s: fg_targets.shapes / vels must be 8-byte (fp32) / 16-byte (fp64) aligned", who);
+    if (((uintptr_t)tg->index % sizeof(int32_t)) != 0)
+        return fail(FG_ERR_ARG, "%s: fg_targets.index must be 4-byte aligned", who);
+    return FG_OK;
+}
+
+template <typename T>
+void set_targets(fg::KArgs<T>& a, const fg_targets* tg) {
+    typedef typename fg::Ops<T>::R2 R2;
+    if (!tg) return;                                                // fill_args left the bank empty (count 0)
+    a.tgt_shape = (const R2*)tg->shapes; a.tgt_vel = (const R2*)tg->vels;
+    a.tgt_index = tg->index; a.tgt_count = tg->count;
+}
+
 template <typename T>
 size_t smem_bytes(const fg::KArgs<T>& a, int scenario, bool het) {
     typedef typename fg::Ops<T>::R2 R2;
@@ -280,8 +304,8 @@ size_t fast_pairs_bytes(const fg::KArgs<T>& a) {
     return (8 * (size_t)a.EPC * NP + (size_t)a.EPC * 32) * sizeof(float) + 2 * (size_t)a.EPC * sizeof(unsigned) + 16;
 }
 
-template <typename T, int SCN, bool PHYS, bool OBSREW, bool HET, int OM, bool FP>
-int launch_one(const fg::KArgs<T>& a, size_t smem, cudaStream_t st) {
+template <typename T, int SCN, bool PHYS, bool OBSREW, bool HET, int OM, bool FP, bool TGT>
+int launch_one_tgt(const fg::KArgs<T>& a, size_t smem, cudaStream_t st) {
     const int grid = (a.E + a.EPC - 1) / a.EPC;
     fg::KArgs<T> b = a;
     if (FP) {
@@ -297,13 +321,21 @@ int launch_one(const fg::KArgs<T>& a, size_t smem, cudaStream_t st) {
         b.cells = 0;
     }
     {
-        cudaError_t e1 = ensure_dyn_smem<fg::k_step<T, SCN, PHYS, OBSREW, HET, OM, FP>>(smem);
+        cudaError_t e1 = ensure_dyn_smem<fg::k_step<T, SCN, PHYS, OBSREW, HET, OM, FP, TGT>>(smem);
         if (e1 != cudaSuccess) return fail(FG_ERR_CUDA, "cudaFuncSetAttribute failed: %s", cudaGetErrorString(e1));
     }
-    fg::k_step<T, SCN, PHYS, OBSREW, HET, OM, FP><<<grid, fg::kBlock, smem, st>>>(b);
+    fg::k_step<T, SCN, PHYS, OBSREW, HET, OM, FP, TGT><<<grid, fg::kBlock, smem, st>>>(b);
     cudaError_t err = cudaGetLastError();
     if (err != cudaSuccess) return fail(FG_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(err));
     return FG_OK;
+}
+
+// formation_hd_env steps with a target bank take the TGT instantiation of the same kernel
+template <typename T, int SCN, bool PHYS, bool OBSREW, bool HET, int OM, bool FP>
+int launch_one(const fg::KArgs<T>& a, size_t smem, cudaStream_t st) {
+    if constexpr (SCN == fg::kScnHD && PHYS && OBSREW)
+        if (a.tgt_count > 0) return launch_one_tgt<T, SCN, PHYS, OBSREW, HET, OM, FP, true>(a, smem, st);
+    return launch_one_tgt<T, SCN, PHYS, OBSREW, HET, OM, FP, false>(a, smem, st);
 }
 
 // Fast pair loops (fg_pairs.cuh): fp32, formation_hd_env, uniform agents, 32 <= N (a warp spans <= 2 envs).
@@ -366,7 +398,7 @@ int launch_obstacle(const fg::KArgs<T>& a, void* stream) {
 // observation-span image per warp).  Computed once per instantiation; all GPUs of a box are alike.
 struct WarpGeom { int ctas[4]; int best; int sms; };      // index: log2(w), w = 1, 2, 4, 8
 
-template <typename T, int N, bool WOBS, int SCN, bool STD, int POL = 0>
+template <typename T, int N, bool WOBS, int SCN, bool STD, int POL = 0, bool TGT = false>
 const WarpGeom& warp_geom() {
     static const WarpGeom geom = [] {
         typedef fg::WarpLayout<T, N, WOBS> LY;
@@ -380,10 +412,10 @@ const WarpGeom& warp_geom() {
             const size_t smem = (size_t)w * LY::stride;
             g_.ctas[l] = 0;
             if (smem > 227 * 1024 || w > LY::MAXW) continue;
-            if (cudaFuncSetAttribute(fg::k_hd_warp<T, N, WOBS, SCN, STD, POL>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+            if (cudaFuncSetAttribute(fg::k_hd_warp<T, N, WOBS, SCN, STD, POL, TGT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                      (int)smem) != cudaSuccess) { cudaGetLastError(); continue; }
             int ctas = 0;
-            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas, fg::k_hd_warp<T, N, WOBS, SCN, STD, POL>, 32 * w, smem)
+            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas, fg::k_hd_warp<T, N, WOBS, SCN, STD, POL, TGT>, 32 * w, smem)
                 != cudaSuccess) { cudaGetLastError(); continue; }
             g_.ctas[l] = ctas;
             if (ctas * w > best_res) { best_res = ctas * w; g_.best = l; }
@@ -391,24 +423,24 @@ const WarpGeom& warp_geom() {
         // the probing above left the limit at the SMALLEST footprint, and a limit below the launch's request makes
         // the launch fail (also under the 48 KB default): restore the default-or-larger value; launches raise it
         // further through ensure_dyn_smem when they need more than 48 KB
-        cudaFuncSetAttribute(fg::k_hd_warp<T, N, WOBS, SCN, STD, POL>, cudaFuncAttributeMaxDynamicSharedMemorySize, 48 * 1024);
+        cudaFuncSetAttribute(fg::k_hd_warp<T, N, WOBS, SCN, STD, POL, TGT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 48 * 1024);
         cudaGetLastError();
         return g_;
     }();
     return geom;
 }
 
-template <typename T, int N, bool WOBS, int SCN, bool STD, int POL = 0>
-int launch_warp_n(const fg::KArgs<T>& a, cudaStream_t st) {
+template <typename T, int N, bool WOBS, int SCN, bool STD, int POL = 0, bool TGT = false>
+int launch_warp_tgt(const fg::KArgs<T>& a, cudaStream_t st) {
     typedef fg::WarpLayout<T, N, WOBS> LY;
-    const WarpGeom& gm = warp_geom<T, N, WOBS, SCN, STD, POL>();
+    const WarpGeom& gm = warp_geom<T, N, WOBS, SCN, STD, POL, TGT>();
     const int spans = (a.E + LY::EPW - 1) / LY::EPW;
     int l = gm.best;
     while (l > 0 && (spans >> l) < 2 * gm.sms) --l;                // small batches: spread over the SMs
     if (gm.ctas[l] < 1) return fail(FG_ERR_CUDA, "k_hd_warp does not fit on this device%s");
     const int w = 1 << l;
     const size_t smem = (size_t)w * LY::stride;
-    cudaError_t err = ensure_dyn_smem<fg::k_hd_warp<T, N, WOBS, SCN, STD, POL>>(smem);
+    cudaError_t err = ensure_dyn_smem<fg::k_hd_warp<T, N, WOBS, SCN, STD, POL, TGT>>(smem);
     if (err != cudaSuccess) return fail(FG_ERR_CUDA, "cudaFuncSetAttribute failed: %s", cudaGetErrorString(err));
     // persistent warps: at most one resident wave; each warp walks spans gw, gw + nwarps, ...
     int grid = (spans + w - 1) / w;
@@ -416,10 +448,18 @@ int launch_warp_n(const fg::KArgs<T>& a, cudaStream_t st) {
     wave *= std::max(1, fgabi::switches().waves.load(std::memory_order_relaxed));
     if (grid > wave) grid = wave;
     if ((grid * w) & 1) ++grid;                                    // even warp count (16-byte phase, fg_warp.cuh)
-    fg::k_hd_warp<T, N, WOBS, SCN, STD, POL><<<grid, 32 * w, smem, st>>>(a);
+    fg::k_hd_warp<T, N, WOBS, SCN, STD, POL, TGT><<<grid, 32 * w, smem, st>>>(a);
     err = cudaGetLastError();
     if (err != cudaSuccess) return fail(FG_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(err));
     return FG_OK;
+}
+
+// formation_hd_env runs with a target bank take the TGT instantiation of the same kernel
+template <typename T, int N, bool WOBS, int SCN, bool STD, int POL = 0>
+int launch_warp_n(const fg::KArgs<T>& a, cudaStream_t st) {
+    if constexpr (SCN == fg::kScnHD)
+        if (a.tgt_count > 0) return launch_warp_tgt<T, N, WOBS, SCN, STD, POL, true>(a, st);
+    return launch_warp_tgt<T, N, WOBS, SCN, STD, POL, false>(a, st);
 }
 
 template <typename T, int N, int SCN = fg::kScnHD>
@@ -508,11 +548,14 @@ int obs_reward_impl(const fg_params* p, const fg_buffers* b, int scenario, int E
 template <typename T>
 int step_fused_impl(const fg_params* p, const fg_buffers* b, int scenario, int E, int N, int L, int n_steps,
                     int random_actions, int auto_reset, uint64_t seed, uint32_t tick, uint32_t env_offset,
-                    void* stream) {
+                    void* stream, const fg_targets* tg) {
     NvtxRange nvtx_("fg_step_fused");
-    fg::KArgs<T> a;
-    int rc = fill_args<T>(a, p, b, scenario, E, N, L, seed, tick, env_offset);
+    int rc = check_targets<T>(tg, scenario, "fg_step_fused_targets");
     if (rc) return rc;
+    fg::KArgs<T> a;
+    rc = fill_args<T>(a, p, b, scenario, E, N, L, seed, tick, env_offset);
+    if (rc) return rc;
+    set_targets<T>(a, tg);
     if (!b->pos || !b->vel || !b->reward || !b->done || !b->step)
         return fail(FG_ERR_ARG, "fg_step_fused: pos/vel/reward/done/step must be non-null%s");
     if (!random_actions && !b->act) return fail(FG_ERR_ARG, "fg_step_fused: act is null and random_actions == 0%s");
@@ -562,11 +605,14 @@ int step_fused_impl(const fg_params* p, const fg_buffers* b, int scenario, int E
 
 template <typename T>
 int reset_impl(const fg_params* p, const fg_buffers* b, int scenario, int E, int N, int L, const uint8_t* mask,
-               uint64_t seed, uint32_t tick, uint32_t env_offset, void* stream) {
+               uint64_t seed, uint32_t tick, uint32_t env_offset, void* stream, const fg_targets* tg) {
     NvtxRange nvtx_("fg_reset");
-    fg::KArgs<T> a;
-    int rc = fill_args<T>(a, p, b, scenario, E, N, L, seed, tick, env_offset);
+    int rc = check_targets<T>(tg, scenario, "fg_reset_targets");
     if (rc) return rc;
+    fg::KArgs<T> a;
+    rc = fill_args<T>(a, p, b, scenario, E, N, L, seed, tick, env_offset);
+    if (rc) return rc;
+    set_targets<T>(a, tg);
     if (!b->pos || !b->vel) return fail(FG_ERR_ARG, "fg_reset: pos/vel must be non-null%s");
     if (scenario == FG_SCENARIO_HD && (!b->ideal_shape || !b->ideal_vel))
         return fail(FG_ERR_ARG, "fg_reset(hd): ideal_shape/ideal_vel must be non-null%s");

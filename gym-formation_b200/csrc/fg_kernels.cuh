@@ -77,7 +77,24 @@ template <typename T> struct KArgs {
     uint8_t* nan_flag;               // (opt) [E]: set to 1 (never cleared) when the env holds a non-finite position (Q9)
     T pol_mult[8];                   // fused device controller (fg_warp.cuh, POL): log(M)/log(n) per BFS layer, top first
     WallT<T> walls[kMaxWalls];
+    // formation_hd_env target bank (fg_targets; read only by the reset blocks): tgt_count = K tasks, 0 = no bank
+    const R2* tgt_shape;             // [K,N] raw shapes, replacing the kResetLandmark draw
+    const R2* tgt_vel;               // (opt) [K] ideal velocities, replacing the kResetIdealVel draw
+    const int32_t* tgt_index;        // (opt) [E] task per env; out of [0, K) = draw
+    int tgt_count;
 };
+
+// Task of env e (global id ge) at a reset with tick tk: tgt_index[e] when it names an entry of the bank, else
+// drawn uniformly from Philox.  Only called when tgt_count > 0.
+template <typename T>
+__device__ __forceinline__ uint32_t target_task(const KArgs<T>& a, int e, uint32_t ge, uint32_t tk) {
+    const uint32_t K = (uint32_t)a.tgt_count;
+    if (a.tgt_index) {
+        const int32_t k = a.tgt_index[e];
+        if (k >= 0 && (uint32_t)k < K) return (uint32_t)k;
+    }
+    return __umulhi(philox(a.seed, ge, 0u, tk, kResetTarget).x, K);
+}
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
     return (uint32_t)__cvta_generic_to_shared(p);
@@ -199,7 +216,9 @@ __device__ __forceinline__ void wall_force(const WallT<T>& w, T px, T py, T size
 // shared memory, the whole tile leaves as one bulk store.
 // FP: fast pair loops of fg_pairs.cuh (fp32, hd, uniform agents, N >= 32): structure-of-arrays partner
 // data, packed FFMA2/FADD2/FMUL2 arithmetic, group filters, warp-shuffle centroid and reductions.
-template <typename T, int SCN, bool PHYS, bool OBSREW, bool HET, int OM, bool FP>
+// TGT: formation_hd_env with a target bank (KArgs::tgt_*).  Its own instantiation, so that the reset block of the
+// product kernels -- and with it their register allocation -- is the same as without the feature.
+template <typename T, int SCN, bool PHYS, bool OBSREW, bool HET, int OM, bool FP, bool TGT = false>
 __global__ void __launch_bounds__(kBlock, (OM == 3 && SCN == kScnBasic) ? 5 : (OM == 2 || OM == 3 || FP) ? 4 : 3) k_step(const __grid_constant__ KArgs<T> a) {
     typedef Ops<T> O;
     typedef typename O::R2 R2;
@@ -1043,11 +1062,17 @@ __global__ void __launch_bounds__(kBlock, (OM == 3 && SCN == kScnBasic) ? 5 : (O
                     if (SCN == kScnHD) {
                         U4 q = philox(a.seed, ge, (uint32_t)i, tk, kResetLandmark);
                         lraw = O::make(uniform_pm1<T>(q.x), uniform_pm1<T>(q.y));
+                        uint32_t kt = 0;
+                        if constexpr (TGT) {                  // target bank: the task's raw shape
+                            kt = target_task<T>(a, e, ge, tk);
+                            lraw = a.tgt_shape[(size_t)kt * N + i];
+                        }
                         s_old[t] = lraw;                      // scratch: s_old is dead after the physics
                         if (a.lm) a.lm[g] = lraw;
                         if (i == 0) {
                             U4 w = philox(a.seed, ge, 0u, tk, kResetIdealVel);
                             R2 iv = O::make(uniform_pm1<T>(w.x), uniform_pm1<T>(w.y));
+                            if (TGT && a.tgt_vel) iv = a.tgt_vel[kt];
                             s_iv[le] = iv; a.ivel[e] = iv;
                         }
                     }
@@ -1365,10 +1390,17 @@ __global__ void k_reset(const __grid_constant__ KArgs<T> a, const uint8_t* __res
         a.vel[g] = zero;
         if (a.comm) a.comm[g] = zero;
     }
+    // formation_hd_env with a target bank: the task's raw shape replaces the landmark draws (same centring below)
+    uint32_t kt = 0;
+    const R2* bank = nullptr;
+    if (SCN == kScnHD && a.tgt_count > 0) {
+        kt = target_task<T>(a, e, ge, tick0);
+        bank = a.tgt_shape + (size_t)kt * N;
+    }
     T sx = 0, sy = 0;
     for (int k = 0; k < L; ++k) {
         U4 r = philox(a.seed, ge, (uint32_t)k, tick0, kResetLandmark);
-        R2 l = O::make(uniform_pm1<T>(r.x), uniform_pm1<T>(r.y));
+        R2 l = bank ? bank[k] : O::make(uniform_pm1<T>(r.x), uniform_pm1<T>(r.y));
         sx = O::add(sx, l.x); sy = O::add(sy, l.y);
         if (a.lm) a.lm[(size_t)e * L + k] = l;
     }
@@ -1376,11 +1408,11 @@ __global__ void k_reset(const __grid_constant__ KArgs<T> a, const uint8_t* __res
         T mx = O::div(sx, (T)N), my = O::div(sy, (T)N);
         for (int k = 0; k < N; ++k) {
             U4 r = philox(a.seed, ge, (uint32_t)k, tick0, kResetLandmark);
-            a.shape[(size_t)e * N + k] =
-                O::make(O::sub(uniform_pm1<T>(r.x), mx), O::sub(uniform_pm1<T>(r.y), my));
+            R2 l = bank ? bank[k] : O::make(uniform_pm1<T>(r.x), uniform_pm1<T>(r.y));
+            a.shape[(size_t)e * N + k] = O::make(O::sub(l.x, mx), O::sub(l.y, my));
         }
         U4 w = philox(a.seed, ge, 0u, tick0, kResetIdealVel);
-        a.ivel[e] = O::make(uniform_pm1<T>(w.x), uniform_pm1<T>(w.y));
+        a.ivel[e] = (bank && a.tgt_vel) ? a.tgt_vel[kt] : O::make(uniform_pm1<T>(w.x), uniform_pm1<T>(w.y));
     }
     if (a.step) a.step[e] = 0;
     if (a.ep_return) a.ep_return[e] = (T)0;

@@ -83,7 +83,8 @@ enum Purpose : uint32_t {
     kResetIdealVel = 2,  // .xy -> ideal velocity         (formation_hd_env.py:95)
     kUNoise = 3,         // Box-Muller pair -> motor noise (core.py:232-233)
     kCNoise = 4,         // Box-Muller pair -> comm noise  (core.py:284-285)
-    kAction = 5          // .xy -> random-policy action    (test.py:20)
+    kAction = 5,         // .xy -> random-policy action    (test.py:20)
+    kResetTarget = 6     // .x  -> task of a target bank (fg_targets), umulhi(x, K); agent = 0
 };
 
 __host__ __device__ __forceinline__ void philox_mulhilo(uint32_t a, uint32_t b, uint32_t* hi, uint32_t* lo) {

@@ -24,6 +24,8 @@ EXPORTS = [
     "fg_step_fused", "fg_step_fused_f64", "fg_reset", "fg_reset_f64",
     "fg_random_actions", "fg_random_actions_f64", "fg_fp32_probe", "fg_write_probe", "fg_policy_bfs", "fg_policy_bfs_f64",
     "fg_obs_to_host", "fg_pair_distances", "fg_pair_distances_f64", "fg_step_policy", "fg_step_policy_f64",
+    "fg_reset_targets", "fg_reset_targets_f64", "fg_step_fused_targets", "fg_step_fused_targets_f64",
+    "fg_step_policy_targets", "fg_step_policy_targets_f64",
 ]
 
 
@@ -65,6 +67,12 @@ class fg_buffers(C.Structure):
     ]
 
 
+class fg_targets(C.Structure):
+    """Target bank of formation_hd_env (the ``*_targets`` entry points): K raw shapes [K,N,2], optional ideal
+    velocities [K,2] and an optional per-env task index [E] (out of [0, K) = draw)."""
+    _fields_ = [("shapes", C.c_void_p), ("vels", C.c_void_p), ("index", C.c_void_p), ("count", C.c_int32)]
+
+
 _lib = None
 
 
@@ -101,6 +109,12 @@ def load():
             [P(fg_params), P(fg_buffers), I, I, I, I, I, I, I, U64, U32, U32, VP]
         getattr(lib, "fg_reset" + sfx).argtypes = \
             [P(fg_params), P(fg_buffers), I, I, I, I, VP, U64, U32, U32, VP]
+        getattr(lib, "fg_step_fused_targets" + sfx).argtypes = \
+            [P(fg_params), P(fg_buffers), I, I, I, I, I, I, I, U64, U32, U32, VP, P(fg_targets)]
+        getattr(lib, "fg_step_policy_targets" + sfx).argtypes = \
+            [P(fg_params), P(fg_buffers), I, I, I, I, I, I, I, U64, U32, U32, VP, P(fg_targets)]
+        getattr(lib, "fg_reset_targets" + sfx).argtypes = \
+            [P(fg_params), P(fg_buffers), I, I, I, I, VP, U64, U32, U32, VP, P(fg_targets)]
         getattr(lib, "fg_random_actions" + sfx).argtypes = [VP, I, I, U64, U32, U32, VP, VP]
         getattr(lib, "fg_policy_bfs" + sfx).argtypes = [VP, VP, VP, VP, I, I, I, VP]
         getattr(lib, "fg_pair_distances" + sfx).argtypes = [VP, VP, I, I, VP, VP, VP, VP, VP]

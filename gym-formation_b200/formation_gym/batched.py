@@ -52,6 +52,36 @@ def obs_dim(scenario, num_agents, num_landmarks=3, num_obs=3):
     return 4 + 2 * num_landmarks + 4 * (num_agents - 1)
 
 
+def _target_bank(scenario, E, N, shapes, vels, index):
+    """Validate a formation_hd_env target bank (include/formation_gym_b200.h fg_targets) on the host: None, or
+    (shapes [K,N,2], vels [K,2] or None, index [E] int32 or None) as CPU tensors.  Every reset -- reset() and the
+    in-kernel auto-reset -- gives env e the task k = index[e] when that is in [0, K), else a uniform draw:
+    ideal_shape = shapes[k] centred as reset_world centres its landmarks (formation_hd_env.py:93), ideal_vel =
+    vels[k] (drawn as without a bank when vels is None)."""
+    if shapes is None:
+        if vels is not None or index is not None:
+            raise ValueError("target_vels / target_index need target_shapes")
+        return None
+    if scenario != "formation_hd_env":
+        raise ValueError("target banks are defined for formation_hd_env only (got %r)" % (scenario,))
+    shapes = torch.as_tensor(shapes).detach().cpu().to(torch.float64)
+    if shapes.dim() != 3 or shapes.shape[0] < 1 or tuple(shapes.shape[1:]) != (N, 2):
+        raise ValueError("target_shapes must have shape (K, %d, 2) with K >= 1, got %s" % (N, tuple(shapes.shape)))
+    K = int(shapes.shape[0])
+    if vels is not None:
+        vels = torch.as_tensor(vels).detach().cpu().to(torch.float64)
+        if tuple(vels.shape) != (K, 2):
+            raise ValueError("target_vels must have shape (%d, 2), got %s" % (K, tuple(vels.shape)))
+    if index is not None:
+        index = torch.as_tensor(index).detach().cpu()
+        if index.dtype.is_floating_point or index.dtype.is_complex or index.dtype == torch.bool:
+            raise ValueError("target_index must hold integers, got %s" % index.dtype)
+        if tuple(index.shape) != (E,):
+            raise ValueError("target_index must have shape (%d,), got %s" % (E, tuple(index.shape)))
+        index = index.to(torch.int64).clamp(-1, 2 ** 31 - 1).to(torch.int32)   # out of range stays out of range
+    return shapes, vels, index
+
+
 class BatchedFormationEnv:
     """E independent envs of N agents on one GPU.
 
@@ -67,11 +97,13 @@ class BatchedFormationEnv:
                  agent_mass=None, agent_sizes=None, agent_accel=None, agent_max_speed=None,
                  walls=(), dt=0.1, damping=0.25, contact_force=1e2, contact_margin=1e-3,
                  sensitivity=5.0, num_obs=3, obs_range=0.7, num_obstacles=3, obstacle_size=0.15,
-                 obstacle_mass=1.0, obstacle_floor=-2.2, obstacle_fall_vy=-1.0):
+                 obstacle_mass=1.0, obstacle_floor=-2.2, obstacle_fall_vy=-1.0, target_shapes=None,
+                 target_vels=None, target_index=None):
         if scenario not in SCENARIOS:
             raise ValueError("unknown scenario %r (supported: %s)" % (scenario, sorted(SCENARIOS)))
         if dtype not in (torch.float32, torch.float64):
             raise ValueError("dtype must be torch.float32 or torch.float64")
+        bank = _target_bank(scenario, int(num_envs), int(num_agents), target_shapes, target_vels, target_index)
         self._lib = nat.load()                      # raises when the CUDA extension is missing
         self._fns = {}
         if not torch.cuda.is_available():
@@ -164,6 +196,7 @@ class BatchedFormationEnv:
         self._ext_bufs = None
         self._bfs_primed = 0          # fan-out n while self.actions holds the controller's output for the current state (step_bfs)
         self._bufs = self._make_buffers()
+        self._set_target_bank(bank)
 
     # ------------------------------------------------------------------ plumbing
     def _make_buffers(self, act=None, obs="default"):
@@ -184,6 +217,32 @@ class BatchedFormationEnv:
         b.tick_dev = nat.ptr(self._tick_dev) if self._device_tick else None
         b.nan_flag = nat.ptr(self.nan_flag)
         return b
+
+    def _set_target_bank(self, bank):
+        """Device copies of a validated target bank (``_target_bank``) and the fg_targets block that points at them."""
+        self.target_shapes = self.target_vels = self.target_index = None
+        self._targets = None
+        if bank is None:
+            return
+        shapes, vels, index = bank
+        kw = dict(device=self.device, dtype=self.dtype)
+        if index is None:
+            index = torch.full((self.E,), -1, dtype=torch.int32)            # every reset draws
+        # kept alive here: the struct holds raw pointers.  target_index may be rewritten in place between calls (a
+        # curriculum); the next reset reads it in stream order.
+        self.target_shapes = shapes.to(**kw).contiguous()
+        self.target_vels = None if vels is None else vels.to(**kw).contiguous()
+        self.target_index = index.to(device=self.device).contiguous()
+        t = nat.fg_targets()
+        t.shapes, t.vels = nat.ptr(self.target_shapes), nat.ptr(self.target_vels)
+        t.index, t.count = nat.ptr(self.target_index), int(shapes.shape[0])
+        self._targets = t
+
+    def _call(self, name, *args):
+        """Entry point ``name`` (``name + '_targets'`` with the target bank appended when one is set)."""
+        if self._targets is not None:
+            return self._fn(name + "_targets")(*args, C.byref(self._targets))
+        return self._fn(name)(*args)
 
     def _stream(self):
         # raw cudaStream_t of torch's CURRENT stream on this device (what torch.cuda.current_stream(dev).cuda_stream
@@ -248,9 +307,8 @@ class BatchedFormationEnv:
                 raise ValueError("mask must have shape (E,)")
         self._bfs_primed = 0
         with self._on_device():
-            rc = self._fn("fg_reset")(C.byref(self.params), C.byref(self._bufs), self.scn, self.E, self.N,
-                                      self.L, nat.ptr(m), self.seed_value, self._next_tick(),
-                                      self.env_offset, self._stream())
+            rc = self._call("fg_reset", C.byref(self.params), C.byref(self._bufs), self.scn, self.E, self.N,
+                            self.L, nat.ptr(m), self.seed_value, self._next_tick(), self.env_offset, self._stream())
             nat.check(rc, "fg_reset")
             self.launches += 1
         if mask is None:
@@ -359,9 +417,9 @@ class BatchedFormationEnv:
             self.bfs_actions(n)
         n_steps = int(n_steps)
         with self._on_device():
-            rc = self._fn("fg_step_policy")(C.byref(self.params), C.byref(self._bufs), self.scn, self.E, self.N,
-                                            self.L, n_steps, n, int(self.auto_reset), self.seed_value,
-                                            self._next_tick(n_steps, True), self.env_offset, self._stream())
+            rc = self._call("fg_step_policy", C.byref(self.params), C.byref(self._bufs), self.scn, self.E, self.N,
+                            self.L, n_steps, n, int(self.auto_reset), self.seed_value,
+                            self._next_tick(n_steps, True), self.env_offset, self._stream())
             nat.check(rc, "fg_step_policy")
             self.launches += 1                 # (calls; a configuration without a fused instantiation launches 2 per step)
         self._bfs_primed = n
@@ -376,10 +434,9 @@ class BatchedFormationEnv:
     def _launch_fused(self, bufs, n_steps, random_actions):
         self._bfs_primed = 0
         with self._on_device():
-            rc = self._fn("fg_step_fused")(C.byref(self.params), C.byref(bufs), self.scn, self.E, self.N,
-                                           self.L, n_steps, random_actions, int(self.auto_reset),
-                                           self.seed_value, self._next_tick(n_steps, True), self.env_offset,
-                                           self._stream())
+            rc = self._call("fg_step_fused", C.byref(self.params), C.byref(bufs), self.scn, self.E, self.N,
+                            self.L, n_steps, random_actions, int(self.auto_reset), self.seed_value,
+                            self._next_tick(n_steps, True), self.env_offset, self._stream())
             nat.check(rc, "fg_step_fused")
             self.launches += 1
 
@@ -480,7 +537,7 @@ class BatchedFormationEnv:
     def state_dict(self):
         sd = {k: getattr(self, k).clone() for k in
               ("pos", "vel", "comm", "step_count", "ep_return", "ep_collisions", "stats", "nan_flag")}
-        for k in ("landmarks", "landmark_vel", "ideal_shape", "ideal_vel"):
+        for k in ("landmarks", "landmark_vel", "ideal_shape", "ideal_vel", "target_index"):
             if getattr(self, k) is not None:
                 sd[k] = getattr(self, k).clone()
         sd["rng"] = {"seed": self.seed_value, "env_offset": self.env_offset,

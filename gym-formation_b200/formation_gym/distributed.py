@@ -76,9 +76,15 @@ def summarize(stats):
 
 
 def make_sharded_env(scenario, num_envs_total, num_agents, episode_length=None, **kwargs):
-    """This rank's shard of a ``num_envs_total``-env job (rank/world from torch.distributed)."""
+    """This rank's shard of a ``num_envs_total``-env job (rank/world from torch.distributed).  A ``target_index`` of
+    the whole job ([num_envs_total]) is sliced to the shard; target banks are shared by all ranks."""
     from .batched import BatchedFormationEnv
     rank = dist.get_rank() if dist.is_initialized() else 0
     world = dist.get_world_size() if dist.is_initialized() else 1
     lo, hi = shard_range(num_envs_total, rank, world)
+    if kwargs.get("target_index") is not None:
+        ti = torch.as_tensor(kwargs["target_index"])
+        if tuple(ti.shape) != (int(num_envs_total),):
+            raise ValueError("target_index must have shape (%d,) (one task per env of the job)" % int(num_envs_total))
+        kwargs["target_index"] = ti[lo:hi]
     return BatchedFormationEnv(scenario, hi - lo, num_agents, episode_length, env_offset=lo, **kwargs)

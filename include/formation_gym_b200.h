@@ -157,6 +157,21 @@ typedef struct fg_buffers {
                                   fg_step_fused and fg_obs_reward; costs no traffic while every env is finite. */
 } fg_buffers;
 
+/* Target bank of formation_hd_env (the *_targets entry points): `count` = K formation tasks, DEVICE arrays in the entry
+ * point's real type.  At every reset of env e -- fg_reset_targets and the in-kernel auto-reset alike -- the env takes
+ * task k = index[e] when index is given and 0 <= index[e] < K, else k drawn uniformly from Philox (purpose 6,
+ * umulhi(x, K)).  shapes[k] replaces the uniform landmark draw of reset_world (formation_hd_env.py:89) and is centred
+ * with the same arithmetic (ideal_shape = raw - mean(raw), :93; tracked landmarks receive the raw entry); vels[k], when
+ * given, replaces the ideal_vel draw (:95).  Positions, velocities, comm, step and the episode accumulators take the
+ * same draws as without a bank.  Scenario.generate_shape (formation_hd_env.py:123-139) gives hierarchical entries. */
+typedef struct fg_targets {
+    const void* shapes;        /* [K,N,2] raw target shapes */
+    const void* vels;          /* (opt) [K,2] target ideal velocities; NULL = drawn as without a bank */
+    const int32_t* index;      /* (opt) [E] task per env, read at each reset (a curriculum may rewrite it between
+                                  calls, in stream order); an entry outside [0, K) -- e.g. -1 -- means "draw" */
+    int32_t count;             /* K >= 1 */
+} fg_targets;
+
 int fg_abi_version(void);
 const char* fg_last_error(void);
 
@@ -237,6 +252,24 @@ int fg_reset_f64(const fg_params* p, const fg_buffers* b, int scenario, int E, i
                  const uint8_t* mask, uint64_t seed, uint32_t tick, uint32_t env_offset,
                  void* stream);
 
+/* fg_reset / fg_step_fused / fg_step_policy with a target bank (fg_targets above): every reset the call performs --
+ * the masked reset, or the auto-reset of an env whose episode ends -- takes the env's task from the bank.  Everything
+ * else is the plain entry point's; t == NULL is exactly the plain entry point (which is this call with NULL).
+ * FG_ERR_ARG unless scenario == FG_SCENARIO_HD, t->count >= 1, t->shapes != NULL and shapes / vels are 8-byte (fp32)
+ * / 16-byte (fp64) aligned (index: 4-byte). */
+int fg_reset_targets(const fg_params* p, const fg_buffers* b, int scenario, int E, int N, int L,
+                     const uint8_t* mask, uint64_t seed, uint32_t tick, uint32_t env_offset, void* stream,
+                     const fg_targets* t);
+int fg_reset_targets_f64(const fg_params* p, const fg_buffers* b, int scenario, int E, int N, int L,
+                         const uint8_t* mask, uint64_t seed, uint32_t tick, uint32_t env_offset, void* stream,
+                         const fg_targets* t);
+int fg_step_fused_targets(const fg_params* p, const fg_buffers* b, int scenario, int E, int N, int L,
+                          int n_steps, int random_actions, int auto_reset,
+                          uint64_t seed, uint32_t tick, uint32_t env_offset, void* stream, const fg_targets* t);
+int fg_step_fused_targets_f64(const fg_params* p, const fg_buffers* b, int scenario, int E, int N, int L,
+                              int n_steps, int random_actions, int auto_reset,
+                              uint64_t seed, uint32_t tick, uint32_t env_offset, void* stream, const fg_targets* t);
+
 /* World.calculate_distances (formation_gym/core.py:156-180), the distance cache behind World.cache_dists, for every env:
  * ent_pos [E,M,2] entity positions in world.entities order (agents, then landmarks), ent_size [M] ->
  * dist_vect [E,M,M,2] (p_a - p_b above the diagonal, the negative below), dist_mag [E,M,M]
@@ -283,6 +316,15 @@ int fg_step_policy(const fg_params* p, const fg_buffers* b, int scenario, int E,
 int fg_step_policy_f64(const fg_params* p, const fg_buffers* b, int scenario, int E, int N, int L, int n_steps,
                        int num_agents_per_layer, int auto_reset, uint64_t seed, uint32_t tick, uint32_t env_offset,
                        void* stream);
+/* fg_step_policy whose auto-resets take the env's task from a target bank (fg_targets, see fg_reset_targets); the
+ * controller then steers towards the new task from the first step of the episode.  Same dispatch (one launch or two
+ * per step) as fg_step_policy. */
+int fg_step_policy_targets(const fg_params* p, const fg_buffers* b, int scenario, int E, int N, int L, int n_steps,
+                           int num_agents_per_layer, int auto_reset, uint64_t seed, uint32_t tick,
+                           uint32_t env_offset, void* stream, const fg_targets* t);
+int fg_step_policy_targets_f64(const fg_params* p, const fg_buffers* b, int scenario, int E, int N, int L,
+                               int n_steps, int num_agents_per_layer, int auto_reset, uint64_t seed, uint32_t tick,
+                               uint32_t env_offset, void* stream, const fg_targets* t);
 
 /* Diagnostics, not on the step path: FP32 pipe probes used by bench.py to MEASURE the FP32 peak the
  * large-N step+reward kernel is graded against (BASELINE.json north_star: "% of FP32 peak at 243
