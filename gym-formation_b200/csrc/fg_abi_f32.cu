@@ -107,14 +107,26 @@ int fg_step_fused(const fg_params* p, const fg_buffers* b, int scenario, int E, 
                   int random_actions, int auto_reset, uint64_t seed, uint32_t tick, uint32_t env_offset,
                   void* stream) {
     return step_fused_impl<float>(p, b, scenario, E, N, L, n_steps, random_actions, auto_reset, seed, tick,
-                                  env_offset, stream, nullptr);
+                                  env_offset, stream, nullptr, nullptr);
 }
 
 int fg_step_fused_targets(const fg_params* p, const fg_buffers* b, int scenario, int E, int N, int L, int n_steps,
                           int random_actions, int auto_reset, uint64_t seed, uint32_t tick, uint32_t env_offset,
                           void* stream, const fg_targets* t) {
     return step_fused_impl<float>(p, b, scenario, E, N, L, n_steps, random_actions, auto_reset, seed, tick,
-                                  env_offset, stream, t);
+                                  env_offset, stream, t, nullptr);
+}
+
+int fg_step_fused_final(const fg_params* p, const fg_buffers* b, int scenario, int E, int N, int L, int n_steps,
+                        int random_actions, int auto_reset, uint64_t seed, uint32_t tick, uint32_t env_offset,
+                        void* stream, const fg_targets* t, const fg_final* f) {
+    return step_fused_impl<float>(p, b, scenario, E, N, L, n_steps, random_actions, auto_reset, seed, tick,
+                                  env_offset, stream, t, f);
+}
+
+int fg_final_obs(const fg_params* p, const fg_final* f, const uint8_t* done, void* obs, int scenario, int E,
+                 int N, int L, void* stream) {
+    return final_obs_impl<float>(p, f, done, obs, scenario, E, N, L, stream);
 }
 
 int fg_reset(const fg_params* p, const fg_buffers* b, int scenario, int E, int N, int L, const uint8_t* mask,

@@ -265,6 +265,38 @@ void set_targets(fg::KArgs<T>& a, const fg_targets* tg) {
     a.tgt_index = tg->index; a.tgt_count = tg->count;
 }
 
+// Terminal block (fg_final): validated before anything else (no device call on a bad argument); f == NULL = no block.
+// step != 0: a step entry point (auto-reset on, one step per call: then the mask of written envs is the step's done).
+template <typename T>
+int check_final(const fg_final* f, const fg_params* p, int scenario, int auto_reset, int n_steps, bool step,
+                const char* who) {
+    typedef typename fg::Ops<T>::R2 R2;
+    if (!f) return FG_OK;
+    if (step && !auto_reset) return fail(FG_ERR_ARG, "%s: a terminal block needs auto_reset != 0", who);
+    if (step && n_steps != 1) return fail(FG_ERR_ARG, "%s: a terminal block needs n_steps == 1", who);
+    if (!f->pos || !f->vel) return fail(FG_ERR_ARG, "%s: fg_final.pos / vel must be non-null", who);
+    if (scenario == FG_SCENARIO_HD && (!f->ideal_shape || !f->ideal_vel))
+        return fail(FG_ERR_ARG, "%s: fg_final.ideal_shape / ideal_vel must be non-null for formation_hd_env", who);
+    if (scenario != FG_SCENARIO_HD && !f->landmarks)
+        return fail(FG_ERR_ARG, "%s: fg_final.landmarks must be non-null for this scenario", who);
+    if (p && !p->silent && !f->comm) return fail(FG_ERR_ARG, "%s: fg_final.comm must be non-null for non-silent agents", who);
+    const void* vec[] = {f->pos, f->vel, f->comm, f->ideal_shape, f->ideal_vel, f->landmarks};
+    for (const void* q : vec)
+        if (((uintptr_t)q % sizeof(R2)) != 0)
+            return fail(FG_ERR_ARG, "%s: fg_final arrays must be 8-byte (fp32) / 16-byte (fp64) aligned", who);
+    return FG_OK;
+}
+
+template <typename T>
+void set_final(fg::KArgs<T>& a, const fg_final* f, const fg_params* p, int scenario) {
+    typedef typename fg::Ops<T>::R2 R2;
+    if (!f) return;                                                 // fill_args left the block empty (fin_pos NULL)
+    a.fin_pos = (R2*)f->pos; a.fin_vel = (R2*)f->vel;
+    a.fin_comm = p->silent ? nullptr : (R2*)f->comm;
+    if (scenario == FG_SCENARIO_HD) { a.fin_shape = (R2*)f->ideal_shape; a.fin_ivel = (R2*)f->ideal_vel; }
+    else a.fin_lm = (R2*)f->landmarks;
+}
+
 template <typename T>
 size_t smem_bytes(const fg::KArgs<T>& a, int scenario, bool het) {
     typedef typename fg::Ops<T>::R2 R2;
@@ -304,8 +336,8 @@ size_t fast_pairs_bytes(const fg::KArgs<T>& a) {
     return (8 * (size_t)a.EPC * NP + (size_t)a.EPC * 32) * sizeof(float) + 2 * (size_t)a.EPC * sizeof(unsigned) + 16;
 }
 
-template <typename T, int SCN, bool PHYS, bool OBSREW, bool HET, int OM, bool FP, bool TGT>
-int launch_one_tgt(const fg::KArgs<T>& a, size_t smem, cudaStream_t st) {
+template <typename T, int SCN, bool PHYS, bool OBSREW, bool HET, int OM, bool FP, bool EXT>
+int launch_one_ext(const fg::KArgs<T>& a, size_t smem, cudaStream_t st) {
     const int grid = (a.E + a.EPC - 1) / a.EPC;
     fg::KArgs<T> b = a;
     if (FP) {
@@ -321,21 +353,21 @@ int launch_one_tgt(const fg::KArgs<T>& a, size_t smem, cudaStream_t st) {
         b.cells = 0;
     }
     {
-        cudaError_t e1 = ensure_dyn_smem<fg::k_step<T, SCN, PHYS, OBSREW, HET, OM, FP, TGT>>(smem);
+        cudaError_t e1 = ensure_dyn_smem<fg::k_step<T, SCN, PHYS, OBSREW, HET, OM, FP, EXT>>(smem);
         if (e1 != cudaSuccess) return fail(FG_ERR_CUDA, "cudaFuncSetAttribute failed: %s", cudaGetErrorString(e1));
     }
-    fg::k_step<T, SCN, PHYS, OBSREW, HET, OM, FP, TGT><<<grid, fg::kBlock, smem, st>>>(b);
+    fg::k_step<T, SCN, PHYS, OBSREW, HET, OM, FP, EXT><<<grid, fg::kBlock, smem, st>>>(b);
     cudaError_t err = cudaGetLastError();
     if (err != cudaSuccess) return fail(FG_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(err));
     return FG_OK;
 }
 
-// formation_hd_env steps with a target bank take the TGT instantiation of the same kernel
+// steps with a target bank or a terminal block, and fg_final_obs, take the EXT instantiation of the same kernel
 template <typename T, int SCN, bool PHYS, bool OBSREW, bool HET, int OM, bool FP>
 int launch_one(const fg::KArgs<T>& a, size_t smem, cudaStream_t st) {
-    if constexpr (SCN == fg::kScnHD && PHYS && OBSREW)
-        if (a.tgt_count > 0) return launch_one_tgt<T, SCN, PHYS, OBSREW, HET, OM, FP, true>(a, smem, st);
-    return launch_one_tgt<T, SCN, PHYS, OBSREW, HET, OM, FP, false>(a, smem, st);
+    if constexpr (OBSREW)
+        if (fg::reset_ext(a)) return launch_one_ext<T, SCN, PHYS, OBSREW, HET, OM, FP, true>(a, smem, st);
+    return launch_one_ext<T, SCN, PHYS, OBSREW, HET, OM, FP, false>(a, smem, st);
 }
 
 // Fast pair loops (fg_pairs.cuh): fp32, formation_hd_env, uniform agents, 32 <= N (a warp spans <= 2 envs).
@@ -374,8 +406,8 @@ int launch(const fg::KArgs<T>& a, int scenario, const fg_params* p, void* stream
 
 
 // formation_hd_obs_env (fg_obstacle.cuh)
-template <typename T, bool PHYS, bool OBSREW = true>
-int launch_obstacle(const fg::KArgs<T>& a, void* stream) {
+template <typename T, bool PHYS, bool OBSREW, bool EXT>
+int launch_obstacle_ext(const fg::KArgs<T>& a, void* stream) {
     typedef typename fg::Ops<T>::R2 R2;
     typedef typename fg::Ops<T>::Bits Bits;
     const size_t nA = (size_t)a.EPC * a.N;
@@ -383,14 +415,21 @@ int launch_obstacle(const fg::KArgs<T>& a, void* stream) {
                   + a.EPC * sizeof(Bits) + 3 * a.EPC * sizeof(int);
     smem = (smem + 15) & ~(size_t)15;
     {
-        cudaError_t e1 = ensure_dyn_smem<fg::k_step_obst<T, PHYS, OBSREW>>(smem);
+        cudaError_t e1 = ensure_dyn_smem<fg::k_step_obst<T, PHYS, OBSREW, EXT>>(smem);
         if (e1 != cudaSuccess) return fail(FG_ERR_CUDA, "cudaFuncSetAttribute failed: %s", cudaGetErrorString(e1));
     }
     const int grid = (a.E + a.EPC - 1) / a.EPC;
-    fg::k_step_obst<T, PHYS, OBSREW><<<grid, fg::kBlock, smem, (cudaStream_t)stream>>>(a);
+    fg::k_step_obst<T, PHYS, OBSREW, EXT><<<grid, fg::kBlock, smem, (cudaStream_t)stream>>>(a);
     cudaError_t err = cudaGetLastError();
     if (err != cudaSuccess) return fail(FG_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(err));
     return FG_OK;
+}
+
+template <typename T, bool PHYS, bool OBSREW = true>
+int launch_obstacle(const fg::KArgs<T>& a, void* stream) {
+    if constexpr (OBSREW)
+        if (fg::reset_ext(a)) return launch_obstacle_ext<T, PHYS, OBSREW, true>(a, stream);
+    return launch_obstacle_ext<T, PHYS, OBSREW, false>(a, stream);
 }
 
 // ---- warp-autonomous fast path (fg_warp.cuh) ----------------------------------------------------
@@ -398,7 +437,7 @@ int launch_obstacle(const fg::KArgs<T>& a, void* stream) {
 // observation-span image per warp).  Computed once per instantiation; all GPUs of a box are alike.
 struct WarpGeom { int ctas[4]; int best; int sms; };      // index: log2(w), w = 1, 2, 4, 8
 
-template <typename T, int N, bool WOBS, int SCN, bool STD, int POL = 0, bool TGT = false>
+template <typename T, int N, bool WOBS, int SCN, bool STD, int POL = 0, bool EXT = false>
 const WarpGeom& warp_geom() {
     static const WarpGeom geom = [] {
         typedef fg::WarpLayout<T, N, WOBS> LY;
@@ -412,10 +451,10 @@ const WarpGeom& warp_geom() {
             const size_t smem = (size_t)w * LY::stride;
             g_.ctas[l] = 0;
             if (smem > 227 * 1024 || w > LY::MAXW) continue;
-            if (cudaFuncSetAttribute(fg::k_hd_warp<T, N, WOBS, SCN, STD, POL, TGT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+            if (cudaFuncSetAttribute(fg::k_hd_warp<T, N, WOBS, SCN, STD, POL, EXT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                      (int)smem) != cudaSuccess) { cudaGetLastError(); continue; }
             int ctas = 0;
-            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas, fg::k_hd_warp<T, N, WOBS, SCN, STD, POL, TGT>, 32 * w, smem)
+            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas, fg::k_hd_warp<T, N, WOBS, SCN, STD, POL, EXT>, 32 * w, smem)
                 != cudaSuccess) { cudaGetLastError(); continue; }
             g_.ctas[l] = ctas;
             if (ctas * w > best_res) { best_res = ctas * w; g_.best = l; }
@@ -423,24 +462,24 @@ const WarpGeom& warp_geom() {
         // the probing above left the limit at the SMALLEST footprint, and a limit below the launch's request makes
         // the launch fail (also under the 48 KB default): restore the default-or-larger value; launches raise it
         // further through ensure_dyn_smem when they need more than 48 KB
-        cudaFuncSetAttribute(fg::k_hd_warp<T, N, WOBS, SCN, STD, POL, TGT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 48 * 1024);
+        cudaFuncSetAttribute(fg::k_hd_warp<T, N, WOBS, SCN, STD, POL, EXT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 48 * 1024);
         cudaGetLastError();
         return g_;
     }();
     return geom;
 }
 
-template <typename T, int N, bool WOBS, int SCN, bool STD, int POL = 0, bool TGT = false>
-int launch_warp_tgt(const fg::KArgs<T>& a, cudaStream_t st) {
+template <typename T, int N, bool WOBS, int SCN, bool STD, int POL = 0, bool EXT = false>
+int launch_warp_ext(const fg::KArgs<T>& a, cudaStream_t st) {
     typedef fg::WarpLayout<T, N, WOBS> LY;
-    const WarpGeom& gm = warp_geom<T, N, WOBS, SCN, STD, POL, TGT>();
+    const WarpGeom& gm = warp_geom<T, N, WOBS, SCN, STD, POL, EXT>();
     const int spans = (a.E + LY::EPW - 1) / LY::EPW;
     int l = gm.best;
     while (l > 0 && (spans >> l) < 2 * gm.sms) --l;                // small batches: spread over the SMs
     if (gm.ctas[l] < 1) return fail(FG_ERR_CUDA, "k_hd_warp does not fit on this device%s");
     const int w = 1 << l;
     const size_t smem = (size_t)w * LY::stride;
-    cudaError_t err = ensure_dyn_smem<fg::k_hd_warp<T, N, WOBS, SCN, STD, POL, TGT>>(smem);
+    cudaError_t err = ensure_dyn_smem<fg::k_hd_warp<T, N, WOBS, SCN, STD, POL, EXT>>(smem);
     if (err != cudaSuccess) return fail(FG_ERR_CUDA, "cudaFuncSetAttribute failed: %s", cudaGetErrorString(err));
     // persistent warps: at most one resident wave; each warp walks spans gw, gw + nwarps, ...
     int grid = (spans + w - 1) / w;
@@ -448,18 +487,17 @@ int launch_warp_tgt(const fg::KArgs<T>& a, cudaStream_t st) {
     wave *= std::max(1, fgabi::switches().waves.load(std::memory_order_relaxed));
     if (grid > wave) grid = wave;
     if ((grid * w) & 1) ++grid;                                    // even warp count (16-byte phase, fg_warp.cuh)
-    fg::k_hd_warp<T, N, WOBS, SCN, STD, POL, TGT><<<grid, 32 * w, smem, st>>>(a);
+    fg::k_hd_warp<T, N, WOBS, SCN, STD, POL, EXT><<<grid, 32 * w, smem, st>>>(a);
     err = cudaGetLastError();
     if (err != cudaSuccess) return fail(FG_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(err));
     return FG_OK;
 }
 
-// formation_hd_env runs with a target bank take the TGT instantiation of the same kernel
+// runs with a target bank or a terminal block take the EXT instantiation of the same kernel
 template <typename T, int N, bool WOBS, int SCN, bool STD, int POL = 0>
 int launch_warp_n(const fg::KArgs<T>& a, cudaStream_t st) {
-    if constexpr (SCN == fg::kScnHD)
-        if (a.tgt_count > 0) return launch_warp_tgt<T, N, WOBS, SCN, STD, POL, true>(a, st);
-    return launch_warp_tgt<T, N, WOBS, SCN, STD, POL, false>(a, st);
+    if (fg::reset_ext(a)) return launch_warp_ext<T, N, WOBS, SCN, STD, POL, true>(a, st);
+    return launch_warp_ext<T, N, WOBS, SCN, STD, POL, false>(a, st);
 }
 
 template <typename T, int N, int SCN = fg::kScnHD>
@@ -545,17 +583,45 @@ int obs_reward_impl(const fg_params* p, const fg_buffers* b, int scenario, int E
     return launch<T, false, true>(a, scenario, p, stream);
 }
 
+// Terminal observations (fg_final_obs): the observation pass of fg_obs_reward (k_step / k_step_obst without PHYS) on the
+// terminal block, in the EXT instantiation that skips CTAs without an ended env and writes no reward.
+template <typename T>
+int final_obs_impl(const fg_params* p, const fg_final* f, const uint8_t* done, void* obs, int scenario, int E, int N,
+                   int L, void* stream) {
+    NvtxRange nvtx_("fg_final_obs");
+    if (!f) return fail(FG_ERR_ARG, "fg_final_obs: the terminal block must be non-null%s");
+    int rc = check_final<T>(f, p, scenario, 1, 1, false, "fg_final_obs");
+    if (rc) return rc;
+    if (!done || !obs) return fail(FG_ERR_ARG, "fg_final_obs: done / obs must be non-null%s");
+    fg_buffers b;
+    memset(&b, 0, sizeof(b));
+    b.pos = f->pos; b.vel = f->vel; b.obs = obs;
+    if (p && !p->silent) b.comm = f->comm;
+    if (scenario == FG_SCENARIO_HD) { b.ideal_shape = f->ideal_shape; b.ideal_vel = f->ideal_vel; }
+    else b.landmarks = f->landmarks;                                // (hd: no landmark side effect)
+    fg::KArgs<T> a;
+    rc = fill_args<T>(a, p, &b, scenario, E, N, L, 0, 0, 0);
+    if (rc) return rc;
+    set_final<T>(a, f, p, scenario);
+    a.fin_done = done;                                              // reward, step, done, nan_flag, lmv: NULL above
+    if (scenario == FG_SCENARIO_HD_OBSTACLE) return launch_obstacle<T, false>(a, stream);
+    return launch<T, false, true>(a, scenario, p, stream);
+}
+
 template <typename T>
 int step_fused_impl(const fg_params* p, const fg_buffers* b, int scenario, int E, int N, int L, int n_steps,
                     int random_actions, int auto_reset, uint64_t seed, uint32_t tick, uint32_t env_offset,
-                    void* stream, const fg_targets* tg) {
+                    void* stream, const fg_targets* tg, const fg_final* fin) {
     NvtxRange nvtx_("fg_step_fused");
     int rc = check_targets<T>(tg, scenario, "fg_step_fused_targets");
+    if (rc) return rc;
+    rc = check_final<T>(fin, p, scenario, auto_reset, n_steps, true, "fg_step_fused_final");
     if (rc) return rc;
     fg::KArgs<T> a;
     rc = fill_args<T>(a, p, b, scenario, E, N, L, seed, tick, env_offset);
     if (rc) return rc;
     set_targets<T>(a, tg);
+    set_final<T>(a, fin, p, scenario);
     if (!b->pos || !b->vel || !b->reward || !b->done || !b->step)
         return fail(FG_ERR_ARG, "fg_step_fused: pos/vel/reward/done/step must be non-null%s");
     if (!random_actions && !b->act) return fail(FG_ERR_ARG, "fg_step_fused: act is null and random_actions == 0%s");

@@ -82,7 +82,16 @@ template <typename T> struct KArgs {
     const R2* tgt_vel;               // (opt) [K] ideal velocities, replacing the kResetIdealVel draw
     const int32_t* tgt_index;        // (opt) [E] task per env; out of [0, K) = draw
     int tgt_count;
+    // terminal block (fg_final; written only by the reset blocks of the EXT instantiations): fin_pos == NULL = none.
+    // fg_final_obs reads it back as the state (pos / vel / ...) and fin_done as the mask of ended envs.
+    R2* fin_pos; R2* fin_vel; R2* fin_comm;
+    R2* fin_shape; R2* fin_ivel; R2* fin_lm;
+    const uint8_t* fin_done;         // fg_final_obs: done [E,N] of the step
 };
+
+// An instantiation with the reset extension (template flag EXT) runs when a target bank or a terminal block is set.
+template <typename T>
+__host__ __device__ __forceinline__ bool reset_ext(const KArgs<T>& a) { return a.tgt_count > 0 || a.fin_pos != nullptr; }
 
 // Task of env e (global id ge) at a reset with tick tk: tgt_index[e] when it names an entry of the bank, else
 // drawn uniformly from Philox.  Only called when tgt_count > 0.
@@ -216,14 +225,17 @@ __device__ __forceinline__ void wall_force(const WallT<T>& w, T px, T py, T size
 // shared memory, the whole tile leaves as one bulk store.
 // FP: fast pair loops of fg_pairs.cuh (fp32, hd, uniform agents, N >= 32): structure-of-arrays partner
 // data, packed FFMA2/FADD2/FMUL2 arithmetic, group filters, warp-shuffle centroid and reductions.
-// TGT: formation_hd_env with a target bank (KArgs::tgt_*).  Its own instantiation, so that the reset block of the
-// product kernels -- and with it their register allocation -- is the same as without the feature.
-template <typename T, int SCN, bool PHYS, bool OBSREW, bool HET, int OM, bool FP, bool TGT = false>
+// EXT: the reset extension -- a target bank (KArgs::tgt_*, formation_hd_env) and / or a terminal block (KArgs::fin_*),
+// both run-time tests inside.  Its own instantiation, so that the reset block of the product kernels -- and with it
+// their register allocation -- is the same as without the features.  Without PHYS, EXT is fg_final_obs: the state is
+// the terminal block, a CTA without an ended env (fin_done) exits at once, and no reward is written.
+template <typename T, int SCN, bool PHYS, bool OBSREW, bool HET, int OM, bool FP, bool EXT = false>
 __global__ void __launch_bounds__(kBlock, (OM == 3 && SCN == kScnBasic) ? 5 : (OM == 2 || OM == 3 || FP) ? 4 : 3) k_step(const __grid_constant__ KArgs<T> a) {
     typedef Ops<T> O;
     typedef typename O::R2 R2;
     typedef typename O::Bits Bits;
     extern __shared__ __align__(16) unsigned char smem_raw[];
+    constexpr bool FINOBS = EXT && !PHYS;
 
     const int N = a.N, EPC = a.EPC, L = a.L;
     const int nA = EPC * N;
@@ -288,6 +300,10 @@ __global__ void __launch_bounds__(kBlock, (OM == 3 && SCN == kScnBasic) ? 5 : (O
     const int nvalid = min(EPC, a.E - tile0);                 // envs of this tile that exist
     const size_t g = (size_t)e * N + i;                       // global agent index
     const uint32_t ge = a.env_offset + (uint32_t)e;           // global env id (RNG counter)
+
+    if constexpr (FINOBS) {                                   // rows only where an episode ended (EPC <= kBlock)
+        if (!__syncthreads_or(t < nvalid && a.fin_done[(size_t)(tile0 + t) * N] != 0)) return;
+    }
 
     if (HET) {
         for (int q = t; q < N; q += kBlock) {
@@ -1031,7 +1047,7 @@ __global__ void __launch_bounds__(kBlock, (OM == 3 && SCN == kScnBasic) ? 5 : (O
             const int coltot = s_col[le];
             // shared reward = sum_i r_i (environment.py:136): N*base - total collisions, in fp64
             const double R = (double)N * (double)base - (double)coltot;
-            a.reward[g] = (T)R;
+            if (!FINOBS) a.reward[g] = (T)R;
             if (a.indiv) a.indiv[g] = r;
             if (a.done) a.done[g] = (uint8_t)(a.step ? (stp >= a.world_length) : 0);
             if (i == 0 && a.nan_flag && s_bad[le]) a.nan_flag[e] = 1;           // the reference's failure mode (Q9), sticky
@@ -1055,6 +1071,16 @@ __global__ void __launch_bounds__(kBlock, (OM == 3 && SCN == kScnBasic) ? 5 : (O
                 const uint32_t tk = tick0 + (uint32_t)ts;
                 R2 lraw = O::make((T)0, (T)0);
                 if (dn) {
+                    if constexpr (EXT) {                      // terminal block: the post-step state, before the reset
+                        if (a.fin_pos) {
+                            a.fin_pos[g] = p; a.fin_vel[g] = v;
+                            if (!a.silent) a.fin_comm[g] = s_c[t];
+                            if (SCN == kScnHD) {
+                                a.fin_shape[g] = s_s[t];
+                                if (i == 0) a.fin_ivel[e] = s_iv[le];
+                            }
+                        }
+                    }
                     U4 r = philox(a.seed, ge, (uint32_t)i, tk, kResetAgent);
                     p = O::make(uniform_pm1<T>(r.x), uniform_pm1<T>(r.y));
                     v = O::make((T)0, (T)0);
@@ -1063,16 +1089,18 @@ __global__ void __launch_bounds__(kBlock, (OM == 3 && SCN == kScnBasic) ? 5 : (O
                         U4 q = philox(a.seed, ge, (uint32_t)i, tk, kResetLandmark);
                         lraw = O::make(uniform_pm1<T>(q.x), uniform_pm1<T>(q.y));
                         uint32_t kt = 0;
-                        if constexpr (TGT) {                  // target bank: the task's raw shape
-                            kt = target_task<T>(a, e, ge, tk);
-                            lraw = a.tgt_shape[(size_t)kt * N + i];
+                        if constexpr (EXT) {                  // target bank: the task's raw shape
+                            if (a.tgt_count > 0) {
+                                kt = target_task<T>(a, e, ge, tk);
+                                lraw = a.tgt_shape[(size_t)kt * N + i];
+                            }
                         }
                         s_old[t] = lraw;                      // scratch: s_old is dead after the physics
                         if (a.lm) a.lm[g] = lraw;
                         if (i == 0) {
                             U4 w = philox(a.seed, ge, 0u, tk, kResetIdealVel);
                             R2 iv = O::make(uniform_pm1<T>(w.x), uniform_pm1<T>(w.y));
-                            if (TGT && a.tgt_vel) iv = a.tgt_vel[kt];
+                            if (EXT && a.tgt_count > 0 && a.tgt_vel) iv = a.tgt_vel[kt];
                             s_iv[le] = iv; a.ivel[e] = iv;
                         }
                     }
@@ -1082,6 +1110,7 @@ __global__ void __launch_bounds__(kBlock, (OM == 3 && SCN == kScnBasic) ? 5 : (O
                     for (int q = t; q < nvalid * L; q += kBlock) {
                         int qe = (int)fastdiv((uint32_t)q, a.magic_l), k = q - qe * L;
                         if (s_dn[qe]) {
+                            if (EXT && a.fin_pos) a.fin_lm[(size_t)tile0 * L + q] = s_s[q];   // terminal block
                             U4 r = philox(a.seed, a.env_offset + (uint32_t)(tile0 + qe), (uint32_t)k, tk, kResetLandmark);
                             R2 l = O::make(uniform_pm1<T>(r.x), uniform_pm1<T>(r.y));
                             s_s[q] = l; a.lm[(size_t)tile0 * L + q] = l;

@@ -7,7 +7,7 @@
 
 namespace {
 
-template <typename T, int N, int L, int SCN, int NOBS, bool STD>
+template <typename T, int N, int L, int SCN, int NOBS, bool STD, bool EXT>
 const WarpGeom& lm_geom() {
     static const WarpGeom geom = [] {
         typedef fg::LmLayout<T, N, L, SCN, NOBS> LY;
@@ -21,44 +21,51 @@ const WarpGeom& lm_geom() {
             const size_t smem = (size_t)w * LY::stride;
             g_.ctas[l] = 0;
             if (smem > 227 * 1024 || w > LY::MAXW) continue;
-            if (cudaFuncSetAttribute(fg::k_lm_warp<T, N, L, SCN, NOBS, STD>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+            if (cudaFuncSetAttribute(fg::k_lm_warp<T, N, L, SCN, NOBS, STD, EXT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                      (int)smem) != cudaSuccess) { cudaGetLastError(); continue; }
             int ctas = 0;
-            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas, fg::k_lm_warp<T, N, L, SCN, NOBS, STD>, 32 * w, smem)
+            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas, fg::k_lm_warp<T, N, L, SCN, NOBS, STD, EXT>, 32 * w, smem)
                 != cudaSuccess) { cudaGetLastError(); continue; }
             g_.ctas[l] = ctas;
             if (ctas * w > best_res) { best_res = ctas * w; g_.best = l; }
         }
         // (see warp_geom: the probing left the limit at the smallest footprint)
-        cudaFuncSetAttribute(fg::k_lm_warp<T, N, L, SCN, NOBS, STD>, cudaFuncAttributeMaxDynamicSharedMemorySize, 48 * 1024);
+        cudaFuncSetAttribute(fg::k_lm_warp<T, N, L, SCN, NOBS, STD, EXT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 48 * 1024);
         cudaGetLastError();
         return g_;
     }();
     return geom;
 }
 
-template <typename T, int N, int L, int SCN, int NOBS>
-int launch_lm_n(const fg::KArgs<T>& a, cudaStream_t st) {
+template <typename T, int N, int L, int SCN, int NOBS, bool EXT>
+int launch_lm_ext(const fg::KArgs<T>& a, cudaStream_t st) {
     constexpr bool STD = std::is_same<T, float>::value;            // fp32: the standard configuration only (caller checked)
     typedef fg::LmLayout<T, N, L, SCN, NOBS> LY;
-    const WarpGeom& gm = lm_geom<T, N, L, SCN, NOBS, STD>();
+    const WarpGeom& gm = lm_geom<T, N, L, SCN, NOBS, STD, EXT>();
     const int spans = (a.E + LY::EPW - 1) / LY::EPW;
     int l = gm.best;
     while (l > 0 && (spans >> l) < 2 * gm.sms) --l;                // small batches: spread over the SMs
     if (gm.ctas[l] < 1) return fail(FG_ERR_CUDA, "k_lm_warp does not fit on this device%s");
     const int w = 1 << l;
     const size_t smem = (size_t)w * LY::stride;
-    cudaError_t err = ensure_dyn_smem<fg::k_lm_warp<T, N, L, SCN, NOBS, STD>>(smem);
+    cudaError_t err = ensure_dyn_smem<fg::k_lm_warp<T, N, L, SCN, NOBS, STD, EXT>>(smem);
     if (err != cudaSuccess) return fail(FG_ERR_CUDA, "cudaFuncSetAttribute failed: %s", cudaGetErrorString(err));
     int grid = (spans + w - 1) / w;                                // persistent warps: at most one resident wave
     int wave = gm.sms * gm.ctas[l];
     wave *= std::max(1, fgabi::switches().waves.load(std::memory_order_relaxed));
     if (grid > wave) grid = wave;
     if ((grid * w) & 1) ++grid;                                    // even warp count (16-byte phase, fg_warp.cuh)
-    fg::k_lm_warp<T, N, L, SCN, NOBS, STD><<<grid, 32 * w, smem, st>>>(a);
+    fg::k_lm_warp<T, N, L, SCN, NOBS, STD, EXT><<<grid, 32 * w, smem, st>>>(a);
     err = cudaGetLastError();
     if (err != cudaSuccess) return fail(FG_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(err));
     return FG_OK;
+}
+
+// runs with a terminal block take the EXT instantiation of the same kernel
+template <typename T, int N, int L, int SCN, int NOBS>
+int launch_lm_n(const fg::KArgs<T>& a, cudaStream_t st) {
+    if (fg::reset_ext(a)) return launch_lm_ext<T, N, L, SCN, NOBS, true>(a, st);
+    return launch_lm_ext<T, N, L, SCN, NOBS, false>(a, st);
 }
 
 // Instantiations: make_world's default landmark counts (5 / 4) and num_obs = 3 for 3 .. 9 agents -- what

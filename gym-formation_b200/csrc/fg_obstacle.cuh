@@ -35,13 +35,17 @@ __device__ __forceinline__ void obstacle_reset(uint64_t seed, uint32_t ge, int s
 
 // OBSREW = false: World.step alone (core.py:206-225) on a world with obstacles -- no scenario hooks, so the
 // obstacles keep their INTEGRATED velocity (the (0, -1) rule is the reward hook's side effect).
-template <typename T, bool PHYS, bool OBSREW = true>
+// EXT (reset extension, as in k_step): the auto-reset copies the terminal state into the terminal block (KArgs::fin_*).
+// Without PHYS, EXT is fg_final_obs: the state is the terminal block, a CTA without an ended env (fin_done) exits at
+// once, and no reward is written.
+template <typename T, bool PHYS, bool OBSREW = true, bool EXT = false>
 __global__ void __launch_bounds__(kBlock, 2) k_step_obst(const __grid_constant__ KArgs<T> a) {
     static_assert(PHYS || OBSREW, "nothing to do");
     typedef Ops<T> O_;
     typedef typename O_::R2 R2;
     typedef typename O_::Bits Bits;
     extern __shared__ __align__(16) unsigned char smem_raw[];
+    constexpr bool FINOBS = EXT && !PHYS;
 
     const int N = a.N, EPC = a.EPC, L = a.L, NO = a.n_obst, LG = a.L - a.n_obst;
     const int nA = EPC * N;
@@ -75,6 +79,10 @@ __global__ void __launch_bounds__(kBlock, 2) k_step_obst(const __grid_constant__
     const T dmin_oo = O_::add(a.osize, a.osize);
     const T cut_ao = dmin_ao + a.kcut * a.margin, cut_oo = dmin_oo + a.kcut * a.margin;
     const T cut2_ao = cut_ao * cut_ao, cut2_oo = cut_oo * cut_oo;
+
+    if constexpr (FINOBS) {                                  // rows only where an episode ended (EPC <= kBlock)
+        if (!__syncthreads_or(t < nvalid && a.fin_done[(size_t)(tile0 + t) * N] != 0)) return;
+    }
 
     R2 p = O_::make((T)0, (T)0), v = p, u = p;
     int stp = 0;
@@ -296,7 +304,7 @@ __global__ void __launch_bounds__(kBlock, 2) k_step_obst(const __grid_constant__
             for (int c = 0; c < col; ++c) r = O_::sub(r, (T)2);                   // rew -= 2 per collision
             const int coltot = s_col[le];
             const double R = (double)N * (double)base - 2.0 * (double)coltot;    // environment.py:136
-            a.reward[g] = (T)R;
+            if (!FINOBS) a.reward[g] = (T)R;
             if (a.indiv) a.indiv[g] = r;
             if (a.done) a.done[g] = (uint8_t)(a.step ? (stp >= a.world_length) : 0);
             if (i == 0 && a.nan_flag && s_bad[le]) a.nan_flag[e] = 1;           // the reference's failure mode (Q9), sticky
@@ -322,6 +330,7 @@ __global__ void __launch_bounds__(kBlock, 2) k_step_obst(const __grid_constant__
             if (__syncthreads_or(dn ? 1 : 0)) {
                 const uint32_t tk = tick0 + (uint32_t)ts;
                 if (dn) {
+                    if (EXT && a.fin_pos) { a.fin_pos[g] = p; a.fin_vel[g] = v; }   // terminal block: post-step state
                     U4 r = philox(a.seed, ge, (uint32_t)i, tk, kResetAgent);
                     p = O_::make(uniform_pm1<T>(r.x), uniform_pm1<T>(r.y));
                     v = O_::make((T)0, (T)0);
@@ -332,6 +341,8 @@ __global__ void __launch_bounds__(kBlock, 2) k_step_obst(const __grid_constant__
                 for (int q = t; q < nvalid * L; q += kBlock) {
                     const int qe = q / L, k = q - qe * L;
                     if (!s_dn[qe]) continue;
+                    if (EXT && a.fin_pos)                    // goals, then the obstacles at their post-step positions
+                        a.fin_lm[(size_t)tile0 * L + q] = k < LG ? s_lm[q] : s_on[qe * NO + (k - LG)];
                     const uint32_t gq = a.env_offset + (uint32_t)(tile0 + qe);
                     if (k < LG) {
                         U4 r = philox(a.seed, gq, (uint32_t)k, tk, kResetLandmark);

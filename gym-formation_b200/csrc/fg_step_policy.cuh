@@ -39,12 +39,14 @@ bool std_config(const fg::KArgs<T>& a) {
 template <typename T>
 int step_policy_impl(const fg_params* p, const fg_buffers* b, int scenario, int E, int N, int L, int n_steps,
                      int n, int auto_reset, uint64_t seed, uint32_t tick, uint32_t env_offset, void* stream,
-                     const fg_targets* tg,
+                     const fg_targets* tg, const fg_final* fin,
                      int (*step_fused)(const fg_params*, const fg_buffers*, int, int, int, int, int, int, int, uint64_t,
-                                       uint32_t, uint32_t, void*, const fg_targets*),
+                                       uint32_t, uint32_t, void*, const fg_targets*, const fg_final*),
                      int (*policy_bfs)(const void*, const void*, const void*, void*, int, int, int, void*)) {
     NvtxRange nvtx_("fg_step_policy");
     int rc = check_targets<T>(tg, scenario, "fg_step_policy_targets");
+    if (rc) return rc;
+    rc = check_final<T>(fin, p, scenario, auto_reset, n_steps, true, "fg_step_policy_final");
     if (rc) return rc;
     if (scenario != FG_SCENARIO_HD)
         return fail(FG_ERR_ARG, "fg_step_policy: the controller reads formation_hd_env observations "
@@ -64,6 +66,7 @@ int step_policy_impl(const fg_params* p, const fg_buffers* b, int scenario, int 
     rc = fill_args<T>(a, p, b, scenario, E, N, L, seed, tick, env_offset);
     if (rc) return rc;
     set_targets<T>(a, tg);
+    set_final<T>(a, fin, p, scenario);
     const bool fused = b->vel && b->reward && b->done && b->step && warp_path_ok<T>(a, scenario, p, b) && std_config<T>(a);
     if (fused) {
         a.random_actions = 0; a.auto_reset = auto_reset;
@@ -91,7 +94,7 @@ int step_policy_impl(const fg_params* p, const fg_buffers* b, int scenario, int 
     // two launches per step: the kernels a caller would launch itself (same results as the fused form)
     for (int ts = 0; ts < n_steps; ++ts) {
         rc = step_fused(p, b, scenario, E, N, L, 1, 0, auto_reset, seed, tick + (b->tick_dev ? 0u : (uint32_t)ts),
-                        env_offset, stream, tg);
+                        env_offset, stream, tg, fin);
         if (rc) return rc;
         rc = policy_bfs(b->pos, b->ideal_shape, b->ideal_vel, const_cast<void*>(b->act), E, N, n, stream);
         if (rc) return rc;

@@ -6,12 +6,20 @@ extern "C" int fg_step_policy(const fg_params* p, const fg_buffers* b, int scena
                               int num_agents_per_layer, int auto_reset, uint64_t seed, uint32_t tick,
                               uint32_t env_offset, void* stream) {
     return step_policy_impl<float>(p, b, scenario, E, N, L, n_steps, num_agents_per_layer, auto_reset, seed, tick,
-                                   env_offset, stream, nullptr, &fg_step_fused_targets, &fg_policy_bfs);
+                                   env_offset, stream, nullptr, nullptr, &fg_step_fused_final, &fg_policy_bfs);
 }
 
 extern "C" int fg_step_policy_targets(const fg_params* p, const fg_buffers* b, int scenario, int E, int N, int L,
                                       int n_steps, int num_agents_per_layer, int auto_reset, uint64_t seed,
                                       uint32_t tick, uint32_t env_offset, void* stream, const fg_targets* t) {
     return step_policy_impl<float>(p, b, scenario, E, N, L, n_steps, num_agents_per_layer, auto_reset, seed, tick,
-                                   env_offset, stream, t, &fg_step_fused_targets, &fg_policy_bfs);
+                                   env_offset, stream, t, nullptr, &fg_step_fused_final, &fg_policy_bfs);
+}
+
+extern "C" int fg_step_policy_final(const fg_params* p, const fg_buffers* b, int scenario, int E, int N, int L,
+                                    int n_steps, int num_agents_per_layer, int auto_reset, uint64_t seed,
+                                    uint32_t tick, uint32_t env_offset, void* stream, const fg_targets* t,
+                                    const fg_final* f) {
+    return step_policy_impl<float>(p, b, scenario, E, N, L, n_steps, num_agents_per_layer, auto_reset, seed, tick,
+                                   env_offset, stream, t, f, &fg_step_fused_final, &fg_policy_bfs);
 }

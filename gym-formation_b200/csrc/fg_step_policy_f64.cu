@@ -5,12 +5,20 @@ extern "C" int fg_step_policy_f64(const fg_params* p, const fg_buffers* b, int s
                                   int n_steps, int num_agents_per_layer, int auto_reset, uint64_t seed, uint32_t tick,
                                   uint32_t env_offset, void* stream) {
     return step_policy_impl<double>(p, b, scenario, E, N, L, n_steps, num_agents_per_layer, auto_reset, seed, tick,
-                                    env_offset, stream, nullptr, &fg_step_fused_targets_f64, &fg_policy_bfs_f64);
+                                    env_offset, stream, nullptr, nullptr, &fg_step_fused_final_f64, &fg_policy_bfs_f64);
 }
 
 extern "C" int fg_step_policy_targets_f64(const fg_params* p, const fg_buffers* b, int scenario, int E, int N, int L,
                                           int n_steps, int num_agents_per_layer, int auto_reset, uint64_t seed,
                                           uint32_t tick, uint32_t env_offset, void* stream, const fg_targets* t) {
     return step_policy_impl<double>(p, b, scenario, E, N, L, n_steps, num_agents_per_layer, auto_reset, seed, tick,
-                                    env_offset, stream, t, &fg_step_fused_targets_f64, &fg_policy_bfs_f64);
+                                    env_offset, stream, t, nullptr, &fg_step_fused_final_f64, &fg_policy_bfs_f64);
+}
+
+extern "C" int fg_step_policy_final_f64(const fg_params* p, const fg_buffers* b, int scenario, int E, int N, int L,
+                                        int n_steps, int num_agents_per_layer, int auto_reset, uint64_t seed,
+                                        uint32_t tick, uint32_t env_offset, void* stream, const fg_targets* t,
+                                        const fg_final* f) {
+    return step_policy_impl<double>(p, b, scenario, E, N, L, n_steps, num_agents_per_layer, auto_reset, seed, tick,
+                                    env_offset, stream, t, f, &fg_step_fused_final_f64, &fg_policy_bfs_f64);
 }

@@ -98,16 +98,16 @@ template <typename T, int N, bool WOBS> struct WarpLayout {
 // positions, the ideal shape and ideal_vel are already on chip, so the controller costs its arithmetic only: no second
 // launch, no re-read of the state (fg_policy.cuh: policy_chain; each lane evaluates the nodes of its own leaders).
 //
-// TGT (formation_hd_env): the auto-reset takes the env's task from the target bank (KArgs::tgt_*).  A separate
+// EXT (reset extension): the auto-reset takes the env's task from the target bank (KArgs::tgt_*, formation_hd_env) and
+// copies the terminal state into the terminal block (KArgs::fin_*), each when set (run-time tests).  A separate
 // instantiation: the reset block shares the registers of the step, and a bank branch compiled into every kernel changed
 // the allocation (and added spills) of the product instantiations.
-template <typename T, int N, bool WOBS, int SCN = kScnHD, bool STD = false, int POL = 0, bool TGT = false>
+template <typename T, int N, bool WOBS, int SCN = kScnHD, bool STD = false, int POL = 0, bool EXT = false>
 // (basic_formation_env, N = 3: four 8-warp CTAs per SM -- 64 registers, no spills -- measured 80.9 vs 88.7 us per 1 M envs;
 // the hd instantiation of the same N loses with them: 89.2 vs 82.0 us)
 __global__ void __launch_bounds__(32 * WarpLayout<T, N, WOBS>::MAXW, (SCN == kScnBasic && sizeof(T) == 4) ? 4 : WarpLayout<T, N, WOBS>::MINB) k_hd_warp(const __grid_constant__ KArgs<T> a) {
     static_assert(SCN == kScnHD || WarpLayout<T, N, WOBS>::LATE_FILL, "basic rows are written by the late fill");
     static_assert(POL == 0 || (SCN == kScnHD && PolLevels<N, POL>::v > 0), "POL: formation_hd_env with N = POL^k agents");
-    static_assert(!TGT || SCN == kScnHD, "TGT: formation_hd_env target banks");
     typedef Ops<T> O;
     typedef typename O::R2 R2;
     typedef typename O::Bits Bits;
@@ -479,6 +479,13 @@ __global__ void __launch_bounds__(32 * WarpLayout<T, N, WOBS>::MAXW, (SCN == kSc
             const uint32_t tk = tick0 + (uint32_t)ts;
             R2 lraw = zero;
             if (dn) {
+                if constexpr (EXT) {                                        // terminal block: the post-step state
+                    if (a.fin_pos) {
+                        a.fin_pos[g] = p; a.fin_vel[g] = v;
+                        if (SCN == kScnBasic) a.fin_lm[g] = S;              // landmark `lane` of the span (L == N)
+                        else { a.fin_shape[g] = S; if (i == 0) a.fin_ivel[e] = iv; }
+                    }
+                }
                 U4 r = philox(a.seed, ge, (uint32_t)i, tk, kResetAgent);
                 p = O::make(uniform_pm1<T>(r.x), uniform_pm1<T>(r.y));
                 v = zero;
@@ -495,10 +502,12 @@ __global__ void __launch_bounds__(32 * WarpLayout<T, N, WOBS>::MAXW, (SCN == kSc
                 } else {
                     U4 w = philox(a.seed, ge, 0u, tk, kResetIdealVel);
                     iv = O::make(uniform_pm1<T>(w.x), uniform_pm1<T>(w.y));
-                    if constexpr (TGT) {                                    // target bank: the task's shape / velocity
-                        const uint32_t kt = target_task<T>(a, e, ge, tk);
-                        lraw = a.tgt_shape[(size_t)kt * N + i];
-                        if (a.tgt_vel) iv = a.tgt_vel[kt];
+                    if constexpr (EXT) {                                    // target bank: the task's shape / velocity
+                        if (a.tgt_count > 0) {
+                            const uint32_t kt = target_task<T>(a, e, ge, tk);
+                            lraw = a.tgt_shape[(size_t)kt * N + i];
+                            if (a.tgt_vel) iv = a.tgt_vel[kt];
+                        }
                     }
                     s_pold[lane] = lraw;                                    // scratch: pold is dead until the next step
                     if (i == 0) a.ivel[e] = iv;

@@ -70,7 +70,9 @@ template <typename T, int N, int L, int SCN, int NOBS> struct LmLayout {
 // unit mass, no max_speed, one step per launch, step / done / indiv / ep_return / ep_collisions / stats present, no comm
 // buffer): the warp-uniform run-time tests of these are compiled out, as in fg_warp.cuh.  The fp32 build has only
 // this instantiation (anything else takes the tile kernel), the fp64 build only the generic one.
-template <typename T, int N, int L, int SCN, int NOBS, bool STD>
+// EXT (reset extension, as in fg_warp.cuh): the auto-reset copies the terminal state into the terminal block
+// (KArgs::fin_*); its own instantiation, so that the kernels of runs without a block keep their register allocation.
+template <typename T, int N, int L, int SCN, int NOBS, bool STD, bool EXT = false>
 // (three 8-warp CTAs per SM, <= 80 registers: for the obstacle scenario two CTAs at up to 128 registers run 62.6 -> 69.7 us
 // per 262144 envs of 4 agents, four at 64 registers with 56 bytes of spills 62.3 -> 68.4 us)
 __global__ void __launch_bounds__(32 * LmLayout<T, N, L, SCN, NOBS>::MAXW, 3) k_lm_warp(const __grid_constant__ KArgs<T> a) {
@@ -457,6 +459,15 @@ __global__ void __launch_bounds__(32 * LmLayout<T, N, L, SCN, NOBS>::MAXW, 3) k_
         if (a.auto_reset && __any_sync(FULL, dn)) {
             const uint32_t tk = tick0 + (uint32_t)ts;
             if (dn) {
+                if constexpr (EXT) {                                        // terminal block: the post-step state
+                    if (a.fin_pos) {
+                        a.fin_pos[g] = p; a.fin_vel[g] = v;
+#pragma unroll
+                        for (int k0 = 0; k0 < LG; k0 += N)
+                            if (k0 + i < LG) a.fin_lm[(size_t)e * L + k0 + i] = s_lm[le * L + k0 + i];
+                        if (OBST && i < NO) a.fin_lm[(size_t)e * L + LG + i] = s_on[le * NO + i];
+                    }
+                }
                 U4 r = philox(a.seed, ge, (uint32_t)i, tk, kResetAgent);
                 p = O::make(uniform_pm1<T>(r.x), uniform_pm1<T>(r.y));
                 v = zero;

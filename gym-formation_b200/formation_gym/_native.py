@@ -25,7 +25,8 @@ EXPORTS = [
     "fg_random_actions", "fg_random_actions_f64", "fg_fp32_probe", "fg_write_probe", "fg_policy_bfs", "fg_policy_bfs_f64",
     "fg_obs_to_host", "fg_pair_distances", "fg_pair_distances_f64", "fg_step_policy", "fg_step_policy_f64",
     "fg_reset_targets", "fg_reset_targets_f64", "fg_step_fused_targets", "fg_step_fused_targets_f64",
-    "fg_step_policy_targets", "fg_step_policy_targets_f64",
+    "fg_step_policy_targets", "fg_step_policy_targets_f64", "fg_step_fused_final", "fg_step_fused_final_f64",
+    "fg_step_policy_final", "fg_step_policy_final_f64", "fg_final_obs", "fg_final_obs_f64",
 ]
 
 
@@ -73,6 +74,13 @@ class fg_targets(C.Structure):
     _fields_ = [("shapes", C.c_void_p), ("vels", C.c_void_p), ("index", C.c_void_p), ("count", C.c_int32)]
 
 
+class fg_final(C.Structure):
+    """Terminal block (the ``*_final`` entry points and ``fg_final_obs``): device arrays shaped like the state that
+    receive the post-step state of every env whose episode ends in an auto-resetting step."""
+    _fields_ = [("pos", C.c_void_p), ("vel", C.c_void_p), ("comm", C.c_void_p), ("ideal_shape", C.c_void_p),
+                ("ideal_vel", C.c_void_p), ("landmarks", C.c_void_p)]
+
+
 _lib = None
 
 
@@ -115,6 +123,11 @@ def load():
             [P(fg_params), P(fg_buffers), I, I, I, I, I, I, I, U64, U32, U32, VP, P(fg_targets)]
         getattr(lib, "fg_reset_targets" + sfx).argtypes = \
             [P(fg_params), P(fg_buffers), I, I, I, I, VP, U64, U32, U32, VP, P(fg_targets)]
+        getattr(lib, "fg_step_fused_final" + sfx).argtypes = \
+            [P(fg_params), P(fg_buffers), I, I, I, I, I, I, I, U64, U32, U32, VP, P(fg_targets), P(fg_final)]
+        getattr(lib, "fg_step_policy_final" + sfx).argtypes = \
+            [P(fg_params), P(fg_buffers), I, I, I, I, I, I, I, U64, U32, U32, VP, P(fg_targets), P(fg_final)]
+        getattr(lib, "fg_final_obs" + sfx).argtypes = [P(fg_params), P(fg_final), VP, VP, I, I, I, I, VP]
         getattr(lib, "fg_random_actions" + sfx).argtypes = [VP, I, I, U64, U32, U32, VP, VP]
         getattr(lib, "fg_policy_bfs" + sfx).argtypes = [VP, VP, VP, VP, I, I, I, VP]
         getattr(lib, "fg_pair_distances" + sfx).argtypes = [VP, VP, I, I, VP, VP, VP, VP, VP]

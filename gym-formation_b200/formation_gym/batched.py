@@ -98,12 +98,14 @@ class BatchedFormationEnv:
                  walls=(), dt=0.1, damping=0.25, contact_force=1e2, contact_margin=1e-3,
                  sensitivity=5.0, num_obs=3, obs_range=0.7, num_obstacles=3, obstacle_size=0.15,
                  obstacle_mass=1.0, obstacle_floor=-2.2, obstacle_fall_vy=-1.0, target_shapes=None,
-                 target_vels=None, target_index=None):
+                 target_vels=None, target_index=None, record_final=False):
         if scenario not in SCENARIOS:
             raise ValueError("unknown scenario %r (supported: %s)" % (scenario, sorted(SCENARIOS)))
         if dtype not in (torch.float32, torch.float64):
             raise ValueError("dtype must be torch.float32 or torch.float64")
         bank = _target_bank(scenario, int(num_envs), int(num_agents), target_shapes, target_vels, target_index)
+        if record_final and not auto_reset:
+            raise ValueError("record_final records the state an auto-reset overwrites: it needs auto_reset=True")
         self._lib = nat.load()                      # raises when the CUDA extension is missing
         self._fns = {}
         if not torch.cuda.is_available():
@@ -197,6 +199,7 @@ class BatchedFormationEnv:
         self._bfs_primed = 0          # fan-out n while self.actions holds the controller's output for the current state (step_bfs)
         self._bufs = self._make_buffers()
         self._set_target_bank(bank)
+        self._set_final_block(bool(record_final))
 
     # ------------------------------------------------------------------ plumbing
     def _make_buffers(self, act=None, obs="default"):
@@ -238,8 +241,40 @@ class BatchedFormationEnv:
         t.index, t.count = nat.ptr(self.target_index), int(shapes.shape[0])
         self._targets = t
 
+    def _set_final_block(self, on):
+        """Terminal block (include/formation_gym_b200.h fg_final): ``final_*`` tensors shaped like the state.  An
+        auto-resetting step copies into them the post-step state of every env whose episode it ends (``done[:, 0]``),
+        before the reset overwrites it; the entries of other envs keep what they held."""
+        self.record_final = on
+        self.final_pos = self.final_vel = self.final_comm = None
+        self.final_ideal_shape = self.final_ideal_vel = self.final_landmarks = None
+        self._final = None
+        self._final_obs = None
+        if not on:
+            return
+        kw = dict(device=self.device, dtype=self.dtype)
+        E, N, L = self.E, self.N, self.L
+        self.final_pos = torch.zeros(E, N, 2, **kw)
+        self.final_vel = torch.zeros(E, N, 2, **kw)
+        if not self.silent:
+            self.final_comm = torch.zeros(E, N, 2, **kw)
+        if self.scn == nat.FG_SCENARIO_HD:
+            self.final_ideal_shape = torch.zeros(E, N, 2, **kw)
+            self.final_ideal_vel = torch.zeros(E, 2, **kw)
+        else:
+            self.final_landmarks = torch.zeros(E, L, 2, **kw)
+        f = nat.fg_final()
+        f.pos, f.vel, f.comm = nat.ptr(self.final_pos), nat.ptr(self.final_vel), nat.ptr(self.final_comm)
+        f.ideal_shape, f.ideal_vel = nat.ptr(self.final_ideal_shape), nat.ptr(self.final_ideal_vel)
+        f.landmarks = nat.ptr(self.final_landmarks)
+        self._final = f
+
     def _call(self, name, *args):
-        """Entry point ``name`` (``name + '_targets'`` with the target bank appended when one is set)."""
+        """Entry point ``name``; with a terminal block ``name + '_final'`` (target bank or NULL, then the block), else
+        ``name + '_targets'`` with the target bank appended when one is set.  Resets take no terminal block."""
+        if self._final is not None and name != "fg_reset":
+            t = C.byref(self._targets) if self._targets is not None else None
+            return self._fn(name + "_final")(*args, t, C.byref(self._final))
         if self._targets is not None:
             return self._fn(name + "_targets")(*args, C.byref(self._targets))
         return self._fn(name)(*args)
@@ -360,6 +395,25 @@ class BatchedFormationEnv:
         self._launch_fused(self._bufs, 1, 2 if record_actions else 1)
         return self.obs, self.reward, self.done, {"individual_reward": self.indiv}
 
+    def final_observation(self):
+        """Terminal observations of the last step: ``obs [E,N,D]`` whose rows of the envs with ``done[:, 0]`` are the
+        observation of the state the episode ended in -- bit-identical to what that step returns with
+        ``auto_reset=False`` (baselines' ``infos[e]['terminal_observation']``; every episode here ends on the time
+        limit, so a value target bootstraps from it).  Rows of other envs are unspecified.  Needs
+        ``record_final=True``.  One launch into a buffer owned by this object (allocated on first use, overwritten by
+        the next call), no synchronisation: it may be captured in a CUDA graph.  A CTA of envs none of which ended
+        exits at once, so a call after a step that ended no episode costs about one launch."""
+        if self._final is None:
+            raise ValueError("final_observation needs record_final=True")
+        if self._final_obs is None:
+            self._final_obs = torch.zeros(self.E, self.N, self.D, device=self.device, dtype=self.dtype)
+        with self._on_device():
+            rc = self._fn("fg_final_obs")(C.byref(self.params), C.byref(self._final), nat.ptr(self._done_u8),
+                                          nat.ptr(self._final_obs), self.scn, self.E, self.N, self.L, self._stream())
+            nat.check(rc, "fg_final_obs")
+            self.launches += 1
+        return self._final_obs
+
     def nan_envs(self, clear=False):
         """Indices of envs that hit the reference's documented failure mode since the flags were last cleared:
         coincident agents make ``delta_pos / dist`` NaN (core.py:312) and the env's state and rewards stay NaN until
@@ -410,6 +464,8 @@ class BatchedFormationEnv:
         (``fg_step_policy``; N = 3 with 3 agents per layer, 4 / 8 with 2, 16 with 4), the step kernel
         + the controller kernel otherwise -- same results.  The first call after anything else changed the state
         (reset, step, load_state_dict, ...) computes the first actions with ``bfs_actions`` (one extra launch)."""
+        if self._final is not None and int(n_steps) != 1:
+            raise ValueError("record_final: one step per call (done[:, 0] is the mask of the recorded envs)")
         n = int(num_agents_per_layer)
         if self.scn != nat.FG_SCENARIO_HD or not self.silent:
             raise nat.NativeError("the hand-written controller is defined for formation_hd_env with silent agents")
@@ -428,6 +484,8 @@ class BatchedFormationEnv:
     def rollout_random(self, n_steps):
         """``n_steps`` random-policy steps in ONE launch with the state held on chip; obs / reward /
         done buffers hold the last step's values afterwards."""
+        if self._final is not None and int(n_steps) != 1:
+            raise ValueError("record_final: one step per call (done[:, 0] is the mask of the recorded envs)")
         self._launch_fused(self._bufs, int(n_steps), 1)
         return self.obs, self.reward, self.done, {"individual_reward": self.indiv}
 

@@ -27,17 +27,21 @@ from .batched import BatchedFormationEnv
 
 
 class _EnvInfo(object):
-    """infos[e]: list-like of N dicts {'individual_reward': r_i} of one env, built on demand."""
-    __slots__ = ("_row",)
+    """infos[e]: list-like of N dicts {'individual_reward': r_i} of one env, built on demand; with
+    'terminal_observation': agent i's row when the env's episode ended in this step (record_final)."""
+    __slots__ = ("_row", "_term")
 
-    def __init__(self, row):
+    def __init__(self, row, term=None):
         self._row = row
+        self._term = term
 
     def __len__(self):
         return len(self._row)
 
     def __getitem__(self, i):
-        return {'individual_reward': float(self._row[i])}
+        if self._term is None:
+            return {'individual_reward': float(self._row[i])}
+        return {'individual_reward': float(self._row[i]), 'terminal_observation': self._term[i]}
 
     def __iter__(self):
         return (self[i] for i in range(len(self)))
@@ -46,15 +50,24 @@ class _EnvInfo(object):
 class InfoBatch(object):
     """``infos`` of one vectorised step.  ``infos[e][i]['individual_reward']`` like the tuple of info
     lists the reference's ``step_wait`` returns (env_wrappers.py:71-72), without creating E*N dicts;
-    ``infos.individual_reward`` is the whole ``[E,N]`` array / tensor."""
+    ``infos.individual_reward`` is the whole ``[E,N]`` array / tensor.  With ``record_final``, on the steps where
+    episodes end, ``infos.terminal_observation`` is the whole ``[E,N,D]`` array / tensor of terminal observations
+    (rows valid where ``dones[:, 0]``) and ``infos[e][i]['terminal_observation']`` agent i's row, for the envs that
+    ended only (the key of baselines' / SB3's VecEnvs, per agent)."""
+    terminal_observation = None
 
-    def __init__(self, individual_reward):
+    def __init__(self, individual_reward, terminal_observation=None, done=None):
         self.individual_reward = individual_reward
+        if terminal_observation is not None:
+            self.terminal_observation = terminal_observation
+            self._done = done
 
     def __len__(self):
         return int(self.individual_reward.shape[0])
 
     def __getitem__(self, e):
+        if self.terminal_observation is not None and bool(self._done[e, 0]):
+            return _EnvInfo(self.individual_reward[e], self.terminal_observation[e])
         return _EnvInfo(self.individual_reward[e])
 
     def __iter__(self):
@@ -91,6 +104,11 @@ class CudaVecEnv(object):
         self._pending = None
         self._age = None
         self._np_dtype = np.float32 if e.dtype == torch.float32 else np.float64
+        # record_final: terminal observations in the infos of the steps where episodes end.  All envs are reset
+        # together and share one episode length, so the host knows those steps (None: unknown -> every step)
+        self.record_final = e.record_final
+        self._final_age = None
+        self._final_pending = None
         if self.to_numpy:
             # pinned host staging: actions in, obs / rewards / dones / individual rewards out
             self._act_h = torch.empty(e.E, e.N, act_dim, dtype=e.dtype).pin_memory()
@@ -119,6 +137,10 @@ class CudaVecEnv(object):
             self._views = tuple(t.numpy() for t in (self._obs_h, self._rew_h, self._done_h, self._ind_h))
             for v in self._views:
                 v.flags.writeable = False
+            if self.record_final:
+                self._fobs_h = torch.empty(e.obs.shape, dtype=e.dtype).pin_memory()
+                self._fobs_view = self._fobs_h.numpy()
+                self._fobs_view.flags.writeable = False
 
     # ------------------------------------------------------------------ VecEnv interface
     @property
@@ -132,6 +154,7 @@ class CudaVecEnv(object):
         self.waiting = False
         obs = self.env.reset()
         self._age = 0
+        self._final_age = 0
         return self._obs_out(obs)
 
     def reset_task(self):
@@ -153,6 +176,16 @@ class CudaVecEnv(object):
             self._act_d.copy_(self._act_h, non_blocking=True)
             actions = self._act_d
         self._pending = e.step(actions)
+        self._final_pending = None
+        if self.record_final:
+            ending = self._final_age is None
+            if not ending:
+                self._final_age += 1
+                ending = self._final_age % e.world_length == 0
+            if ending:                                              # episodes (may) end in this step
+                self._final_pending = e.final_observation()
+                if self.to_numpy:
+                    self._fobs_h.copy_(self._final_pending, non_blocking=True)
         if self.to_numpy:                                           # D2H overlaps nothing else: queue it now
             obs, rew, done, info = self._pending
             self._fetch_obs(obs)
@@ -168,10 +201,15 @@ class CudaVecEnv(object):
             raise RuntimeError("step_wait called without step_async")
         self.waiting = False
         obs, rew, done, info = self._pending
-        self._pending = None
+        fobs, self._pending, self._final_pending = self._final_pending, None, None
         if self.to_numpy:
             torch.cuda.current_stream(self.env.device).synchronize()
+            if fobs is not None:
+                return (self._views[0], self._views[1], self._views[2],
+                        InfoBatch(self._views[3], self._fobs_view, self._views[2]))
             return (self._views[0], self._views[1], self._views[2], InfoBatch(self._views[3]))
+        if fobs is not None:
+            return obs, rew, done, InfoBatch(info["individual_reward"], fobs, done)
         return obs, rew, done, InfoBatch(info["individual_reward"])
 
     def step(self, actions):

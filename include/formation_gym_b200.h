@@ -172,6 +172,22 @@ typedef struct fg_targets {
     int32_t count;             /* K >= 1 */
 } fg_targets;
 
+/* Terminal block (the *_final entry points): caller-owned DEVICE arrays in the entry point's real type, shaped like the
+ * state arrays.  When a single-step call with auto_reset ends env e's episode, the kernel copies env e's post-step
+ * state -- what the call returns with auto_reset == 0 -- into the block before the auto-reset overwrites it.  Entries
+ * of envs whose episode did not end are not written; the mask of written envs is the step's own done[e*N].  Every
+ * episode ends on the time limit (environment.py:172-177), so this is the state s_T a trainer bootstraps V(s_T) from
+ * (baselines' infos[e]['terminal_observation']; fg_final_obs below). */
+typedef struct fg_final {
+    void* pos;                 /* [E,N,2] */
+    void* vel;                 /* [E,N,2] */
+    void* comm;                /* [E,N,2], non-silent agents only (ignored for silent ones) */
+    void* ideal_shape;         /* [E,N,2], formation_hd_env only */
+    void* ideal_vel;           /* [E,2], formation_hd_env only */
+    void* landmarks;           /* [E,L,2], every other scenario (formation_hd_obs_env: goals, then the obstacles at their
+                                  post-step positions) */
+} fg_final;
+
 int fg_abi_version(void);
 const char* fg_last_error(void);
 
@@ -325,6 +341,37 @@ int fg_step_policy_targets(const fg_params* p, const fg_buffers* b, int scenario
 int fg_step_policy_targets_f64(const fg_params* p, const fg_buffers* b, int scenario, int E, int N, int L,
                                int n_steps, int num_agents_per_layer, int auto_reset, uint64_t seed, uint32_t tick,
                                uint32_t env_offset, void* stream, const fg_targets* t);
+
+/* fg_step_fused_targets / fg_step_policy_targets that also record the terminal state of every env whose episode ends
+ * in this call into the terminal block f (fg_final above).  f == NULL is exactly the _targets call; t == NULL is
+ * allowed (no bank).  Everything the call computes -- obs, reward, done, indiv, state, step, episode statistics,
+ * nan_flag, the Philox draws -- is bit for bit the call without a block.  FG_ERR_ARG, before any device call, when
+ * f != NULL and: auto_reset == 0 or n_steps != 1; pos or vel is NULL; formation_hd_env lacks ideal_shape or
+ * ideal_vel; another scenario lacks landmarks; non-silent agents lack comm; a pointer is not 8-byte (fp32) /
+ * 16-byte (fp64) aligned.  The target-bank checks are those of the _targets calls. */
+int fg_step_fused_final(const fg_params* p, const fg_buffers* b, int scenario, int E, int N, int L,
+                        int n_steps, int random_actions, int auto_reset, uint64_t seed, uint32_t tick,
+                        uint32_t env_offset, void* stream, const fg_targets* t, const fg_final* f);
+int fg_step_fused_final_f64(const fg_params* p, const fg_buffers* b, int scenario, int E, int N, int L,
+                            int n_steps, int random_actions, int auto_reset, uint64_t seed, uint32_t tick,
+                            uint32_t env_offset, void* stream, const fg_targets* t, const fg_final* f);
+int fg_step_policy_final(const fg_params* p, const fg_buffers* b, int scenario, int E, int N, int L, int n_steps,
+                         int num_agents_per_layer, int auto_reset, uint64_t seed, uint32_t tick,
+                         uint32_t env_offset, void* stream, const fg_targets* t, const fg_final* f);
+int fg_step_policy_final_f64(const fg_params* p, const fg_buffers* b, int scenario, int E, int N, int L,
+                             int n_steps, int num_agents_per_layer, int auto_reset, uint64_t seed, uint32_t tick,
+                             uint32_t env_offset, void* stream, const fg_targets* t, const fg_final* f);
+
+/* Terminal observations: obs [E,N,D] rows of every env with done[e*N] != 0, computed from the terminal block f by the
+ * observation code of fg_obs_reward -- bit-identical to the rows the same step writes with auto_reset == 0.  Rows of
+ * other envs are unspecified (a CTA holding an ended env also rewrites its other envs' rows).  Writes no other memory:
+ * no reward, no landmark side effect, no nan_flag.  A CTA whose envs all have done == 0 exits before any observation
+ * work, so a call after a step where no episode ended costs about one launch.  Same FG_ERR_ARG rules for f as the
+ * _final steps (without the auto_reset / n_steps ones); done and obs must be non-null. */
+int fg_final_obs(const fg_params* p, const fg_final* f, const uint8_t* done, void* obs, int scenario, int E, int N,
+                 int L, void* stream);
+int fg_final_obs_f64(const fg_params* p, const fg_final* f, const uint8_t* done, void* obs, int scenario, int E, int N,
+                     int L, void* stream);
 
 /* Diagnostics, not on the step path: FP32 pipe probes used by bench.py to MEASURE the FP32 peak the
  * large-N step+reward kernel is graded against (BASELINE.json north_star: "% of FP32 peak at 243
