@@ -129,6 +129,11 @@ int fg_final_obs(const fg_params* p, const fg_final* f, const uint8_t* done, voi
     return final_obs_impl<float>(p, f, done, obs, scenario, E, N, L, stream);
 }
 
+int fg_obs_gather(const fg_params* p, const fg_final* states, long long R, const int64_t* rows, int B, void* obs,
+                  int scenario, int N, int L, void* stream) {
+    return obs_gather_impl<float>(p, states, R, rows, B, obs, scenario, N, L, stream);
+}
+
 int fg_reset(const fg_params* p, const fg_buffers* b, int scenario, int E, int N, int L, const uint8_t* mask,
              uint64_t seed, uint32_t tick, uint32_t env_offset, void* stream) {
     return reset_impl<float>(p, b, scenario, E, N, L, mask, seed, tick, env_offset, stream, nullptr);

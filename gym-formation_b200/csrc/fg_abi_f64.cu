@@ -48,6 +48,11 @@ int fg_final_obs_f64(const fg_params* p, const fg_final* f, const uint8_t* done,
     return final_obs_impl<double>(p, f, done, obs, scenario, E, N, L, stream);
 }
 
+int fg_obs_gather_f64(const fg_params* p, const fg_final* states, long long R, const int64_t* rows, int B, void* obs,
+                      int scenario, int N, int L, void* stream) {
+    return obs_gather_impl<double>(p, states, R, rows, B, obs, scenario, N, L, stream);
+}
+
 int fg_reset_f64(const fg_params* p, const fg_buffers* b, int scenario, int E, int N, int L, const uint8_t* mask,
                  uint64_t seed, uint32_t tick, uint32_t env_offset, void* stream) {
     return reset_impl<double>(p, b, scenario, E, N, L, mask, seed, tick, env_offset, stream, nullptr);

@@ -608,6 +608,33 @@ int final_obs_impl(const fg_params* p, const fg_final* f, const uint8_t* done, v
     return launch<T, false, true>(a, scenario, p, stream);
 }
 
+// Observations of sampled state records (fg_obs_gather): the same pass on a block of R records, in gather mode -- output
+// slot b of the tile kernel reads record rows[b] (fg_kernels.cuh KArgs::gth_rows).
+template <typename T>
+int obs_gather_impl(const fg_params* p, const fg_final* s, long long R, const int64_t* rows, int B, void* obs,
+                    int scenario, int N, int L, void* stream) {
+    NvtxRange nvtx_("fg_obs_gather");
+    if (!s) return fail(FG_ERR_ARG, "fg_obs_gather: the state block must be non-null%s");
+    if (!rows || !obs) return fail(FG_ERR_ARG, "fg_obs_gather: rows / obs must be non-null%s");
+    if (R < 1 || B < 1) return fail(FG_ERR_ARG, "fg_obs_gather: R and B must be >= 1%s");
+    int rc = check_final<T>(s, p, scenario, 1, 1, false, "fg_obs_gather");
+    if (rc) return rc;
+    if (((uintptr_t)rows % sizeof(int64_t)) != 0) return fail(FG_ERR_ARG, "fg_obs_gather: rows must be 8-byte aligned%s");
+    fg_buffers b;
+    memset(&b, 0, sizeof(b));
+    b.pos = s->pos; b.vel = s->vel; b.obs = obs;
+    if (p && !p->silent) b.comm = s->comm;
+    if (scenario == FG_SCENARIO_HD) { b.ideal_shape = s->ideal_shape; b.ideal_vel = s->ideal_vel; }
+    else b.landmarks = s->landmarks;                                // (hd: no landmark side effect)
+    fg::KArgs<T> a;
+    rc = fill_args<T>(a, p, &b, scenario, B, N, L, 0, 0, 0);        // E = B output slots
+    if (rc) return rc;
+    set_final<T>(a, s, p, scenario);
+    a.gth_rows = rows; a.gth_count = R;                             // reward, step, done, nan_flag, lmv: NULL above
+    if (scenario == FG_SCENARIO_HD_OBSTACLE) return launch_obstacle<T, false>(a, stream);
+    return launch<T, false, true>(a, scenario, p, stream);
+}
+
 template <typename T>
 int step_fused_impl(const fg_params* p, const fg_buffers* b, int scenario, int E, int N, int L, int n_steps,
                     int random_actions, int auto_reset, uint64_t seed, uint32_t tick, uint32_t env_offset,

@@ -87,11 +87,26 @@ template <typename T> struct KArgs {
     R2* fin_pos; R2* fin_vel; R2* fin_comm;
     R2* fin_shape; R2* fin_ivel; R2* fin_lm;
     const uint8_t* fin_done;         // fg_final_obs: done [E,N] of the step
+    // gather mode of the observation pass (fg_obs_gather; read only by the EXT && !PHYS instantiations): the state is a
+    // block of gth_count records (fin_* == pos / vel / ... shaped [R, ...]) and output slot b takes record gth_rows[b];
+    // a slot whose index is outside [0, gth_count) reads nothing and gets NaN state.  gth_rows == NULL = off.
+    const int64_t* gth_rows;
+    long long gth_count;
 };
 
-// An instantiation with the reset extension (template flag EXT) runs when a target bank or a terminal block is set.
+// An instantiation with the reset extension (template flag EXT) runs when a target bank, a terminal block or a gather
+// row list is set.
 template <typename T>
-__host__ __device__ __forceinline__ bool reset_ext(const KArgs<T>& a) { return a.tgt_count > 0 || a.fin_pos != nullptr; }
+__host__ __device__ __forceinline__ bool reset_ext(const KArgs<T>& a) {
+    return a.tgt_count > 0 || a.fin_pos != nullptr || a.gth_rows != nullptr;
+}
+
+// Gather mode: record of output slot b, or -1 when its index names no record (then the slot reads nothing).
+template <typename T>
+__device__ __forceinline__ long long gather_record(const KArgs<T>& a, int b) {
+    const long long r = a.gth_rows[b];
+    return (r >= 0 && r < a.gth_count) ? r : -1;
+}
 
 // Task of env e (global id ge) at a reset with tick tk: tgt_index[e] when it names an entry of the bank, else
 // drawn uniformly from Philox.  Only called when tgt_count > 0.
@@ -301,9 +316,20 @@ __global__ void __launch_bounds__(kBlock, (OM == 3 && SCN == kScnBasic) ? 5 : (O
     const size_t g = (size_t)e * N + i;                       // global agent index
     const uint32_t ge = a.env_offset + (uint32_t)e;           // global env id (RNG counter)
 
-    if constexpr (FINOBS) {                                   // rows only where an episode ended (EPC <= kBlock)
-        if (!__syncthreads_or(t < nvalid && a.fin_done[(size_t)(tile0 + t) * N] != 0)) return;
+    // Gather mode (FINOBS with gth_rows): this thread reads agent i of record rec = gth_rows[e] (64-bit addressing: a
+    // block of T x E records passes 2^32 bytes quickly); rec < 0 names no record: NaN state, nothing is read.  The rows
+    // still leave at the tile position e, so the observation writers below are those of fg_final_obs.
+    long long rec = e;
+    if constexpr (FINOBS) {
+        if (a.gth_rows) {
+            if (active) rec = gather_record(a, e);
+        } else if (!__syncthreads_or(t < nvalid && a.fin_done[(size_t)(tile0 + t) * N] != 0)) {
+            return;                                           // rows only where an episode ended (EPC <= kBlock)
+        }
     }
+    const size_t gs = FINOBS ? (size_t)rec * N + i : g;       // agent index of the state read
+    const bool miss = FINOBS && rec < 0;
+    const R2 nan2 = O::make((T)NAN, (T)NAN);
 
     if (HET) {
         for (int q = t; q < N; q += kBlock) {
@@ -337,8 +363,8 @@ __global__ void __launch_bounds__(kBlock, (OM == 3 && SCN == kScnBasic) ? 5 : (O
     R2 p = O::make((T)0, (T)0), v = p, u = p, uc = p;
     int stp = 0;
     if (active) {
-        p = a.pos[g];
-        v = a.vel[g];
+        p = miss ? nan2 : a.pos[gs];
+        v = miss ? nan2 : a.vel[gs];
         if (PHYS && !a.random_actions) {
             u = a.act[g * a.act_r2];
             if (a.act_r2 > 1) uc = a.act[g * a.act_r2 + 1];
@@ -346,26 +372,28 @@ __global__ void __launch_bounds__(kBlock, (OM == 3 && SCN == kScnBasic) ? 5 : (O
         if (PHYS) s_old[t] = a.cpos ? a.cpos[g] : p; else { s_new[t] = p; s_v[t] = v; }
         if (OBSREW) {
             if (SCN == kScnHD) {
-                const R2 S0 = a.shape[g];
+                const R2 S0 = miss ? nan2 : a.shape[gs];
                 s_s[t] = S0;
                 if constexpr (FP) { RN(le, i, 3) = (float)S0.x; RN(le, i, 4) = (float)S0.y; }
                 if constexpr (OM == 2) {
                     if (a.row_early && !a.row_chunk) {   // static row images [comm zeros (N-1) | ideal_shape (N) | ideal_vel], both phases
                         R2* im0 = s_rt_img + (size_t)le * 2 * rt_img;
                         R2* im1 = im0 + rt_img;
+                        // (fg_obs_gather: a slot without a record gets NaN in place of the comm zeros too)
+                        const R2 cz = miss ? nan2 : O::make((T)0, (T)0);
                         im0[N - 1 + i] = S0; im1[N - 1 + i] = S0;
-                        if (i < N - 1) { im0[i] = O::make((T)0, (T)0); im1[i] = O::make((T)0, (T)0); }
+                        if (i < N - 1) { im0[i] = cz; im1[i] = cz; }
                     }
                 }
             }
             if (a.step) stp = a.step[e];
-            if (!PHYS) s_c[t] = a.comm ? a.comm[g] : O::make((T)0, (T)0);
+            if (!PHYS) s_c[t] = miss ? nan2 : (a.comm ? a.comm[gs] : O::make((T)0, (T)0));
         }
     }
     if (OBSREW) {
         if (SCN == kScnHD) {
             if (active && i == 0) {
-                const R2 iv0 = a.ivel[e];
+                const R2 iv0 = miss ? nan2 : a.ivel[FINOBS ? (size_t)rec : (size_t)e];
                 s_iv[le] = iv0;
                 if constexpr (OM == 2) {
                     if (a.row_early && !a.row_chunk) {
@@ -373,6 +401,12 @@ __global__ void __launch_bounds__(kBlock, (OM == 3 && SCN == kScnBasic) ? 5 : (O
                         im0[2 * N - 1] = iv0; im0[rt_img + 2 * N - 1] = iv0;
                     }
                 }
+            }
+        } else if (FINOBS && a.gth_rows) {
+            for (int q = t; q < nvalid * L; q += kBlock) {
+                const int qe = (int)fastdiv((uint32_t)q, a.magic_l), k = q - qe * L;
+                const long long r = gather_record(a, tile0 + qe);
+                s_s[q] = r < 0 ? nan2 : a.lm[(size_t)r * L + k];
             }
         } else {
             for (int q = t; q < nvalid * L; q += kBlock) s_s[q] = a.lm[(size_t)tile0 * L + q];
@@ -427,7 +461,11 @@ __global__ void __launch_bounds__(kBlock, (OM == 3 && SCN == kScnBasic) ? 5 : (O
                 for (int m = sl; m < N - 1; m += NS) {
                     const R2 pj = P[m + (m >= ri)];
                     row[1 + m] = O::make(O::sub(pj.x, pi.x), O::sub(pj.y, pi.y));   // other_pos (formation_hd_env.py:55)
-                    row[N + m] = zero2;                                             // comm of the others (silent)
+                    // comm of the others (silent: zeros; fg_obs_gather reads s_c, NaN for a slot without a record).
+                    // (if constexpr: the product instantiations' lambda must not capture s_c)
+                    R2 cz = zero2;
+                    if constexpr (FINOBS) cz = s_c[rle * N + m + (m >= ri)];
+                    row[N + m] = cz;
                 }
                 for (int m = sl; m < N; m += NS) row[2 * N - 1 + m] = S[m];         // ideal_shape.flatten()
                 if (sl == 0) { row[0] = s_v[R]; row[3 * N - 1] = s_iv[rle]; }       // p_vel, ideal_vel
@@ -748,7 +786,7 @@ __global__ void __launch_bounds__(kBlock, (OM == 3 && SCN == kScnBasic) ? 5 : (O
                         img[off + k] = O::make(O::sub(pj.x, pi.x), O::sub(pj.y, pi.y));
                     }
                     if (lane_ == 0) {
-                        if (!odd) { img[0] = s_v[row]; img[N] = O::make((T)0, (T)0); }
+                        if (!odd) { img[0] = s_v[row]; img[N] = FINOBS ? s_c[rle * N + (ri == 0)] : O::make((T)0, (T)0); }
                         else if (row > 0) { img[0] = s_iv[ri == 0 ? rle - 1 : rle]; img[1] = s_v[row]; }   // previous row's env
                         else O::stcs(out, s_v[row]);
                         if (!odd && row == nrows - 1) O::stcs(out + 3 * N - 1, s_iv[rle]);   // nobody follows
@@ -1178,7 +1216,9 @@ __global__ void __launch_bounds__(kBlock, (OM == 3 && SCN == kScnBasic) ? 5 : (O
                     R2* im0 = s_rt_img + (size_t)qe * 2 * rt_img;
                     R2* im1 = im0 + rt_img;
                     for (int k = t; k < 2 * N; k += kBlock) {
-                        R2 val = (k < N - 1) ? O::make((T)0, (T)0) : (k < 2 * N - 1 ? s_s[qe * N + (k - (N - 1))] : s_iv[qe]);
+                        // (comm zeros of silent agents; fg_obs_gather takes them from s_c: NaN for a slot without a record)
+                        R2 val = (k < N - 1) ? (FINOBS ? s_c[qe * N + k] : O::make((T)0, (T)0))
+                                             : (k < 2 * N - 1 ? s_s[qe * N + (k - (N - 1))] : s_iv[qe]);
                         im0[k] = val; im1[k] = val;
                     }
                 }

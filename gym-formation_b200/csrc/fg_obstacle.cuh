@@ -80,25 +80,44 @@ __global__ void __launch_bounds__(kBlock, 2) k_step_obst(const __grid_constant__
     const T cut_ao = dmin_ao + a.kcut * a.margin, cut_oo = dmin_oo + a.kcut * a.margin;
     const T cut2_ao = cut_ao * cut_ao, cut2_oo = cut_oo * cut_oo;
 
-    if constexpr (FINOBS) {                                  // rows only where an episode ended (EPC <= kBlock)
-        if (!__syncthreads_or(t < nvalid && a.fin_done[(size_t)(tile0 + t) * N] != 0)) return;
+    // Gather mode (fg_obs_gather, as in k_step): slot e reads record gth_rows[e] with 64-bit addressing; a slot without
+    // a record reads nothing and gets NaN state.
+    long long rec = e;
+    if constexpr (FINOBS) {
+        if (a.gth_rows) {
+            if (active) rec = gather_record(a, e);
+        } else if (!__syncthreads_or(t < nvalid && a.fin_done[(size_t)(tile0 + t) * N] != 0)) {
+            return;                                          // rows only where an episode ended (EPC <= kBlock)
+        }
     }
+    const R2 nan2 = O_::make((T)NAN, (T)NAN);
 
     R2 p = O_::make((T)0, (T)0), v = p, u = p;
     int stp = 0;
     if (active) {
-        p = a.pos[g];
-        v = a.vel[g];
+        const size_t gs = FINOBS ? (size_t)rec * N + i : g;
+        p = (FINOBS && rec < 0) ? nan2 : a.pos[gs];
+        v = (FINOBS && rec < 0) ? nan2 : a.vel[gs];
         if (PHYS && !a.random_actions) u = a.act[g];
         if (PHYS) s_old[t] = p; else { s_new[t] = p; s_v[t] = v; }
         if (a.step) stp = a.step[e];
     }
-    for (int q = t; q < nvalid * L; q += kBlock) s_lm[q] = a.lm[(size_t)tile0 * L + q];
-    for (int q = t; q < nvalid * NO; q += kBlock) {
-        const int qe = q / NO, k = q - qe * NO;
-        const size_t gi = (size_t)(tile0 + qe) * L + LG + k;
-        s_ov[q] = a.lmv ? a.lmv[gi] : O_::make((T)0, (T)0);
-        if (!PHYS) s_on[q] = a.lm[gi];
+    if (FINOBS && a.gth_rows) {                              // goals and obstacles of each slot's record
+        for (int q = t; q < nvalid * L; q += kBlock) {
+            const int qe = q / L, k = q - qe * L;
+            const long long r = gather_record(a, tile0 + qe);
+            const R2 l = r < 0 ? nan2 : a.lm[(size_t)r * L + k];
+            s_lm[q] = l;
+            if (k >= LG) { s_on[qe * NO + (k - LG)] = l; s_ov[qe * NO + (k - LG)] = O_::make((T)0, (T)0); }
+        }
+    } else {
+        for (int q = t; q < nvalid * L; q += kBlock) s_lm[q] = a.lm[(size_t)tile0 * L + q];
+        for (int q = t; q < nvalid * NO; q += kBlock) {
+            const int qe = q / NO, k = q - qe * NO;
+            const size_t gi = (size_t)(tile0 + qe) * L + LG + k;
+            s_ov[q] = a.lmv ? a.lmv[gi] : O_::make((T)0, (T)0);
+            if (!PHYS) s_on[q] = a.lm[gi];
+        }
     }
 
     if (PHYS) __syncthreads();                               // the obstacle positions above, for the checks below
@@ -393,6 +412,8 @@ __global__ void __launch_bounds__(kBlock, 2) k_step_obst(const __grid_constant__
                     int j = k - (1 + LG + NO); j += (j >= ri);
                     const R2 pj = s_new[rle * N + j], pi = s_new[row];
                     val = O_::make(O_::sub(pj.x, pi.x), O_::sub(pj.y, pi.y));
+                } else if (FINOBS && a.gth_rows) {
+                    val = gather_record(a, tile0 + rle) < 0 ? nan2 : O_::make((T)0, (T)0);   // comm zeros; NaN slot
                 } else val = O_::make((T)0, (T)0);
                 out[q] = val;
             }

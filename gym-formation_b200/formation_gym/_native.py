@@ -27,6 +27,7 @@ EXPORTS = [
     "fg_reset_targets", "fg_reset_targets_f64", "fg_step_fused_targets", "fg_step_fused_targets_f64",
     "fg_step_policy_targets", "fg_step_policy_targets_f64", "fg_step_fused_final", "fg_step_fused_final_f64",
     "fg_step_policy_final", "fg_step_policy_final_f64", "fg_final_obs", "fg_final_obs_f64",
+    "fg_obs_gather", "fg_obs_gather_f64",
 ]
 
 
@@ -128,6 +129,8 @@ def load():
         getattr(lib, "fg_step_policy_final" + sfx).argtypes = \
             [P(fg_params), P(fg_buffers), I, I, I, I, I, I, I, U64, U32, U32, VP, P(fg_targets), P(fg_final)]
         getattr(lib, "fg_final_obs" + sfx).argtypes = [P(fg_params), P(fg_final), VP, VP, I, I, I, I, VP]
+        getattr(lib, "fg_obs_gather" + sfx).argtypes = \
+            [P(fg_params), P(fg_final), C.c_longlong, VP, I, VP, I, I, I, VP]
         getattr(lib, "fg_random_actions" + sfx).argtypes = [VP, I, I, U64, U32, U32, VP, VP]
         getattr(lib, "fg_policy_bfs" + sfx).argtypes = [VP, VP, VP, VP, I, I, I, VP]
         getattr(lib, "fg_pair_distances" + sfx).argtypes = [VP, VP, I, I, VP, VP, VP, VP, VP]

@@ -414,6 +414,62 @@ class BatchedFormationEnv:
             self.launches += 1
         return self._final_obs
 
+    def state_record_keys(self):
+        """Names of the state arrays an observation is computed from: ``pos``, ``vel``, ``comm`` (non-silent agents),
+        then ``ideal_shape`` and ``ideal_vel`` (formation_hd_env) or ``landmarks`` (every other scenario)."""
+        keys = ["pos", "vel"] + ([] if self.silent else ["comm"])
+        return keys + (["ideal_shape", "ideal_vel"] if self.scn == nat.FG_SCENARIO_HD else ["landmarks"])
+
+    def gather_observations(self, states, rows, out=None):
+        """Observations of sampled state records (``fg_obs_gather``): ``out [B,N,D]`` where slot b holds the rows of
+        record ``rows[b]``, bit-identical to what a step returned when that state was current.  ``states`` is a dict
+        (or an object with attributes) of record tensors named by ``state_record_keys()``, each shaped like the live
+        state with R records in place of E (``ideal_vel [R,2]``, ``landmarks [R,L,2]``); ``rows`` is an int64 device
+        tensor [B].  Indices may repeat; one outside [0, R) gives slot b a row block of NaN and reads nothing.  Shapes,
+        dtypes and devices are checked before the call; one launch, no synchronisation."""
+        get = states.get if isinstance(states, dict) else (lambda k: getattr(states, k, None))
+        arrs, R = {}, None
+        for k in self.state_record_keys():
+            t = get(k)
+            if not torch.is_tensor(t):
+                raise ValueError("states[%r] must be a tensor" % k)
+            if t.dtype != self.dtype:
+                raise ValueError("states[%r] must have dtype %s, got %s" % (k, self.dtype, t.dtype))
+            if R is None:
+                R = int(t.shape[0]) if t.dim() > 0 else 0
+            want = {"ideal_vel": (R, 2), "landmarks": (R, self.L, 2)}.get(k, (R, self.N, 2))
+            if tuple(t.shape) != want:
+                raise ValueError("states[%r] must have shape %s, got %s" % (k, want, tuple(t.shape)))
+            if not t.is_contiguous():
+                raise ValueError("states[%r] must be contiguous" % k)
+            arrs[k] = t
+        if R < 1:
+            raise ValueError("the state block must hold at least one record")
+        if not torch.is_tensor(rows) or rows.dtype != torch.int64 or rows.dim() != 1 or rows.shape[0] < 1:
+            raise ValueError("rows must be a non-empty 1-D int64 tensor")
+        if not rows.is_contiguous():
+            raise ValueError("rows must be contiguous")
+        B = int(rows.shape[0])
+        if out is not None:
+            if not torch.is_tensor(out) or out.dtype != self.dtype or tuple(out.shape) != (B, self.N, self.D):
+                raise ValueError("out must be a %s tensor of shape %s" % (self.dtype, (B, self.N, self.D)))
+            if not out.is_contiguous():
+                raise ValueError("out must be contiguous")
+        for name, t in list(arrs.items()) + [("rows", rows)] + ([("out", out)] if out is not None else []):
+            if t.device != self.device:
+                raise ValueError("%s must be on %s, got %s" % (name, self.device, t.device))
+        if out is None:
+            out = torch.empty(B, self.N, self.D, device=self.device, dtype=self.dtype)
+        f = nat.fg_final()
+        for k, t in arrs.items():
+            setattr(f, k, nat.ptr(t))
+        with self._on_device():
+            rc = self._fn("fg_obs_gather")(C.byref(self.params), C.byref(f), R, nat.ptr(rows), B, nat.ptr(out),
+                                           self.scn, self.N, self.L, self._stream())
+            nat.check(rc, "fg_obs_gather")
+            self.launches += 1
+        return out
+
     def nan_envs(self, clear=False):
         """Indices of envs that hit the reference's documented failure mode since the flags were last cleared:
         coincident agents make ``delta_pos / dist`` NaN (core.py:312) and the env's state and rewards stay NaN until

@@ -373,6 +373,21 @@ int fg_final_obs(const fg_params* p, const fg_final* f, const uint8_t* done, voi
 int fg_final_obs_f64(const fg_params* p, const fg_final* f, const uint8_t* done, void* obs, int scenario, int E, int N,
                      int L, void* stream);
 
+/* Observations of sampled state records (a replay buffer that stores states, not observations).  `states` is a block of
+ * R records laid out like a terminal block with R in place of E: pos / vel / comm (non-silent agents) [R,N,2], and
+ * ideal_shape [R,N,2] + ideal_vel [R,2] (formation_hd_env) or landmarks [R,L,2] (every other scenario;
+ * formation_hd_obs_env: goals, then obstacles).  rows: DEVICE int64 [B].  obs [B,N,D]: slot b gets the observation rows
+ * of record rows[b], computed by the observation code of fg_obs_reward -- bit-identical to what fg_obs_reward writes for
+ * that state, which is what the step returned when the state was current.  Indices may repeat and come in any order;
+ * records are addressed in 64 bits.  An index outside [0, R), negative included, reads nothing and gives slot b a row
+ * block of NaN.  Writes no other memory: no reward, no landmark side effect, no nan_flag.  FG_ERR_ARG, before any
+ * device call, when states, rows or obs is NULL, R < 1 or B < 1, or on the block rules of fg_final_obs (missing or
+ * misaligned arrays); rows must be 8-byte aligned. */
+int fg_obs_gather(const fg_params* p, const fg_final* states, long long R, const int64_t* rows, int B, void* obs,
+                  int scenario, int N, int L, void* stream);
+int fg_obs_gather_f64(const fg_params* p, const fg_final* states, long long R, const int64_t* rows, int B, void* obs,
+                      int scenario, int N, int L, void* stream);
+
 /* Diagnostics, not on the step path: FP32 pipe probes used by bench.py to MEASURE the FP32 peak the
  * large-N step+reward kernel is graded against (BASELINE.json north_star: "% of FP32 peak at 243
  * agents"; MEASURED_PEAKS.json holds no FP32 figure).  variant 0: scalar FFMA (2 flop/lane/instr),
