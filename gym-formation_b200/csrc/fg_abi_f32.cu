@@ -39,6 +39,8 @@ Switches& switches() {
     (void)init;
     return sw;
 }
+
+int nvtx_enabled() { return switches().nvtx.load(std::memory_order_relaxed); }
 }  // namespace fgabi
 
 extern "C" {

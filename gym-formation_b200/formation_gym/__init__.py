@@ -15,7 +15,7 @@ call that needs the device raises).
 import importlib
 
 __all__ = ["make_env", "make_batched_env", "make_vec_env", "ezpolicy", "get_action_BFS", "MultiAgentEnv",
-           "BatchedFormationEnv", "CudaVecEnv", "StateReplayBuffer", "SCENARIOS"]
+           "BatchedFormationEnv", "CudaVecEnv", "StateReplayBuffer", "PrioritizedStateReplayBuffer", "SCENARIOS"]
 
 SCENARIOS = ("basic_formation_env", "formation_hd_env", "formation_hd_partial_env",
              "formation_hd_partial_range_env", "formation_hd_obs_env")
@@ -176,6 +176,9 @@ def __getattr__(name):
     if name == "StateReplayBuffer":
         from .replay import StateReplayBuffer
         return StateReplayBuffer
+    if name == "PrioritizedStateReplayBuffer":
+        from .replay import PrioritizedStateReplayBuffer
+        return PrioritizedStateReplayBuffer
     if name == "MultiAgentEnv":
         from .environment import MultiAgentEnv
         return MultiAgentEnv

@@ -27,7 +27,8 @@ EXPORTS = [
     "fg_reset_targets", "fg_reset_targets_f64", "fg_step_fused_targets", "fg_step_fused_targets_f64",
     "fg_step_policy_targets", "fg_step_policy_targets_f64", "fg_step_fused_final", "fg_step_fused_final_f64",
     "fg_step_policy_final", "fg_step_policy_final_f64", "fg_final_obs", "fg_final_obs_f64",
-    "fg_obs_gather", "fg_obs_gather_f64",
+    "fg_obs_gather", "fg_obs_gather_f64", "fg_per_layout", "fg_per_fill", "fg_per_update", "fg_per_sample",
+    "fg_per_sample_f64",
 ]
 
 
@@ -82,6 +83,14 @@ class fg_final(C.Structure):
                 ("ideal_vel", C.c_void_p), ("landmarks", C.c_void_p)]
 
 
+class fg_per(C.Structure):
+    """Prioritized-replay sum tree (the ``fg_per_*`` entry points): device arrays of caller-owned memory sized by
+    ``fg_per_layout``."""
+    _fields_ = [("leaf", C.c_void_p), ("sum", C.c_void_p), ("min", C.c_void_p), ("max_leaf", C.c_void_p),
+                ("stamp", C.c_void_p), ("prev", C.c_void_p), ("scratch", C.c_void_p),
+                ("slots", C.c_longlong), ("envs", C.c_longlong)]
+
+
 _lib = None
 
 
@@ -131,9 +140,15 @@ def load():
         getattr(lib, "fg_final_obs" + sfx).argtypes = [P(fg_params), P(fg_final), VP, VP, I, I, I, I, VP]
         getattr(lib, "fg_obs_gather" + sfx).argtypes = \
             [P(fg_params), P(fg_final), C.c_longlong, VP, I, VP, I, I, I, VP]
+        getattr(lib, "fg_per_sample" + sfx).argtypes = \
+            [P(fg_per), VP, I, C.c_double, VP, VP, VP, I, I, VP, VP, VP, VP, VP, VP, VP, VP, VP, VP]
         getattr(lib, "fg_random_actions" + sfx).argtypes = [VP, I, I, U64, U32, U32, VP, VP]
         getattr(lib, "fg_policy_bfs" + sfx).argtypes = [VP, VP, VP, VP, I, I, I, VP]
         getattr(lib, "fg_pair_distances" + sfx).argtypes = [VP, VP, I, I, VP, VP, VP, VP, VP]
+    LL = C.c_longlong
+    lib.fg_per_layout.argtypes = [LL, LL, P(LL), P(I), P(LL)]
+    lib.fg_per_fill.argtypes = [P(fg_per), LL, LL, LL, I, LL, VP]
+    lib.fg_per_update.argtypes = [P(fg_per), VP, VP, VP, I, I, C.c_double, C.c_double, VP]
     lib.fg_obs_to_host.argtypes = [VP, VP, VP, VP, I, I, I, I, I, I, VP]
     lib.fg_fp32_probe.argtypes = [I, I, I, VP, VP]
     lib.fg_write_probe.argtypes = [I, VP, C.c_ulonglong, C.c_uint, I, VP]

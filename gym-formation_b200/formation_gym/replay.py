@@ -7,7 +7,12 @@ of ``obs`` and ``next_obs`` shrinks a transition by 2.4x at formation_hd_env N =
 ``sample`` turns the records back into observation rows with one ``fg_obs_gather`` launch, bit-identical to what the
 steps returned.
 """
+import ctypes as C
+import math
+
 import torch
+
+from . import _native as nat
 
 
 class StateReplayBuffer:
@@ -76,22 +81,24 @@ class StateReplayBuffer:
             v[j].copy_(getattr(env, ("final_" + k) if final else k))
 
     def _claim(self):
-        """Next ring slot; drops its own transition and the one whose s it held."""
+        """Next ring slot; drops its own transition and the one whose s it held.  Returns the slot and the slot of the
+        dropped child transition (-1: none)."""
         j = self._next
         self._valid.pop(j, None)
         c = self._child[j]
+        dropped = -1
         if c >= 0 and self._prev[c] == j and self._prev_stamp[c] == self._stamp[j]:
-            self._valid.pop(c, None)
+            dropped = c if self._valid.pop(c, None) is not None else -1
         self._child[j] = -1
         self._writes += 1
         self._stamp[j] = self._writes
         self._next = (j + 1) % self.capacity
         self._valid_dev = None
-        return j
+        return j, dropped
 
     def mark_start(self):
         """Snapshot the env's current state into the next slot as the start of a chain (no transition)."""
-        j = self._claim()
+        j, _ = self._claim()
         self._copy_state(j, self._S, False)
         self._prev[j] = -1
         self._head = j
@@ -106,7 +113,7 @@ class StateReplayBuffer:
         if tuple(actions.shape) != (env.E, env.N, env.act_dim):
             raise ValueError("actions must have shape %s, got %s" % ((env.E, env.N, env.act_dim), tuple(actions.shape)))
         h = self._head
-        j = self._claim()
+        j, _ = self._claim()
         self.actions[j].copy_(actions)
         self.reward[j].copy_(env.reward[..., 0])
         self.done[j].copy_(env.done[:, 0])
@@ -142,3 +149,150 @@ class StateReplayBuffer:
         obs = env.gather_observations(self.states, rows)
         return {"obs": obs[:B], "next_obs": obs[B:], "actions": self.actions[slot, e], "reward": self.reward[slot, e],
                 "done": done, "env_index": e, "slot": slot}
+
+
+class _PrioritizedBatch(dict):
+    """A ``PrioritizedStateReplayBuffer.sample`` result: a dict that remembers the buffer it came from."""
+    __slots__ = ("buffer",)
+
+
+class PrioritizedStateReplayBuffer(StateReplayBuffer):
+    """``StateReplayBuffer`` with proportional prioritized replay (PER, Schaul et al. 2016; the defaults are baselines'
+    ``PrioritizedReplayBuffer``): transition (slot j, env e) is drawn with probability ``p_je / sum p`` and weighted by
+    ``w = (min p / p_je) ** beta``, i.e. ``(N P)^-beta / max w``.
+
+    The priorities live on the device in a 32-ary sum/min tree (include/formation_gym_b200.h ``fg_per``): one fp64 leaf
+    per transition, 8.5 bytes per transition with the inner nodes, plus 4 bytes of update scratch.  ``add`` gives the
+    new transitions the largest priority written so far (initially 1), ``mark_start`` and the transitions a write drops
+    get 0.  A sample is one ``fg_per_sample`` launch (tree descent, weights, actions, reward, done and the record rows)
+    and one ``fg_obs_gather``; an update is a few launches; neither synchronises.
+
+    Usage::
+
+        buf = PrioritizedStateReplayBuffer(env, capacity, alpha=0.6)
+        env.reset(); buf.mark_start()
+        for t in range(steps):
+            env.step(act); buf.add(act)
+            b = buf.sample(B, beta)                    # + weights, index, stamp
+            td = q(b['obs'], b['actions']) - target(b)
+            loss = (b['weights'] * td ** 2).mean()
+            buf.update_priorities(b, td.detach())      # [B] fp32 / fp64: new priority (|td| + eps) ** alpha
+
+    An update entry whose transition was overwritten or dropped since the sample (the slot's stamp changed), or whose
+    td is NaN / inf, changes nothing; among entries for one transition the last one wins.
+
+    ``priorities`` is a view of the device leaves, so reading it costs nothing; it is for reading only.  The inner nodes
+    are not recomputed from a write through it, so the tree would then no longer sum its leaves: change priorities
+    with ``update_priorities`` (or ``.clone()`` the view before editing a copy).
+    """
+
+    def __init__(self, env, capacity, alpha=0.6, eps=1e-6):
+        alpha, eps = float(alpha), float(eps)
+        if not (math.isfinite(alpha) and alpha >= 0):
+            raise ValueError("alpha must be finite and >= 0, got %r" % alpha)
+        if not (math.isfinite(eps) and eps > 0):
+            raise ValueError("eps must be finite and > 0, got %r" % eps)
+        super().__init__(env, capacity)
+        self.alpha, self.eps = alpha, eps
+        T, E = self.capacity, env.E
+        self._lib = nat.load()
+        nodes, depth, scratch = C.c_longlong(), C.c_int(), C.c_longlong()
+        nat.check(self._lib.fg_per_layout(T, E, C.byref(nodes), C.byref(depth), C.byref(scratch)), "fg_per_layout")
+        self.depth = depth.value
+        kw = dict(device=env.device, dtype=torch.float64)
+        self._leaf = torch.zeros(T * E, **kw)
+        self._sum = torch.zeros(nodes.value, **kw)
+        self._min = torch.full((nodes.value,), float("inf"), **kw)
+        self._max_leaf = torch.ones(1, **kw)
+        self._stamp_dev = torch.zeros(T, dtype=torch.int64, device=env.device)
+        self._prev_dev = torch.full((T,), -1, dtype=torch.int64, device=env.device)
+        self._scratch = torch.zeros(scratch.value // 4, dtype=torch.int32, device=env.device)
+        t = self._tree = nat.fg_per()
+        for k in ("leaf", "sum", "min", "max_leaf", "scratch"):
+            setattr(t, k, nat.ptr(getattr(self, "_" + k)))
+        t.stamp, t.prev = nat.ptr(self._stamp_dev), nat.ptr(self._prev_dev)
+        t.slots, t.envs = T, E
+        self._dropped = -1
+
+    @property
+    def priorities(self):
+        """The leaves as a ``[T, E]`` fp64 view (0 where no transition).  Read-only by contract: a write through it
+        bypasses the tree (see the class docstring)."""
+        return self._leaf.view(self.capacity, self.env.E)
+
+    def _claim(self):
+        j, self._dropped = super()._claim()
+        return j, self._dropped
+
+    def _fill(self, valid):
+        j, env = self._head, self.env
+        with env._on_device():
+            rc = self._lib.fg_per_fill(C.byref(self._tree), j, self._prev[j], self._stamp[j], int(valid), self._dropped,
+                                       env._stream())
+        nat.check(rc, "fg_per_fill")
+
+    def mark_start(self):
+        super().mark_start()
+        self._fill(False)
+
+    def add(self, actions):
+        super().add(actions)
+        self._fill(True)
+
+    def sample(self, batch_size, beta=0.4, generator=None):
+        """``batch_size`` transitions drawn in proportion to their priorities (with replacement), on the device.
+        Returns the keys of ``StateReplayBuffer.sample`` plus ``weights`` [B] (env dtype, ``(min p / p) ** beta``) and
+        ``index``, ``stamp`` [B] (int64; what ``update_priorities`` reads).  No host synchronisation."""
+        B = int(batch_size)
+        if B < 1:
+            raise ValueError("batch_size must be >= 1")
+        beta = float(beta)
+        if not (math.isfinite(beta) and beta >= 0):
+            raise ValueError("beta must be finite and >= 0, got %r" % beta)
+        if not self._valid:
+            raise ValueError("the buffer holds no transition (mark_start(), then step and add())")
+        env = self.env
+        dev, dt = env.device, env.dtype
+        u = torch.rand(B, dtype=torch.float64, generator=generator, device=dev)
+        ids = torch.empty(6, B, dtype=torch.int64, device=dev)       # rows (s, s'), index, stamp, slot, env
+        done = torch.empty(B, dtype=torch.bool, device=dev)
+        w = torch.empty(B, dtype=dt, device=dev)
+        act = torch.empty(B, env.N, env.act_dim, dtype=dt, device=dev)
+        rew = torch.empty(B, env.N, dtype=dt, device=dev)
+        P = nat.ptr
+        with env._on_device():
+            rc = env._fn("fg_per_sample")(C.byref(self._tree), P(u), B, beta, P(self.done), P(self.actions),
+                                          P(self.reward), env.N, env.act_dim, P(ids[0]), P(ids[2]), P(ids[3]),
+                                          P(ids[4]), P(ids[5]), P(done), P(w), P(act), P(rew), env._stream())
+        nat.check(rc, "fg_per_sample")
+        obs = env.gather_observations(self.states, ids[:2].view(-1))
+        out = _PrioritizedBatch(obs=obs[:B], next_obs=obs[B:], actions=act, reward=rew, done=done, env_index=ids[5],
+                                slot=ids[4], weights=w, index=ids[2], stamp=ids[3])
+        out.buffer = self
+        return out
+
+    def update_priorities(self, batch, td_errors):
+        """Set the priorities of the transitions of ``batch`` (a ``sample`` result of this buffer) to
+        ``clamp((|td| + eps) ** alpha, 2**-1022, 2**960)``; ``td_errors`` is an fp32 / fp64 device tensor [B] (a
+        per-agent critic reduces its errors to one per transition first).  Entries whose transition was overwritten or
+        dropped since the sample, and NaN / inf entries, are skipped.  No host synchronisation."""
+        if not isinstance(batch, _PrioritizedBatch) or batch.buffer is not self:
+            raise ValueError("batch must be a sample() result of this buffer")
+        index, stamp = batch.get("index"), batch.get("stamp")
+        if not (torch.is_tensor(index) and torch.is_tensor(stamp) and index.dtype == stamp.dtype == torch.int64
+                and index.dim() == 1 and index.shape == stamp.shape and index.is_contiguous() and stamp.is_contiguous()
+                and index.device == stamp.device == self.env.device):
+            raise ValueError("batch['index'] / batch['stamp'] must be the int64 [B] device tensors sample() returned")
+        B = int(index.shape[0])
+        if not torch.is_tensor(td_errors) or td_errors.dtype not in (torch.float32, torch.float64):
+            raise ValueError("td_errors must be a float32 or float64 tensor")
+        if tuple(td_errors.shape) != (B,):
+            raise ValueError("td_errors must have shape %s, got %s" % ((B,), tuple(td_errors.shape)))
+        if td_errors.device != self.env.device:
+            raise ValueError("td_errors must be on %s, got %s" % (self.env.device, td_errors.device))
+        td = td_errors.contiguous()
+        env = self.env
+        with env._on_device():
+            rc = self._lib.fg_per_update(C.byref(self._tree), nat.ptr(index), nat.ptr(stamp), nat.ptr(td),
+                                         int(td.dtype == torch.float64), B, self.alpha, self.eps, env._stream())
+        nat.check(rc, "fg_per_update")

@@ -388,6 +388,62 @@ int fg_obs_gather(const fg_params* p, const fg_final* states, long long R, const
 int fg_obs_gather_f64(const fg_params* p, const fg_final* states, long long R, const int64_t* rows, int B, void* obs,
                       int scenario, int N, int L, void* stream);
 
+/* Prioritized replay over the transitions of a state-record replay buffer of `slots` slots x `envs` envs (proportional
+ * PER, Schaul et al. 2016, as in baselines' PrioritizedReplayBuffer): a 32-ary sum tree with a min per node.
+ *   Leaves: leaf[j*envs + e] > 0 (the priority) exactly when slot j, env e holds a transition; 0 otherwise.  M = slots *
+ *   envs <= 2^40.  Level 0 is the leaves, read as padded with zeros to a multiple of 32; node i of level k+1 reduces
+ *   nodes 32i .. 32i+31 of level k (children past the end of a level count as sum 0 / min +inf); levels 1 .. depth are
+ *   stored in `sum` / `min` bottom level first, the root (one node) last.  sum = the butterfly sum of the 32 children
+ *   (v_l = v_l + v_{l^off} for off = 16, 8, 4, 2, 1, then v_0: a __shfl_xor reduction); min = the minimum over the
+ *   nonzero leaves below, +inf for none.  The tree is a pure function of the leaves.
+ *   Caller-owned device memory, sized by fg_per_layout and initialised ONCE to: leaf 0, sum 0, min +inf, max_leaf 1.0,
+ *   stamp 0, prev -1, scratch 0 (the calls leave scratch 0 again).  Arrays 8-byte aligned, scratch 4-byte.
+ * None of the calls allocates or synchronises; every argument error returns FG_ERR_ARG before any device call. */
+typedef struct fg_per {
+    double* leaf;              /* [slots*envs] */
+    double* sum;               /* [nodes] internal nodes of every level, bottom level first, root last */
+    double* min;               /* [nodes] same layout */
+    double* max_leaf;          /* [1] running maximum of the leaf values fg_per_update wrote (initially 1.0) */
+    int64_t* stamp;            /* [slots] write count of each slot (fg_per_fill) */
+    int64_t* prev;             /* [slots] slot holding the s of slot j's transition, -1 for none */
+    void* scratch;             /* [scratch_bytes] duplicate resolution of fg_per_update */
+    long long slots, envs;
+} fg_per;
+
+/* Sizes of the tree of slots x envs leaves: internal nodes (all levels), depth (levels above the leaves, >= 1) and the
+ * scratch bytes.  FG_ERR_ARG when a pointer is NULL, slots or envs < 1, or slots * envs > 2^40.  Host only. */
+int fg_per_layout(long long slots, long long envs, long long* nodes, int* depth, long long* scratch_bytes);
+/* A slot was written: stamp[slot] = stamp, prev[slot] = prev, the leaves of `slot` = *max_leaf when valid (a transition:
+ * prev >= 0) else 0 (a chain start), the leaves of drop_slot (-1: none; the transition whose s `slot` held) = 0, then
+ * their ancestors.  FG_ERR_ARG unless 0 <= slot < slots, prev and drop_slot are -1 or another slot, valid is 0 / 1,
+ * stamp >= 0. */
+int fg_per_fill(const fg_per* t, long long slot, long long prev, long long stamp, int valid, long long drop_slot,
+                void* stream);
+/* Priority update for B sampled transitions: index [B] (leaf), stamp [B] (the slot stamp fg_per_sample returned), td [B]
+ * (fp32, or fp64 when td_f64 = 1; device).  Entry b is applied when td[b] is finite, 0 <= index[b] < M, the leaf is > 0
+ * and stamp[slot] still equals stamp[b]; among applied entries of one leaf the largest b wins.  The leaf becomes
+ * clamp((|td| + eps)^alpha, 2^-1022, 2^960), max_leaf the max of itself and the values written, then the ancestors are
+ * recomputed.  FG_ERR_ARG also when B < 1, alpha < 0, eps <= 0 or either is not finite. */
+int fg_per_update(const fg_per* t, const int64_t* index, const int64_t* stamp, const void* td, int td_f64, int B,
+                  double alpha, double eps, void* stream);
+/* B proportional draws: u [B] fp64 in [0, 1) (device), x = u * root.sum; from the root take the smallest child k with
+ * c_k > 0 and x < P_k (inclusive prefix sum), else the last child with c_k > 0, then x -= P_{k-1} clamped into [0, c_k).
+ * A zero leaf is never returned.  Per draw b, with leaf l = slot * envs + e: rows[b] = prev[slot] * envs + e and
+ * rows[B + b] = l + (done[l] ? M : 0) (the record rows of s and s' in StateReplayBuffer's block, for fg_obs_gather),
+ * index[b] = l, stamp_out[b] = stamp[slot], slot_out[b], env_out[b], done_out[b] = done[l], weights[b] =
+ * (root.min / leaf)^beta (fp64, stored in the real type), actions_out [B,N,A] = actions[l] and reward_out [B,N] =
+ * reward[l] from done [slots*envs] (uint8), actions [slots*envs,N,A] and reward [slots*envs,N].  An empty tree gives
+ * -1 indices and NaN.  FG_ERR_ARG also when B < 1, N outside [1, FG_MAX_AGENTS], A outside [1, 64], beta < 0 or not
+ * finite, a pointer NULL or not aligned to its type. */
+int fg_per_sample(const fg_per* t, const double* u, int B, double beta, const uint8_t* done, const void* actions,
+                  const void* reward, int N, int A, int64_t* rows, int64_t* index, int64_t* stamp_out,
+                  int64_t* slot_out, int64_t* env_out, uint8_t* done_out, void* weights, void* actions_out,
+                  void* reward_out, void* stream);
+int fg_per_sample_f64(const fg_per* t, const double* u, int B, double beta, const uint8_t* done, const void* actions,
+                      const void* reward, int N, int A, int64_t* rows, int64_t* index, int64_t* stamp_out,
+                      int64_t* slot_out, int64_t* env_out, uint8_t* done_out, void* weights, void* actions_out,
+                      void* reward_out, void* stream);
+
 /* Diagnostics, not on the step path: FP32 pipe probes used by bench.py to MEASURE the FP32 peak the
  * large-N step+reward kernel is graded against (BASELINE.json north_star: "% of FP32 peak at 243
  * agents"; MEASURED_PEAKS.json holds no FP32 figure).  variant 0: scalar FFMA (2 flop/lane/instr),
