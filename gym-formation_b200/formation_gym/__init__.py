@@ -15,7 +15,8 @@ call that needs the device raises).
 import importlib
 
 __all__ = ["make_env", "make_batched_env", "make_vec_env", "ezpolicy", "get_action_BFS", "MultiAgentEnv",
-           "BatchedFormationEnv", "CudaVecEnv", "StateReplayBuffer", "PrioritizedStateReplayBuffer", "SCENARIOS"]
+           "BatchedFormationEnv", "CudaVecEnv", "StateReplayBuffer", "PrioritizedStateReplayBuffer", "StateRolloutBuffer",
+           "SCENARIOS"]
 
 SCENARIOS = ("basic_formation_env", "formation_hd_env", "formation_hd_partial_env",
              "formation_hd_partial_range_env", "formation_hd_obs_env")
@@ -179,6 +180,9 @@ def __getattr__(name):
     if name == "PrioritizedStateReplayBuffer":
         from .replay import PrioritizedStateReplayBuffer
         return PrioritizedStateReplayBuffer
+    if name == "StateRolloutBuffer":
+        from .rollout import StateRolloutBuffer
+        return StateRolloutBuffer
     if name == "MultiAgentEnv":
         from .environment import MultiAgentEnv
         return MultiAgentEnv

@@ -28,7 +28,7 @@ EXPORTS = [
     "fg_step_policy_targets", "fg_step_policy_targets_f64", "fg_step_fused_final", "fg_step_fused_final_f64",
     "fg_step_policy_final", "fg_step_policy_final_f64", "fg_final_obs", "fg_final_obs_f64",
     "fg_obs_gather", "fg_obs_gather_f64", "fg_per_layout", "fg_per_fill", "fg_per_update", "fg_per_sample",
-    "fg_per_sample_f64",
+    "fg_per_sample_f64", "fg_gae", "fg_gae_f64",
 ]
 
 
@@ -142,6 +142,7 @@ def load():
             [P(fg_params), P(fg_final), C.c_longlong, VP, I, VP, I, I, I, VP]
         getattr(lib, "fg_per_sample" + sfx).argtypes = \
             [P(fg_per), VP, I, C.c_double, VP, VP, VP, I, I, VP, VP, VP, VP, VP, VP, VP, VP, VP, VP]
+        getattr(lib, "fg_gae" + sfx).argtypes = [VP, VP, VP, VP, VP, VP, I, C.c_longlong, I, C.c_double, C.c_double, VP]
         getattr(lib, "fg_random_actions" + sfx).argtypes = [VP, I, I, U64, U32, U32, VP, VP]
         getattr(lib, "fg_policy_bfs" + sfx).argtypes = [VP, VP, VP, VP, I, I, I, VP]
         getattr(lib, "fg_pair_distances" + sfx).argtypes = [VP, VP, I, I, VP, VP, VP, VP, VP]

@@ -444,6 +444,28 @@ int fg_per_sample_f64(const fg_per* t, const double* u, int B, double beta, cons
                       int64_t* slot_out, int64_t* env_out, uint8_t* done_out, void* weights, void* actions_out,
                       void* reward_out, void* stream);
 
+/* Generalized advantage estimation (Schulman et al. 2016) over an on-policy rollout of T steps of E envs x N agents,
+ * with time-limit truncations bootstrapped from the value of the state the episode ended in.  M = E*N columns, column
+ * c = e*N + n; all arrays on the device, in the real type (fp32 / fp64 for _f64) except done:
+ *   reward [T,E,N]; value [T+1,E,N]: value[t] = V(s_t), value[T] the bootstrap value of the rollout's last state;
+ *   done [T,E] uint8: nonzero when env e's episode ended at step t (env.done[:, 0]);
+ *   final_value [T,E,N] or NULL: V of the state the episode that ended at step t ended in; read only where done[t,e];
+ *   adv, ret [T,E,N]: outputs.
+ * With g = (real)gamma and gl = (real)(gamma * lambda) (the product taken in fp64 and rounded once), for every column
+ * from a = 0 and t = T-1 .. 0, every operation separately rounded (no contraction, in both precisions):
+ *   d = done[t*E + e] != 0;  nv = d ? (final_value ? final_value[t*M + c] : 0) : value[(t+1)*M + c]
+ *   delta = (reward[t*M + c] + g*nv) - value[t*M + c];  a = d ? delta : delta + gl*a
+ *   adv[t*M + c] = a;  ret[t*M + c] = a + value[t*M + c]
+ * final_value == NULL treats a truncation as a terminal.  value[t+1] after a done is never read into the result, so a
+ * NaN or inf there does not reach adv / ret.  Every column is independent: the result does not depend on the launch
+ * geometry.  No allocation, no synchronisation.  FG_ERR_ARG, before any device call, when reward / value / done / adv /
+ * ret is NULL, T < 1, E < 1, N outside [1, FG_MAX_AGENTS], T*E*N > 2^48, gamma or lambda is not finite or outside
+ * [0, 1], or an array is not aligned to the real type. */
+int fg_gae(const void* reward, const void* value, const void* final_value, const uint8_t* done, void* adv, void* ret,
+           int T, long long E, int N, double gamma, double lambda, void* stream);
+int fg_gae_f64(const void* reward, const void* value, const void* final_value, const uint8_t* done, void* adv,
+               void* ret, int T, long long E, int N, double gamma, double lambda, void* stream);
+
 /* Diagnostics, not on the step path: FP32 pipe probes used by bench.py to MEASURE the FP32 peak the
  * large-N step+reward kernel is graded against (BASELINE.json north_star: "% of FP32 peak at 243
  * agents"; MEASURED_PEAKS.json holds no FP32 figure).  variant 0: scalar FFMA (2 flop/lane/instr),
