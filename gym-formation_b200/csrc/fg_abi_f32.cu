@@ -39,8 +39,6 @@ Switches& switches() {
     (void)init;
     return sw;
 }
-
-int nvtx_enabled() { return switches().nvtx.load(std::memory_order_relaxed); }
 }  // namespace fgabi
 
 extern "C" {

@@ -4,74 +4,17 @@
 // compiled in parallel by formation_gym/_build.py).
 // Validates arguments, converts fg_params (double) into the kernels' typed argument block and
 // launches asynchronously on the caller's stream.  No allocation, no global state, no sync.
-#include <cstdio>
 #include <cstring>
 #include <cmath>
-
-#include "../../include/formation_gym_b200.h"
 #include <cstdlib>
 #include <type_traits>
+#include <algorithm>
 
+#include "fg_host.cuh"
 #include "fg_kernels.cuh"
 #include "fg_warp.cuh"
 #include "fg_obstacle.cuh"
 #include "fg_policy.cuh"
-
-#include <algorithm>
-#include <atomic>
-#include <nvtx3/nvToolsExt.h>
-
-namespace fgabi {
-extern thread_local char g_err[512];                          // defined in fg_abi_f32.cu, shared by both precisions
-
-// A/B switches for tests and profiling (fg_set_option / FG_<NAME> environment variables, read ONCE when the
-// library is first used -- never on the launch path).  Defaults select the product kernels.
-struct Switches {
-    std::atomic<int> no_fast_pairs{0};      // tile kernel: scalar pair loops instead of fg_pairs.cuh
-    std::atomic<int> force_fast_pairs{0};   // tile kernel: packed pair loops also for 32 <= N < 64 with observations
-    std::atomic<int> no_cells{0};           // packed pair loops: O(N^2) group filters instead of the cell lists
-    std::atomic<int> row_nbuf{2};           // OM == 2: staging buffers per warp (1 or 2)
-    std::atomic<int> no_early_rows{0};      // OM == 2: rows leave after the reward pass
-    std::atomic<int> no_tile_image{0};      // OM == 3 off: flat item loop
-    std::atomic<int> force_tile_kernel{0};  // fg_step_fused never takes the warp-autonomous kernel
-    std::atomic<int> waves{1};              // warp kernel: grid = waves x one resident wave (>= 1)
-    std::atomic<int> no_std_kernel{0};      // warp kernel: never the STD instantiation (standard configuration, flags compiled out)
-    std::atomic<int> l2_prefetch{1};        // warp kernel: prefetch.global.L2 of the state two spans ahead: 0 never, 1 auto, 2 always
-    std::atomic<int> pf_spans{2};           // ... how many spans ahead (2 .. 8)
-    std::atomic<int> row_chunks{1};         // OM == 2: chunked row writer (RC whole rows per image, one bulk store per chunk)
-    std::atomic<int> row_chunk_max_log2{7}; // chunked row writer: at most 2^k rows per chunk
-    std::atomic<int> row_min_n{10};         // OM == 2 (bulk-store row writers) from this agent count up
-    std::atomic<int> nvtx{1};               // NVTX ranges around the launches of every entry point
-};
-Switches& switches();                                         // defined in fg_abi_f32.cu
-}
-
-namespace {
-// NVTX range around the launches of one entry point (free when no tool is attached: one load + branch)
-struct NvtxRange {
-    bool on;
-    explicit NvtxRange(const char* name) : on(fgabi::switches().nvtx.load(std::memory_order_relaxed) != 0) {
-        if (on) nvtxRangePushA(name);
-    }
-    ~NvtxRange() { if (on) nvtxRangePop(); }
-};
-
-// cudaFuncAttributeMaxDynamicSharedMemorySize is sticky per (function, device): raise it only when a launch needs
-// more than what was set before (it used to be re-set on every launch: ~1 us of host time per step).
-constexpr int kMaxDev = 64;
-template <auto Kernel>
-cudaError_t ensure_dyn_smem(size_t smem) {
-    static std::atomic<size_t> have[kMaxDev];
-    if (smem <= 48 * 1024) return cudaSuccess;
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= kMaxDev)
-        return cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (smem <= have[dev].load(std::memory_order_acquire)) return cudaSuccess;
-    cudaError_t e = cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e == cudaSuccess) have[dev].store(smem, std::memory_order_release);
-    return e;
-}
-}
 
 namespace fgabi {
 // warp-autonomous kernel of the partial-observation scenarios (fg_lm_f32.cu / fg_lm_f64.cu): FG_OK / error code, or 1
@@ -81,13 +24,6 @@ int launch_lm_warp(const fg::KArgs<double>& a, int scenario, cudaStream_t st);
 }  // namespace fgabi
 
 namespace {
-
-using fgabi::g_err;
-
-int fail(int code, const char* fmt, const char* detail = "") {
-    snprintf(g_err, sizeof(g_err), fmt, detail);
-    return code;
-}
 
 uint32_t magic_for(int d) {          // floor(2^32 / d) + 1; 0 encodes d == 1 (fastdiv returns q)
     if (d <= 1) return 0u;
@@ -336,9 +272,17 @@ size_t fast_pairs_bytes(const fg::KArgs<T>& a) {
     return (8 * (size_t)a.EPC * NP + (size_t)a.EPC * 32) * sizeof(float) + 2 * (size_t)a.EPC * sizeof(unsigned) + 16;
 }
 
+// Tile kernels (k_step, k_step_obst): EPC envs per CTA of kBlock threads
+template <auto Kernel, typename T>
+int launch_tile(const fg::KArgs<T>& a, size_t smem, cudaStream_t st) {
+    cudaError_t err = ensure_dyn_smem<Kernel>(smem);
+    if (err != cudaSuccess) return fail(FG_ERR_CUDA, "cudaFuncSetAttribute failed: %s", cudaGetErrorString(err));
+    Kernel<<<(a.E + a.EPC - 1) / a.EPC, fg::kBlock, smem, st>>>(a);
+    return launch_status();
+}
+
 template <typename T, int SCN, bool PHYS, bool OBSREW, bool HET, int OM, bool FP, bool EXT>
 int launch_one_ext(const fg::KArgs<T>& a, size_t smem, cudaStream_t st) {
-    const int grid = (a.E + a.EPC - 1) / a.EPC;
     fg::KArgs<T> b = a;
     if (FP) {
         smem += fast_pairs_bytes(a);
@@ -352,14 +296,7 @@ int launch_one_ext(const fg::KArgs<T>& a, size_t smem, cudaStream_t st) {
     } else {
         b.cells = 0;
     }
-    {
-        cudaError_t e1 = ensure_dyn_smem<fg::k_step<T, SCN, PHYS, OBSREW, HET, OM, FP, EXT>>(smem);
-        if (e1 != cudaSuccess) return fail(FG_ERR_CUDA, "cudaFuncSetAttribute failed: %s", cudaGetErrorString(e1));
-    }
-    fg::k_step<T, SCN, PHYS, OBSREW, HET, OM, FP, EXT><<<grid, fg::kBlock, smem, st>>>(b);
-    cudaError_t err = cudaGetLastError();
-    if (err != cudaSuccess) return fail(FG_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(err));
-    return FG_OK;
+    return launch_tile<fg::k_step<T, SCN, PHYS, OBSREW, HET, OM, FP, EXT>>(b, smem, st);
 }
 
 // steps with a target bank or a terminal block, and fg_final_obs, take the EXT instantiation of the same kernel
@@ -414,15 +351,7 @@ int launch_obstacle_ext(const fg::KArgs<T>& a, void* stream) {
     size_t smem = (4 * nA + (size_t)a.EPC * a.L + 2 * (size_t)a.EPC * a.n_obst + 2 * a.EPC) * sizeof(R2)
                   + a.EPC * sizeof(Bits) + 3 * a.EPC * sizeof(int);
     smem = (smem + 15) & ~(size_t)15;
-    {
-        cudaError_t e1 = ensure_dyn_smem<fg::k_step_obst<T, PHYS, OBSREW, EXT>>(smem);
-        if (e1 != cudaSuccess) return fail(FG_ERR_CUDA, "cudaFuncSetAttribute failed: %s", cudaGetErrorString(e1));
-    }
-    const int grid = (a.E + a.EPC - 1) / a.EPC;
-    fg::k_step_obst<T, PHYS, OBSREW, EXT><<<grid, fg::kBlock, smem, (cudaStream_t)stream>>>(a);
-    cudaError_t err = cudaGetLastError();
-    if (err != cudaSuccess) return fail(FG_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(err));
-    return FG_OK;
+    return launch_tile<fg::k_step_obst<T, PHYS, OBSREW, EXT>>(a, smem, (cudaStream_t)stream);
 }
 
 template <typename T, bool PHYS, bool OBSREW = true>
@@ -432,15 +361,15 @@ int launch_obstacle(const fg::KArgs<T>& a, void* stream) {
     return launch_obstacle_ext<T, PHYS, OBSREW, false>(a, stream);
 }
 
-// ---- warp-autonomous fast path (fg_warp.cuh) ----------------------------------------------------
+// ---- warp-autonomous kernels (fg_warp.cuh k_hd_warp, fg_warp_lm.cuh k_lm_warp) ---------------------
 // Resident CTAs per SM for w warps per CTA (occupancy API; shared memory is the limiter: one
 // observation-span image per warp).  Computed once per instantiation; all GPUs of a box are alike.
+// LY: the kernel's layout (stride bytes of shared memory per warp, at most MAXW warps per CTA, EPW envs per span).
 struct WarpGeom { int ctas[4]; int best; int sms; };      // index: log2(w), w = 1, 2, 4, 8
 
-template <typename T, int N, bool WOBS, int SCN, bool STD, int POL = 0, bool EXT = false>
+template <auto Kernel, typename LY>
 const WarpGeom& warp_geom() {
     static const WarpGeom geom = [] {
-        typedef fg::WarpLayout<T, N, WOBS> LY;
         WarpGeom g_; g_.best = 0; g_.sms = 148;
         int dev = 0;
         if (cudaGetDevice(&dev) == cudaSuccess)
@@ -451,35 +380,39 @@ const WarpGeom& warp_geom() {
             const size_t smem = (size_t)w * LY::stride;
             g_.ctas[l] = 0;
             if (smem > 227 * 1024 || w > LY::MAXW) continue;
-            if (cudaFuncSetAttribute(fg::k_hd_warp<T, N, WOBS, SCN, STD, POL, EXT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                     (int)smem) != cudaSuccess) { cudaGetLastError(); continue; }
+            if (cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
+                cudaGetLastError();
+                continue;
+            }
             int ctas = 0;
-            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas, fg::k_hd_warp<T, N, WOBS, SCN, STD, POL, EXT>, 32 * w, smem)
-                != cudaSuccess) { cudaGetLastError(); continue; }
+            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas, Kernel, 32 * w, smem) != cudaSuccess) {
+                cudaGetLastError();
+                continue;
+            }
             g_.ctas[l] = ctas;
             if (ctas * w > best_res) { best_res = ctas * w; g_.best = l; }
         }
         // the probing above left the limit at the SMALLEST footprint, and a limit below the launch's request makes
         // the launch fail (also under the 48 KB default): restore the default-or-larger value; launches raise it
         // further through ensure_dyn_smem when they need more than 48 KB
-        cudaFuncSetAttribute(fg::k_hd_warp<T, N, WOBS, SCN, STD, POL, EXT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 48 * 1024);
+        cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 48 * 1024);
         cudaGetLastError();
         return g_;
     }();
     return geom;
 }
 
-template <typename T, int N, bool WOBS, int SCN, bool STD, int POL = 0, bool EXT = false>
-int launch_warp_ext(const fg::KArgs<T>& a, cudaStream_t st) {
-    typedef fg::WarpLayout<T, N, WOBS> LY;
-    const WarpGeom& gm = warp_geom<T, N, WOBS, SCN, STD, POL, EXT>();
+// name: the kernel's name in the "does not fit" message
+template <auto Kernel, typename LY, typename T>
+int launch_persistent(const fg::KArgs<T>& a, const char* name, cudaStream_t st) {
+    const WarpGeom& gm = warp_geom<Kernel, LY>();
     const int spans = (a.E + LY::EPW - 1) / LY::EPW;
     int l = gm.best;
     while (l > 0 && (spans >> l) < 2 * gm.sms) --l;                // small batches: spread over the SMs
-    if (gm.ctas[l] < 1) return fail(FG_ERR_CUDA, "k_hd_warp does not fit on this device%s");
+    if (gm.ctas[l] < 1) return fail(FG_ERR_CUDA, "%s does not fit on this device", name);
     const int w = 1 << l;
     const size_t smem = (size_t)w * LY::stride;
-    cudaError_t err = ensure_dyn_smem<fg::k_hd_warp<T, N, WOBS, SCN, STD, POL, EXT>>(smem);
+    cudaError_t err = ensure_dyn_smem<Kernel>(smem);
     if (err != cudaSuccess) return fail(FG_ERR_CUDA, "cudaFuncSetAttribute failed: %s", cudaGetErrorString(err));
     // persistent warps: at most one resident wave; each warp walks spans gw, gw + nwarps, ...
     int grid = (spans + w - 1) / w;
@@ -487,10 +420,13 @@ int launch_warp_ext(const fg::KArgs<T>& a, cudaStream_t st) {
     wave *= std::max(1, fgabi::switches().waves.load(std::memory_order_relaxed));
     if (grid > wave) grid = wave;
     if ((grid * w) & 1) ++grid;                                    // even warp count (16-byte phase, fg_warp.cuh)
-    fg::k_hd_warp<T, N, WOBS, SCN, STD, POL, EXT><<<grid, 32 * w, smem, st>>>(a);
-    err = cudaGetLastError();
-    if (err != cudaSuccess) return fail(FG_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(err));
-    return FG_OK;
+    Kernel<<<grid, 32 * w, smem, st>>>(a);
+    return launch_status();
+}
+
+template <typename T, int N, bool WOBS, int SCN, bool STD, int POL = 0, bool EXT = false>
+int launch_warp_ext(const fg::KArgs<T>& a, cudaStream_t st) {
+    return launch_persistent<fg::k_hd_warp<T, N, WOBS, SCN, STD, POL, EXT>, fg::WarpLayout<T, N, WOBS>>(a, "k_hd_warp", st);
 }
 
 // runs with a target bank or a terminal block take the EXT instantiation of the same kernel
@@ -500,18 +436,31 @@ int launch_warp_n(const fg::KArgs<T>& a, cudaStream_t st) {
     return launch_warp_ext<T, N, WOBS, SCN, STD, POL, false>(a, st);
 }
 
+// The standard product configuration: the fp32 warp kernels have an STD instantiation with these run-time tests
+// compiled out (fg_warp.cuh, fg_warp_lm.cuh).  Each caller decides what fp64 runs.
+template <typename T>
+bool std_config(const fg::KArgs<T>& a) {
+    return a.collide && !a.has_vmax && a.mass_one && a.n_steps == 1 && a.step && a.done && a.indiv && a.ep_return &&
+           a.ep_coll && a.stats && !a.comm && !fgabi::switches().no_std_kernel.load(std::memory_order_relaxed);
+}
+
 template <typename T, int N, int SCN = fg::kScnHD>
 int launch_warp(const fg::KArgs<T>& a, cudaStream_t st) {
-    if constexpr (std::is_same<T, float>::value) {
-        // the standard product configuration has its own instantiation with these run-time tests compiled out
-        // (fg_warp.cuh, STD); anything else takes the generic one
-        const bool std_cfg = a.collide && !a.has_vmax && a.mass_one && a.n_steps == 1 &&
-                             a.step && a.done && a.indiv && a.ep_return && a.ep_coll && a.stats && !a.comm &&
-                             !fgabi::switches().no_std_kernel.load(std::memory_order_relaxed);
-        if (std_cfg)
+    // fp32 standard configuration: the STD instantiation; anything else (fp64 too) the generic one
+    if constexpr (std::is_same<T, float>::value)
+        if (std_config(a))
             return a.obs ? launch_warp_n<T, N, true, SCN, true>(a, st) : launch_warp_n<T, N, false, SCN, true>(a, st);
-    }
     return a.obs ? launch_warp_n<T, N, true, SCN, false>(a, st) : launch_warp_n<T, N, false, SCN, false>(a, st);
+}
+
+// What neither warp-autonomous kernel handles: per-agent constants, walls, non-silent agents, cached contact
+// positions, unaligned observations; and the A/B switch for tests and profiling.
+template <typename T>
+bool warp_common_ok(const fg_params* p, const fg_buffers* b) {
+    if (p->agent_mass || p->agent_size_arr || p->agent_accel || p->agent_max_speed) return false;
+    if (p->n_walls != 0 || !p->silent || b->contact_pos) return false;
+    if (((uintptr_t)b->obs) % sizeof(typename fg::Ops<T>::R2)) return false;
+    return !fgabi::switches().force_tile_kernel.load(std::memory_order_relaxed);
 }
 
 // The fast path covers the configurations BASELINE.json names for formation_hd_env with N <= 27.
@@ -527,10 +476,7 @@ bool warp_path_ok(const fg::KArgs<T>& a, int scenario, const fg_params* p, const
         }
         if (b->landmarks) return false;                             // landmark tracking: tile kernel
     }
-    if (p->agent_mass || p->agent_size_arr || p->agent_accel || p->agent_max_speed) return false;
-    if (p->n_walls != 0 || !p->silent || b->contact_pos) return false;
-    if (((uintptr_t)b->obs) % sizeof(typename fg::Ops<T>::R2)) return false;
-    return !fgabi::switches().force_tile_kernel.load(std::memory_order_relaxed);   // A/B switch for tests and profiling
+    return warp_common_ok<T>(p, b);
 }
 
 // formation_hd_partial_env / formation_hd_partial_range_env on the warp-autonomous kernel (fg_warp_lm.cuh)
@@ -539,10 +485,43 @@ bool lm_warp_ok(const fg::KArgs<T>& a, int scenario, const fg_params* p, const f
     if (scenario != FG_SCENARIO_HD_PARTIAL && scenario != FG_SCENARIO_HD_PARTIAL_RANGE &&
         scenario != FG_SCENARIO_HD_OBSTACLE) return false;
     if (a.N < 3 || a.N > 9 || !b->landmarks || !b->obs) return false;
-    if (p->agent_mass || p->agent_size_arr || p->agent_accel || p->agent_max_speed) return false;
-    if (p->n_walls != 0 || !p->silent || b->contact_pos) return false;
-    if (((uintptr_t)b->obs) % sizeof(typename fg::Ops<T>::R2)) return false;
-    return !fgabi::switches().force_tile_kernel.load(std::memory_order_relaxed);   // A/B switch for tests and profiling
+    return warp_common_ok<T>(p, b);
+}
+
+// Per-scenario state: formation_hd_env reads ideal_shape / ideal_vel, every other scenario its landmarks
+int check_state(const fg_buffers* b, int scenario, const char* who) {
+    if (scenario == FG_SCENARIO_HD && (!b->ideal_shape || !b->ideal_vel))
+        return fail(FG_ERR_ARG, "%s(hd): ideal_shape/ideal_vel must be non-null", who);
+    if (scenario != FG_SCENARIO_HD && !b->landmarks)
+        return fail(FG_ERR_ARG, "%s: landmarks must be non-null for this scenario", who);
+    return FG_OK;
+}
+
+// The observation pass without physics (k_step / k_step_obst, PHYS off) of fg_obs_reward, fg_final_obs, fg_obs_gather
+template <typename T>
+int launch_obs(const fg::KArgs<T>& a, int scenario, const fg_params* p, void* stream) {
+    if (scenario == FG_SCENARIO_HD_OBSTACLE) return launch_obstacle<T, false>(a, stream);
+    return launch<T, false, true>(a, scenario, p, stream);
+}
+
+// The observation pass on the E records of a state block (fg_final layout) into obs, in the EXT instantiation:
+// fg_final_obs passes done (the rows of ended envs only), fg_obs_gather rows / R (slot b reads record rows[b] of R).
+// reward, step, done, nan_flag, lmv stay NULL.
+template <typename T>
+int state_obs(const fg_params* p, const fg_final* s, void* obs, int scenario, int E, int N, int L, const uint8_t* done,
+              const int64_t* rows, long long R, void* stream) {
+    fg_buffers b;
+    memset(&b, 0, sizeof(b));
+    b.pos = s->pos; b.vel = s->vel; b.obs = obs;
+    if (p && !p->silent) b.comm = s->comm;
+    if (scenario == FG_SCENARIO_HD) { b.ideal_shape = s->ideal_shape; b.ideal_vel = s->ideal_vel; }
+    else b.landmarks = s->landmarks;                                // (hd: no landmark side effect)
+    fg::KArgs<T> a;
+    int rc = fill_args<T>(a, p, &b, scenario, E, N, L, 0, 0, 0);
+    if (rc) return rc;
+    set_final<T>(a, s, p, scenario);
+    a.fin_done = done; a.gth_rows = rows; a.gth_count = R;
+    return launch_obs<T>(a, scenario, p, stream);
 }
 
 template <typename T>
@@ -574,13 +553,10 @@ int obs_reward_impl(const fg_params* p, const fg_buffers* b, int scenario, int E
     int rc = fill_args<T>(a, p, b, scenario, E, N, L, 0, 0, 0);
     if (rc) return rc;
     if (!b->pos || !b->vel || !b->reward) return fail(FG_ERR_ARG, "fg_obs_reward: pos/vel/reward must be non-null%s");
-    if (scenario == FG_SCENARIO_HD && (!b->ideal_shape || !b->ideal_vel))
-        return fail(FG_ERR_ARG, "fg_obs_reward(hd): ideal_shape/ideal_vel must be non-null%s");
-    if (scenario != FG_SCENARIO_HD && !b->landmarks)
-        return fail(FG_ERR_ARG, "fg_obs_reward: landmarks must be non-null for this scenario%s");
+    rc = check_state(b, scenario, "fg_obs_reward");
+    if (rc) return rc;
     a.step = nullptr; a.done = nullptr; a.ep_return = nullptr; a.ep_coll = nullptr; a.stats = nullptr;
-    if (scenario == FG_SCENARIO_HD_OBSTACLE) return launch_obstacle<T, false>(a, stream);
-    return launch<T, false, true>(a, scenario, p, stream);
+    return launch_obs<T>(a, scenario, p, stream);
 }
 
 // Terminal observations (fg_final_obs): the observation pass of fg_obs_reward (k_step / k_step_obst without PHYS) on the
@@ -593,19 +569,7 @@ int final_obs_impl(const fg_params* p, const fg_final* f, const uint8_t* done, v
     int rc = check_final<T>(f, p, scenario, 1, 1, false, "fg_final_obs");
     if (rc) return rc;
     if (!done || !obs) return fail(FG_ERR_ARG, "fg_final_obs: done / obs must be non-null%s");
-    fg_buffers b;
-    memset(&b, 0, sizeof(b));
-    b.pos = f->pos; b.vel = f->vel; b.obs = obs;
-    if (p && !p->silent) b.comm = f->comm;
-    if (scenario == FG_SCENARIO_HD) { b.ideal_shape = f->ideal_shape; b.ideal_vel = f->ideal_vel; }
-    else b.landmarks = f->landmarks;                                // (hd: no landmark side effect)
-    fg::KArgs<T> a;
-    rc = fill_args<T>(a, p, &b, scenario, E, N, L, 0, 0, 0);
-    if (rc) return rc;
-    set_final<T>(a, f, p, scenario);
-    a.fin_done = done;                                              // reward, step, done, nan_flag, lmv: NULL above
-    if (scenario == FG_SCENARIO_HD_OBSTACLE) return launch_obstacle<T, false>(a, stream);
-    return launch<T, false, true>(a, scenario, p, stream);
+    return state_obs<T>(p, f, obs, scenario, E, N, L, done, nullptr, 0, stream);
 }
 
 // Observations of sampled state records (fg_obs_gather): the same pass on a block of R records, in gather mode -- output
@@ -620,19 +584,7 @@ int obs_gather_impl(const fg_params* p, const fg_final* s, long long R, const in
     int rc = check_final<T>(s, p, scenario, 1, 1, false, "fg_obs_gather");
     if (rc) return rc;
     if (((uintptr_t)rows % sizeof(int64_t)) != 0) return fail(FG_ERR_ARG, "fg_obs_gather: rows must be 8-byte aligned%s");
-    fg_buffers b;
-    memset(&b, 0, sizeof(b));
-    b.pos = s->pos; b.vel = s->vel; b.obs = obs;
-    if (p && !p->silent) b.comm = s->comm;
-    if (scenario == FG_SCENARIO_HD) { b.ideal_shape = s->ideal_shape; b.ideal_vel = s->ideal_vel; }
-    else b.landmarks = s->landmarks;                                // (hd: no landmark side effect)
-    fg::KArgs<T> a;
-    rc = fill_args<T>(a, p, &b, scenario, B, N, L, 0, 0, 0);        // E = B output slots
-    if (rc) return rc;
-    set_final<T>(a, s, p, scenario);
-    a.gth_rows = rows; a.gth_count = R;                             // reward, step, done, nan_flag, lmv: NULL above
-    if (scenario == FG_SCENARIO_HD_OBSTACLE) return launch_obstacle<T, false>(a, stream);
-    return launch<T, false, true>(a, scenario, p, stream);
+    return state_obs<T>(p, s, obs, scenario, B, N, L, nullptr, rows, R, stream);   // E = B output slots
 }
 
 template <typename T>
@@ -660,18 +612,9 @@ int step_fused_impl(const fg_params* p, const fg_buffers* b, int scenario, int E
         return fail(FG_ERR_ARG, "fg_step_fused: random_actions supports silent agents only%s");
     if (random_actions == 2 && !b->act)
         return fail(FG_ERR_ARG, "fg_step_fused: random_actions == 2 records the drawn actions in b->act (non-null)%s");
-    if (scenario == FG_SCENARIO_HD && (!b->ideal_shape || !b->ideal_vel))
-        return fail(FG_ERR_ARG, "fg_step_fused(hd): ideal_shape/ideal_vel must be non-null%s");
-    if (scenario != FG_SCENARIO_HD && !b->landmarks)
-        return fail(FG_ERR_ARG, "fg_step_fused: landmarks must be non-null for this scenario%s");
+    rc = check_state(b, scenario, "fg_step_fused");
+    if (rc) return rc;
     a.n_steps = n_steps; a.random_actions = random_actions; a.auto_reset = auto_reset;
-    if (scenario == FG_SCENARIO_HD_OBSTACLE) {
-        if (lm_warp_ok<T>(a, scenario, p, b)) {
-            rc = fgabi::launch_lm_warp(a, scenario, (cudaStream_t)stream);
-            if (rc <= 0) return rc;                                 // (1: no instantiation -> tile kernel)
-        }
-        return launch_obstacle<T, true>(a, stream);
-    }
     if (warp_path_ok<T>(a, scenario, p, b)) {
         cudaStream_t st = (cudaStream_t)stream;
         if (scenario == FG_SCENARIO_BASIC) return launch_warp<T, 3, fg::kScnBasic>(a, st);
@@ -693,6 +636,7 @@ int step_fused_impl(const fg_params* p, const fg_buffers* b, int scenario, int E
         rc = fgabi::launch_lm_warp(a, scenario, (cudaStream_t)stream);
         if (rc <= 0) return rc;                                     // (1: no instantiation -> tile kernel)
     }
+    if (scenario == FG_SCENARIO_HD_OBSTACLE) return launch_obstacle<T, true>(a, stream);
     return launch<T, true, true>(a, scenario, p, stream);
 }
 
@@ -707,18 +651,14 @@ int reset_impl(const fg_params* p, const fg_buffers* b, int scenario, int E, int
     if (rc) return rc;
     set_targets<T>(a, tg);
     if (!b->pos || !b->vel) return fail(FG_ERR_ARG, "fg_reset: pos/vel must be non-null%s");
-    if (scenario == FG_SCENARIO_HD && (!b->ideal_shape || !b->ideal_vel))
-        return fail(FG_ERR_ARG, "fg_reset(hd): ideal_shape/ideal_vel must be non-null%s");
-    if (scenario != FG_SCENARIO_HD && !b->landmarks)
-        return fail(FG_ERR_ARG, "fg_reset: landmarks must be non-null for this scenario%s");
+    rc = check_state(b, scenario, "fg_reset");
+    if (rc) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     const int grid = (E + 127) / 128;
     if (scenario == FG_SCENARIO_HD) fg::k_reset<T, fg::kScnHD><<<grid, 128, 0, st>>>(a, mask);
     else if (scenario == FG_SCENARIO_HD_OBSTACLE) fg::k_reset_obst<T><<<grid, 128, 0, st>>>(a, mask);
     else                            fg::k_reset<T, fg::kScnBasic><<<grid, 128, 0, st>>>(a, mask);
-    cudaError_t err = cudaGetLastError();
-    if (err != cudaSuccess) return fail(FG_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(err));
-    return FG_OK;
+    return launch_status();
 }
 
 template <typename T>
@@ -732,9 +672,7 @@ int random_actions_impl(void* act, int E, int N, uint64_t seed, uint32_t tick, u
     if (grid > 148 * 32) grid = 148 * 32;                           // grid-stride beyond 32 CTAs per SM
     fg::k_random_actions<T><<<grid, 256, 0, (cudaStream_t)stream>>>((typename fg::Ops<T>::R2*)act, n, (uint32_t)N,
                                                                    seed, tick, env_offset, tick_dev);
-    cudaError_t err = cudaGetLastError();
-    if (err != cudaSuccess) return fail(FG_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(err));
-    return FG_OK;
+    return launch_status();
 }
 
 template <typename T>
@@ -748,9 +686,22 @@ int pair_distances_impl(const void* ent, const void* size, int E, int M, void* v
     int grid = (int)std::min<size_t>((total + 255) / 256, (size_t)148 * 16);
     fg::k_pair_distances<T><<<grid, 256, 0, (cudaStream_t)stream>>>((const R2*)ent, (const T*)size, E, M, (R2*)vect, (T*)mag,
                                                                     coll, (T*)mind);
-    cudaError_t err = cudaGetLastError();
-    if (err != cudaSuccess) return fail(FG_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(err));
-    return FG_OK;
+    return launch_status();
+}
+
+// The reference's controller tree over N agents, n per layer: N = n^levels (the reference asserts log(len(obs))/log(n)
+// is an integer, formation_gym/__init__.py:55-56; levels = 0 when it is not) and the multiplier log(M)/log(n) of each
+// layer of M agents, top first (:78).
+struct PolicyTree { int levels; double mult[fg::kPolicyMaxLevels]; };
+
+PolicyTree policy_tree(int N, int n) {
+    PolicyTree t{};
+    int M = N;
+    while (M > 1 && M % n == 0) { M /= n; ++t.levels; }
+    if (M != 1 || t.levels < 1 || t.levels > fg::kPolicyMaxLevels) return PolicyTree{};
+    M = N;
+    for (int l = 0; l < t.levels; ++l) { t.mult[l] = std::log((double)M) / std::log((double)n); M /= n; }
+    return t;
 }
 
 template <typename T>
@@ -761,18 +712,17 @@ int policy_bfs_impl(const void* pos, const void* shape, const void* ivel, void* 
     if (!pos || !shape || !ivel || !act) return fail(FG_ERR_ARG, "fg_policy_bfs: null pointer%s");
     if (E < 1 || N < 1 || N > FG_MAX_AGENTS) return fail(FG_ERR_ARG, "fg_policy_bfs: bad E or N%s");
     if (n < 2 || n > fg::kPolicyMaxFan) return fail(FG_ERR_ARG, "fg_policy_bfs: num_agents_per_layer must be in [2, 8]%s");
+    const PolicyTree tree = policy_tree(N, n);
+    const int levels = tree.levels;
+    if (!levels)
+        return fail(FG_ERR_ARG, "fg_policy_bfs: N must be a power of num_agents_per_layer ('Observation shape error!')%s");
     fg::PArgs<T> a;
     memset(&a, 0, sizeof(a));
-    int levels = 0, M = N;
-    while (M > 1 && M % n == 0) { M /= n; ++levels; }
-    // the reference asserts log(len(obs))/log(n) is an integer (formation_gym/__init__.py:55-56)
-    if (M != 1 || levels < 1 || levels > fg::kPolicyMaxLevels)
-        return fail(FG_ERR_ARG, "fg_policy_bfs: N must be a power of num_agents_per_layer ('Observation shape error!')%s");
     a.pos = (const R2*)pos; a.shape = (const R2*)shape; a.ivel = (const R2*)ivel; a.act = (R2*)act;
     a.E = E; a.N = N; a.n = n; a.levels = levels; a.EPC = fg::kBlock / N; a.magic_n = magic_for(N);
-    M = N;
+    int M = N;
     for (int l = 0; l < levels; ++l) {
-        a.mult[l] = (T)(std::log((double)M) / std::log((double)n));                             // :78
+        a.mult[l] = (T)tree.mult[l];
         a.lev_M[l] = M; a.lev_nxt[l] = M / n; a.lev_nlead[l] = N / (M / n);
         a.mg_M[l] = magic_for(M); a.mg_nxt[l] = magic_for(M / n); a.mg_nlead[l] = magic_for(N / (M / n));
         M /= n;
@@ -798,9 +748,7 @@ int policy_bfs_impl(const void* pos, const void* shape, const void* ivel, void* 
                 default: fg::k_policy_bfs<T, 0><<<grid, fg::kBlock, smem, st>>>(a); break;
             }
     }
-    cudaError_t err = cudaGetLastError();
-    if (err != cudaSuccess) return fail(FG_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(err));
-    return FG_OK;
+    return launch_status();
 }
 
 }  // namespace

@@ -5,35 +5,16 @@
 // [T, E, N], value [T+1, E, N], done [T, E] uint8.  One thread owns one column and walks t = T-1 .. 0; warps are
 // coalesced over c.  Every operation is a separately rounded intrinsic, so nvcc cannot contract a multiply-add and a
 // numpy loop in the same dtype reproduces adv / ret bit for bit (DESIGN.md 3.3g).
-#include <cuda_runtime.h>
 #include <stdint.h>
 #include <cmath>
-#include <cstdio>
-#include <nvtx3/nvToolsExt.h>
 
-#include "../../include/formation_gym_b200.h"
-
-namespace fgabi {
-extern thread_local char g_err[512];                          // defined in fg_abi_f32.cu
-int nvtx_enabled();                                           // the nvtx switch (fg_set_option), fg_abi_f32.cu
-}
+#include "fg_host.cuh"
 
 namespace {
 
 constexpr int kThreads = 256;
 constexpr int kAhead = 8;                                     // rollout steps whose loads are issued before their math
 constexpr long long kMaxElems = 1ll << 48;                    // T*E*N: (T+1)*M*8 bytes stays far below 2^63
-
-int fail(const char* fmt, const char* who) {
-    snprintf(fgabi::g_err, sizeof(fgabi::g_err), fmt, who);
-    return FG_ERR_ARG;
-}
-
-struct NvtxRange {
-    bool on;
-    explicit NvtxRange(const char* name) : on(fgabi::nvtx_enabled() != 0) { if (on) nvtxRangePushA(name); }
-    ~NvtxRange() { if (on) nvtxRangePop(); }
-};
 
 bool aligned(const void* p, size_t a) { return ((uintptr_t)p % a) == 0; }
 
@@ -102,16 +83,19 @@ template <typename T>
 int gae_impl(const void* reward, const void* value, const void* final_value, const uint8_t* done, void* adv,
              void* ret, int T_, long long E, int N, double gamma, double lambda, void* stream, const char* who) {
     NvtxRange nvtx_(who);
-    if (!reward || !value || !done || !adv || !ret) return fail("%s: reward / value / done / adv / ret must be non-null", who);
-    if (T_ < 1) return fail("%s: T must be >= 1", who);
-    if (E < 1) return fail("%s: E must be >= 1", who);
-    if (N < 1 || N > FG_MAX_AGENTS) return fail("%s: N must be in [1, FG_MAX_AGENTS=256]", who);
-    if (E > kMaxElems / ((long long)T_ * N)) return fail("%s: T * E * N must be <= 2^48", who);
-    if (!std::isfinite(gamma) || gamma < 0.0 || gamma > 1.0) return fail("%s: gamma must be finite and in [0, 1]", who);
-    if (!std::isfinite(lambda) || lambda < 0.0 || lambda > 1.0) return fail("%s: lambda must be finite and in [0, 1]", who);
+    if (!reward || !value || !done || !adv || !ret)
+        return fail(FG_ERR_ARG, "%s: reward / value / done / adv / ret must be non-null", who);
+    if (T_ < 1) return fail(FG_ERR_ARG, "%s: T must be >= 1", who);
+    if (E < 1) return fail(FG_ERR_ARG, "%s: E must be >= 1", who);
+    if (N < 1 || N > FG_MAX_AGENTS) return fail(FG_ERR_ARG, "%s: N must be in [1, FG_MAX_AGENTS=256]", who);
+    if (E > kMaxElems / ((long long)T_ * N)) return fail(FG_ERR_ARG, "%s: T * E * N must be <= 2^48", who);
+    if (!std::isfinite(gamma) || gamma < 0.0 || gamma > 1.0)
+        return fail(FG_ERR_ARG, "%s: gamma must be finite and in [0, 1]", who);
+    if (!std::isfinite(lambda) || lambda < 0.0 || lambda > 1.0)
+        return fail(FG_ERR_ARG, "%s: lambda must be finite and in [0, 1]", who);
     if (!aligned(reward, sizeof(T)) || !aligned(value, sizeof(T)) || !aligned(final_value, sizeof(T)) ||
         !aligned(adv, sizeof(T)) || !aligned(ret, sizeof(T)))
-        return fail("%s: reward / value / final_value / adv / ret must be aligned to the real type", who);
+        return fail(FG_ERR_ARG, "%s: reward / value / final_value / adv / ret must be aligned to the real type", who);
     // grid-stride over columns with one wave of resident CTAs: SM count x CTAs per SM at the kernel's register count
     int dev = 0, sms = 0, per_sm = 0;
     cudaError_t err = cudaGetDevice(&dev);
@@ -127,10 +111,7 @@ int gae_impl(const void* reward, const void* value, const void* final_value, con
     k_gae<T><<<(unsigned)blocks, kThreads, 0, (cudaStream_t)stream>>>(
         (const T*)reward, (const T*)value, (const T*)final_value, done, (T*)adv, (T*)ret, T_, E, N, (T)gamma,
         (T)(gamma * lambda));
-    err = cudaGetLastError();
-    if (err == cudaSuccess) return FG_OK;
-    snprintf(fgabi::g_err, sizeof(fgabi::g_err), "%s: kernel launch failed: %s", who, cudaGetErrorString(err));
-    return FG_ERR_CUDA;
+    return launch_status(who);
 }
 
 }  // namespace

@@ -10,18 +10,10 @@
 // (one launch per level), and concurrent writers of one node store identical bits.  Nothing accumulates atomically.
 //
 // Kernels are warp-shaped: a warp owns one node (its 32 children are one coalesced 256-byte load) or one draw.
-#include <cuda_runtime.h>
 #include <stdint.h>
 #include <cmath>
-#include <cstdio>
-#include <nvtx3/nvToolsExt.h>
 
-#include "../../include/formation_gym_b200.h"
-
-namespace fgabi {
-extern thread_local char g_err[512];                          // defined in fg_abi_f32.cu
-int nvtx_enabled();                                           // the nvtx switch (fg_set_option), fg_abi_f32.cu
-}
+#include "fg_host.cuh"
 
 namespace {
 
@@ -29,17 +21,6 @@ constexpr int kMaxDepth = 8;                                  // M <= 2^40 leave
 constexpr long long kMaxLeaves = 1ll << 40;
 constexpr unsigned kFull = 0xffffffffu;
 constexpr int kThreads = 256;                                 // 8 warps per CTA
-
-int fail(const char* fmt, const char* who) {
-    snprintf(fgabi::g_err, sizeof(fgabi::g_err), fmt, who);
-    return FG_ERR_ARG;
-}
-
-struct NvtxRange {
-    bool on;
-    explicit NvtxRange(const char* name) : on(fgabi::nvtx_enabled() != 0) { if (on) nvtxRangePushA(name); }
-    ~NvtxRange() { if (on) nvtxRangePop(); }
-};
 
 // Device view of an fg_per with its layout: cnt[k] nodes at level k (cnt[0] = M leaves), level k >= 1 stored at
 // sum/min + off[k]; the root is sum/min[off[depth]].
@@ -68,33 +49,26 @@ void layout(long long M, Tree* t, long long* nodes, int* depth) {
 }
 
 int check_sizes(long long slots, long long envs, const char* who) {
-    if (slots < 1 || envs < 1) return fail("%s: slots and envs must be >= 1", who);
-    if (slots > kMaxLeaves / envs) return fail("%s: slots * envs must be <= 2^40", who);
+    if (slots < 1 || envs < 1) return fail(FG_ERR_ARG, "%s: slots and envs must be >= 1", who);
+    if (slots > kMaxLeaves / envs) return fail(FG_ERR_ARG, "%s: slots * envs must be <= 2^40", who);
     return FG_OK;
 }
 
 int make_tree(const fg_per* p, Tree* t, const char* who) {
-    if (!p) return fail("%s: the tree must be non-null", who);
+    if (!p) return fail(FG_ERR_ARG, "%s: the tree must be non-null", who);
     int rc = check_sizes(p->slots, p->envs, who);
     if (rc) return rc;
     if (!p->leaf || !p->sum || !p->min || !p->max_leaf || !p->stamp || !p->prev || !p->scratch)
-        return fail("%s: fg_per arrays must be non-null", who);
+        return fail(FG_ERR_ARG, "%s: fg_per arrays must be non-null", who);
     if (!aligned(p->leaf, 8) || !aligned(p->sum, 8) || !aligned(p->min, 8) || !aligned(p->max_leaf, 8) ||
         !aligned(p->stamp, 8) || !aligned(p->prev, 8) || !aligned(p->scratch, 4))
-        return fail("%s: fg_per arrays must be 8-byte aligned (scratch: 4-byte)", who);
+        return fail(FG_ERR_ARG, "%s: fg_per arrays must be 8-byte aligned (scratch: 4-byte)", who);
     t->leaf = p->leaf; t->sum = p->sum; t->mn = p->min; t->max_leaf = p->max_leaf;
     t->stamp = p->stamp; t->prev = p->prev; t->owner = (int*)p->scratch;
     t->T = p->slots; t->E = p->envs; t->M = p->slots * p->envs;
     long long nodes;
     layout(t->M, t, &nodes, &t->depth);
     return FG_OK;
-}
-
-int launch_status(const char* who) {
-    cudaError_t err = cudaGetLastError();
-    if (err == cudaSuccess) return FG_OK;
-    snprintf(fgabi::g_err, sizeof(fgabi::g_err), "%s: kernel launch failed: %s", who, cudaGetErrorString(err));
-    return FG_ERR_CUDA;
 }
 
 unsigned grid_for(long long threads, long long cap = 1ll << 30) {
@@ -284,19 +258,20 @@ int per_sample_impl(const fg_per* p, const double* u, int B, double beta, const 
     Tree t;
     int rc = make_tree(p, &t, who);
     if (rc) return rc;
-    if (B < 1) return fail("%s: B must be >= 1", who);
-    if (N < 1 || N > FG_MAX_AGENTS) return fail("%s: N must be in [1, FG_MAX_AGENTS=256]", who);
-    if (A < 1 || A > 64) return fail("%s: A must be in [1, 64]", who);
-    if (!(beta >= 0.0) || !std::isfinite(beta)) return fail("%s: beta must be finite and >= 0", who);
-    if (!u || !done || !actions || !reward) return fail("%s: u / done / actions / reward must be non-null", who);
+    if (B < 1) return fail(FG_ERR_ARG, "%s: B must be >= 1", who);
+    if (N < 1 || N > FG_MAX_AGENTS) return fail(FG_ERR_ARG, "%s: N must be in [1, FG_MAX_AGENTS=256]", who);
+    if (A < 1 || A > 64) return fail(FG_ERR_ARG, "%s: A must be in [1, 64]", who);
+    if (!(beta >= 0.0) || !std::isfinite(beta)) return fail(FG_ERR_ARG, "%s: beta must be finite and >= 0", who);
+    if (!u || !done || !actions || !reward)
+        return fail(FG_ERR_ARG, "%s: u / done / actions / reward must be non-null", who);
     if (!rows || !index || !stamp_out || !slot_out || !env_out || !done_out || !weights || !actions_out || !reward_out)
-        return fail("%s: outputs must be non-null", who);
+        return fail(FG_ERR_ARG, "%s: outputs must be non-null", who);
     if (!aligned(u, 8) || !aligned(rows, 8) || !aligned(index, 8) || !aligned(stamp_out, 8) || !aligned(slot_out, 8) ||
         !aligned(env_out, 8))
-        return fail("%s: u and the int64 outputs must be 8-byte aligned", who);
+        return fail(FG_ERR_ARG, "%s: u and the int64 outputs must be 8-byte aligned", who);
     if (!aligned(actions, sizeof(T)) || !aligned(reward, sizeof(T)) || !aligned(weights, sizeof(T)) ||
         !aligned(actions_out, sizeof(T)) || !aligned(reward_out, sizeof(T)))
-        return fail("%s: actions / reward / weights must be aligned to the real type", who);
+        return fail(FG_ERR_ARG, "%s: actions / reward / weights must be aligned to the real type", who);
     cudaStream_t st = (cudaStream_t)stream;
     k_per_sample<T><<<grid_for((long long)B * 32), kThreads, 0, st>>>(
         t, u, B, beta, done, (const T*)actions, (const T*)reward, N, A, rows, index, stamp_out, slot_out, env_out,
@@ -316,7 +291,8 @@ void per_update_launch(const Tree& t, const int64_t* index, const int64_t* stamp
 extern "C" {
 
 int fg_per_layout(long long slots, long long envs, long long* nodes, int* depth, long long* scratch_bytes) {
-    if (!nodes || !depth || !scratch_bytes) return fail("%s: nodes / depth / scratch_bytes must be non-null", "fg_per_layout");
+    if (!nodes || !depth || !scratch_bytes)
+        return fail(FG_ERR_ARG, "%s: nodes / depth / scratch_bytes must be non-null", "fg_per_layout");
     int rc = check_sizes(slots, envs, "fg_per_layout");
     if (rc) return rc;
     layout(slots * envs, nullptr, nodes, depth);
@@ -331,12 +307,13 @@ int fg_per_fill(const fg_per* p, long long slot, long long prev, long long stamp
     Tree t;
     int rc = make_tree(p, &t, who);
     if (rc) return rc;
-    if (slot < 0 || slot >= t.T) return fail("%s: slot out of range", who);
-    if (prev < -1 || prev >= t.T || prev == slot) return fail("%s: prev must be -1 or another slot", who);
-    if (drop_slot < -1 || drop_slot >= t.T || drop_slot == slot) return fail("%s: drop_slot must be -1 or another slot", who);
-    if (valid != 0 && valid != 1) return fail("%s: valid must be 0 or 1", who);
-    if (valid && prev < 0) return fail("%s: a valid transition needs prev >= 0", who);
-    if (stamp < 0) return fail("%s: stamp must be >= 0", who);
+    if (slot < 0 || slot >= t.T) return fail(FG_ERR_ARG, "%s: slot out of range", who);
+    if (prev < -1 || prev >= t.T || prev == slot) return fail(FG_ERR_ARG, "%s: prev must be -1 or another slot", who);
+    if (drop_slot < -1 || drop_slot >= t.T || drop_slot == slot)
+        return fail(FG_ERR_ARG, "%s: drop_slot must be -1 or another slot", who);
+    if (valid != 0 && valid != 1) return fail(FG_ERR_ARG, "%s: valid must be 0 or 1", who);
+    if (valid && prev < 0) return fail(FG_ERR_ARG, "%s: a valid transition needs prev >= 0", who);
+    if (stamp < 0) return fail(FG_ERR_ARG, "%s: stamp must be >= 0", who);
     int dev = 0, sms = 0;                                    // grid-stride fill: 8 CTAs per SM cover any E
     cudaError_t err = cudaGetDevice(&dev);
     if (err == cudaSuccess) err = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
@@ -359,13 +336,13 @@ int fg_per_update(const fg_per* p, const int64_t* index, const int64_t* stamp, c
     Tree t;
     int rc = make_tree(p, &t, who);
     if (rc) return rc;
-    if (B < 1) return fail("%s: B must be >= 1", who);
-    if (!index || !stamp || !td) return fail("%s: index / stamp / td must be non-null", who);
-    if (td_f64 != 0 && td_f64 != 1) return fail("%s: td_f64 must be 0 or 1", who);
+    if (B < 1) return fail(FG_ERR_ARG, "%s: B must be >= 1", who);
+    if (!index || !stamp || !td) return fail(FG_ERR_ARG, "%s: index / stamp / td must be non-null", who);
+    if (td_f64 != 0 && td_f64 != 1) return fail(FG_ERR_ARG, "%s: td_f64 must be 0 or 1", who);
     if (!aligned(index, 8) || !aligned(stamp, 8) || !aligned(td, td_f64 ? 8 : 4))
-        return fail("%s: index / stamp / td must be aligned to their type", who);
-    if (!(alpha >= 0.0) || !std::isfinite(alpha)) return fail("%s: alpha must be finite and >= 0", who);
-    if (!(eps > 0.0) || !std::isfinite(eps)) return fail("%s: eps must be finite and > 0", who);
+        return fail(FG_ERR_ARG, "%s: index / stamp / td must be aligned to their type", who);
+    if (!(alpha >= 0.0) || !std::isfinite(alpha)) return fail(FG_ERR_ARG, "%s: alpha must be finite and >= 0", who);
+    if (!(eps > 0.0) || !std::isfinite(eps)) return fail(FG_ERR_ARG, "%s: eps must be finite and > 0", who);
     cudaStream_t st = (cudaStream_t)stream;
     if (td_f64) per_update_launch<double>(t, index, stamp, td, B, alpha, eps, st);
     else per_update_launch<float>(t, index, stamp, td, B, alpha, eps, st);

@@ -23,17 +23,10 @@ namespace {
 
 template <typename T, int N, int POL>
 int launch_warp_pol(const fg::KArgs<T>& a, cudaStream_t st) {
-    // fp32: the standard product configuration only (STD instantiation; launch_warp's test); fp64: the generic one
+    // fp32: the standard product configuration only (STD instantiation; std_config); fp64: the generic one
     constexpr bool STD = std::is_same<T, float>::value;
     return a.obs ? launch_warp_n<T, N, true, fg::kScnHD, STD, POL>(a, st)
                  : launch_warp_n<T, N, false, fg::kScnHD, STD, POL>(a, st);
-}
-
-template <typename T>
-bool std_config(const fg::KArgs<T>& a) {
-    if (!std::is_same<T, float>::value) return true;
-    return a.collide && !a.has_vmax && a.mass_one && a.step && a.done && a.indiv && a.ep_return && a.ep_coll &&
-           a.stats && !a.comm && !fgabi::switches().no_std_kernel.load(std::memory_order_relaxed);
 }
 
 template <typename T>
@@ -53,9 +46,8 @@ int step_policy_impl(const fg_params* p, const fg_buffers* b, int scenario, int 
                                 "(ideal_shape / ideal_vel; formation_gym/__init__.py:19-47)%s");
     if (n_steps < 1) return fail(FG_ERR_ARG, "fg_step_policy: n_steps must be >= 1%s");
     if (n < 2 || n > fg::kPolicyMaxFan) return fail(FG_ERR_ARG, "fg_step_policy: num_agents_per_layer must be in [2, 8]%s");
-    int levels = 0, M = N;
-    while (M > 1 && M % n == 0) { M /= n; ++levels; }
-    if (M != 1 || levels < 1 || levels > fg::kPolicyMaxLevels)
+    const PolicyTree tree = policy_tree(N, n);
+    if (!tree.levels)
         return fail(FG_ERR_ARG, "fg_step_policy: N must be a power of num_agents_per_layer ('Observation shape error!')%s");
     if (!p || !b) return fail(FG_ERR_ARG, "null params/buffers%s");
     if (!b->act || !b->pos || !b->ideal_shape || !b->ideal_vel)
@@ -67,11 +59,12 @@ int step_policy_impl(const fg_params* p, const fg_buffers* b, int scenario, int 
     if (rc) return rc;
     set_targets<T>(a, tg);
     set_final<T>(a, fin, p, scenario);
-    const bool fused = b->vel && b->reward && b->done && b->step && warp_path_ok<T>(a, scenario, p, b) && std_config<T>(a);
+    // (fp64 has no STD instantiation: every configuration the warp path takes is fused)
+    const bool fused = b->vel && b->reward && b->done && b->step && warp_path_ok<T>(a, scenario, p, b) &&
+                       (!std::is_same<T, float>::value || std_config<T>(a));
     if (fused) {
         a.random_actions = 0; a.auto_reset = auto_reset;
-        M = N;
-        for (int l = 0; l < levels; ++l) { a.pol_mult[l] = (T)(std::log((double)M) / std::log((double)n)); M /= n; }   // :78
+        for (int l = 0; l < tree.levels; ++l) a.pol_mult[l] = (T)tree.mult[l];
         cudaStream_t st = (cudaStream_t)stream;
         // fp32 runs the STD instantiation, which is compiled for one step per launch: a rollout is n_steps launches
         // (with a device tick the kernel advances it itself; otherwise the tick argument counts the steps)
